@@ -14,6 +14,7 @@ every N, c4 = 64 x 4096^2 bilateral + CLAHE, c5 = NLM), each with its own roofli
       bench.py --gpus N --steps K --warmup W
   python bench.py --impl reference ...      # CPU arm: the kornia-style torch-CPU twin on the host cores
   python bench.py --no-sub                  # headline only (profiling runs)
+  python bench.py --dump-outputs DIR        # also save a fixed sample of the last timed step's output (DIR/chain_out.npy)
 """
 from __future__ import annotations
 
@@ -35,6 +36,7 @@ UNIT = "Mpixel/s"
 WORKLOAD = ("configs[1]: batch 256 x 512x512 uint16 phantom slices, Gaussian K=9 sigma=1 reflect -> "
             "CLAHE 8x8 clip 2.0 -> unsharp K=9 sigma=1, uint16 out")
 CPU_SAMPLE = 32   # slices of the 256-slice batch the CPU arms time per step
+DUMP_SLICES = 32  # slices of the last timed step's output that --dump-outputs saves (32 MiB as float32)
 
 
 def _peaks():
@@ -262,9 +264,11 @@ def run_reference(args):
         _twin_chain(xt)
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        _twin_chain(xt)
+        y = _twin_chain(xt)
     dt = time.perf_counter() - t0
     value = CPU_SAMPLE * H * W * args.steps / dt / 1e6
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, y)
     secondary = None
     try:   # the C oracle port beside it (labelled secondary)
         import oracle as O
@@ -292,6 +296,22 @@ def run_reference(args):
         "gpu_launches": 0,
     }
     emit(line)
+
+
+def dump_outputs(out_dir: str, y) -> None:
+    """Saves DUMP_SLICES slices of the chain output `y` (N x 1 x H x W), picked with a fixed seed and converted to
+    float32 (exact for uint16), as out_dir/chain_out.npy: the same arguments give the same inputs on every run, so
+    two builds can be compared output for output."""
+    import numpy as np
+    import torch
+
+    idx = torch.from_numpy(np.sort(np.random.default_rng(0).choice(y.shape[0], min(DUMP_SLICES, y.shape[0]), replace=False)))
+    if y.dtype == torch.uint16:   # torch has no CUDA gather for uint16: gather the same bits as int16
+        sample = y.view(torch.int16)[idx.to(y.device)].cpu().numpy().view(np.uint16)
+    else:
+        sample = y[idx.to(y.device)].cpu().numpy()
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "chain_out.npy"), sample.astype(np.float32))
 
 
 # ---------------------------------------------------------------------------------------------- GPU helpers
@@ -685,6 +705,9 @@ def run_ours(args):
     barrier()
     ms_step = _max_over_ranks(dist, dev, e0.elapsed_time(e1)) / args.steps
     value = world * PIXELS / (ms_step * 1e-3) / 1e6
+    if args.dump_outputs and rank == 0:
+        # the ring slot of the last timed step, saved before the replays below overwrite it
+        dump_outputs(args.dump_outputs, ring.plans[(step_no[0] - 1) % len(ring.plans)].out)
 
     # ---- one step alone (single plan, back to back on one stream): what a caller without a ring gets
     for _ in range(3):
@@ -874,7 +897,11 @@ def main():
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--no-sub", action="store_true", help="headline only: skip the c1 / c3 / c4 / c5 sub-records")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write a fixed, seeded sample of the last timed step's output to DIR/chain_out.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -1,4 +1,4 @@
-import sys; sys.path.insert(0,"/root/repo")
+import os, sys; sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np, torch, mie_b200 as M
 from mie_b200 import synthetic
 for nb in (1,2,4,8,16,32):

@@ -1,4 +1,4 @@
-import sys; sys.path.insert(0,".")
+import os, sys; sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np, torch, mie_b200 as M
 from mie_b200 import synthetic
 x=torch.from_numpy(synthetic.phantom_volume((1,512,512),np.int16,0)).cuda().unsqueeze(1)
