@@ -322,6 +322,31 @@ int mie_sk_equalize_adapthist(const void* src, void* dst, int src_dtype, int dst
                               int64_t dst_stride_n, int64_t dst_stride_h,
                               int kr, int kc, double clip_limit, int nbins,
                               void* workspace, size_t workspace_bytes, void* stream);
+/* mie_sk_equalize_adapthist3d: skimage.exposure.equalize_adapthist on a 3-D array — every (d, h, w) volume of the batch
+ * is ONE image (mie_sk_equalize_adapthist treats each plane on its own).  Same dtypes, nbins range and error codes as
+ * the 2-D entry point; (kd, kr, kc) = kernel_size in voxels (skimage default: max(dim/8, 1) per axis), kd*kr*kc <= 2^31-1.
+ * Semantics, in volume coordinates (z, y, x):
+ *   grey  = round_half_even(rescale_intensity(img_as_float(v), out_range=(0, 16383))) with min / max over the VOLUME
+ *           (float64 for integer input, float32 for float32 input); bin = grey / (1 + 16384 / nbins);
+ *   regions: ceil(d/kd) x ceil(h/kr) x ceil(w/kc) boxes anchored at the origin, completed past the far faces by numpy
+ *           'reflect' padding (repeated reflection for pads longer than the axis); per region histogram -> clip_histogram
+ *           with clim = max(int(clip_limit * kd*kr*kc), 1) (clip_limit <= 0: 65535, ASSUMED as in 2-D) ->
+ *           map = int(min(cumsum * (16383 / (kd*kr*kc)) + 0, 16383));
+ *   voxel (z, y, x) lies in block ((z + kd/2) / kd, ...) at position ((z + kd/2) % kd, ...); per axis it blends regions
+ *           clamp(block - 1) and clamp(block) with weights (1 - c, c), c = pos / k (float64); the coefficient of edge
+ *           (ez, ey, ex) is (wx[ex] * wy[ey]) * wz[ez]; acc += (float)(map * coef) in float32 over the edges in
+ *           np.ndindex(2, 2, 2) order (z outermost); truncated to uint16;
+ *   out   = rescale_intensity(out_range=(0, 1)) of that uint16 volume, min / max over the volume.
+ * Launches: min / max, a code -> bin table per volume (integer input), one thread-block cluster per region (large
+ * regions are counted by up to 8 CTAs and merged through distributed shared memory), trilinear blend (+ min / max),
+ * rescale.  The workspace holds n * 65536 table entries whatever the dtype.                                           */
+size_t mie_sk_adapthist3d_workspace_bytes(int64_t n, int d, int h, int w, int kd, int kr, int kc, int nbins);
+int mie_sk_equalize_adapthist3d(const void* src, void* dst, int src_dtype, int dst_dtype,
+                                int64_t n, int d, int h, int w,
+                                int64_t src_stride_n, int64_t src_stride_d, int64_t src_stride_h,
+                                int64_t dst_stride_n, int64_t dst_stride_d, int64_t dst_stride_h,
+                                int kd, int kr, int kc, double clip_limit, int nbins,
+                                void* workspace, size_t workspace_bytes, void* stream);
 size_t mie_sk_equalize_hist_workspace_bytes(int64_t n, int src_dtype);
 int mie_sk_equalize_hist(const void* src, void* dst, int src_dtype, int dst_dtype,
                          int64_t n, int h, int w,

@@ -61,6 +61,9 @@ SIGNATURES = {
     "mie_bilateral_clahe": ([_p, _p, _i, _i, *_planes, _p, _i, _f, _i, _i, _i, _d, _f, _f, _i, _p, _sz, _p], _i),
     "mie_sk_adapthist_workspace_bytes": ([_i64, _i, _i, _i, _i, _i], _sz),
     "mie_sk_equalize_adapthist": ([_p, _p, _i, _i, *_planes, _i, _i, _d, _i, _p, _sz, _p], _i),
+    "mie_sk_adapthist3d_workspace_bytes": ([_i64, _i, _i, _i, _i, _i, _i, _i], _sz),
+    "mie_sk_equalize_adapthist3d": ([_p, _p, _i, _i, _i64, _i, _i, _i, _i64, _i64, _i64, _i64, _i64, _i64,
+                                     _i, _i, _i, _d, _i, _p, _sz, _p], _i),
     "mie_sk_equalize_hist_workspace_bytes": ([_i64, _i], _sz),
     "mie_sk_equalize_hist": ([_p, _p, _i, _i, *_planes, _p, _sz, _p], _i),
     "mie_sk_denoise_bilateral": ([_p, _p, _i, _i, *_planes, _i, _i, _i, _d, _p, _p, _p, _p], _i),

@@ -28,7 +28,8 @@ arithmetic is fp32 (skimage: float64 for integer input): agreement with scipy.nd
 These three have different algorithms from their kornia counterparts (SURVEY.md Appendix B3/B4) and their own
 kernels (csrc/sk_exposure.cu, csrc/sk_bilateral.cu).  They keep skimage's numerics — float64 arithmetic and a float64
 result in [0, 1] for integer images (out_dtype=torch.float32 rounds it once) — and skimage's per-image semantics:
-every (H, W) plane of the input is one image.  RECALLED semantics, restated in oracle/skimage_twin.py (numpy,
+every (H, W) plane of the input is one image.  equalize_adapthist(..., volumetric=True) is skimage's call on a 3-D
+array instead: every (D, H, W) volume is one image with 3-D contextual regions.  RECALLED semantics, restated in oracle/skimage_twin.py (numpy,
 array-level) and oracle/mie_oracle.c (per pixel), which agree bit for bit; tests/test_live_pins.py compares all of it
 with the real package when it is importable.
 """
@@ -123,12 +124,18 @@ def _sk_kernel_size(shape, kernel_size):
 
 
 def equalize_adapthist(image: torch.Tensor, kernel_size=None, clip_limit: float = 0.01, nbins: int = 256, *,
-                       out_dtype=None) -> torch.Tensor:
+                       out_dtype=None, volumetric: bool = False) -> torch.Tensor:
     """skimage.exposure.equalize_adapthist on every (H, W) plane of `image` ((H,W), (C,H,W), (B,C,H,W)).
 
     `kernel_size`: size of the contextual regions in PIXELS (int or (rows, cols); default max(dim // 8, 1)) — not a
     grid like kornia's.  `clip_limit` in [0, 1] is a fraction of the region's pixels; `nbins` <= 4096.
-    Returns float64 (float32 for float32 input) in [0, 1] like skimage, or `out_dtype`."""
+    Returns float64 (float32 for float32 input) in [0, 1] like skimage, or `out_dtype`.
+
+    volumetric=True: the last three dimensions of a (D,H,W), (B,D,H,W) or (B,C,D,H,W) tensor form ONE volume, as
+    skimage treats a 3-D array — 3-D contextual regions of `kernel_size` = (kd, kr, kc) voxels (an int is a cube;
+    default max(dim // 8, 1) per axis), a trilinear blend of 8 region mappings, min / max over the whole volume."""
+    if volumetric:
+        return _equalize_adapthist3d(image, kernel_size, clip_limit, nbins, out_dtype)
     require_cuda(image)
     x, n, h, w = as_planes(image)
     kr, kc = _sk_kernel_size((h, w), kernel_size)
@@ -143,6 +150,31 @@ def equalize_adapthist(image: torch.Tensor, kernel_size=None, clip_limit: float 
         check(L.mie_sk_equalize_adapthist(x.data_ptr(), dst.data_ptr(), DTYPE_CODE[x.dtype], _OUT_CODE[dst.dtype], n, h, w,
                                           h * w, w, h * w, w, kr, kc, float(clip_limit), int(nbins), ws.data_ptr(), ws.numel(),
                                           stream_ptr(x.device)))
+    return dst
+
+
+def _equalize_adapthist3d(image: torch.Tensor, kernel_size, clip_limit, nbins, out_dtype) -> torch.Tensor:
+    if not isinstance(image, torch.Tensor):
+        raise TypeError(f"input must be a torch.Tensor, got {type(image)}")
+    if not 3 <= image.dim() <= 5:
+        raise ValueError(f"volumetric=True expects (D,H,W), (B,D,H,W) or (B,C,D,H,W); got shape {tuple(image.shape)}")
+    d, h, w = (int(s) for s in image.shape[-3:])
+    kd, kr, kc = _sk_kernel_size((d, h, w), kernel_size)
+    if kd <= 0 or kr <= 0 or kc <= 0:
+        raise ValueError("kernel_size entries must be positive")
+    if not 0 < int(nbins) <= 4096:
+        raise NotImplementedError("nbins must be in 1..4096")
+    require_cuda(image)
+    x = image.contiguous()
+    n = x.numel() // (d * h * w) if d * h * w else 0
+    dst = _sk_out(x, out_dtype, torch.float32 if x.dtype == torch.float32 else torch.float64)
+    L = lib()
+    ws = torch.empty(max(L.mie_sk_adapthist3d_workspace_bytes(n, d, h, w, kd, kr, kc, int(nbins)), 1), dtype=torch.uint8,
+                     device=x.device)
+    with torch.cuda.device(x.device):
+        check(L.mie_sk_equalize_adapthist3d(x.data_ptr(), dst.data_ptr(), DTYPE_CODE[x.dtype], _OUT_CODE[dst.dtype], n, d, h,
+                                            w, d * h * w, h * w, w, d * h * w, h * w, w, kd, kr, kc, float(clip_limit),
+                                            int(nbins), ws.data_ptr(), ws.numel(), stream_ptr(x.device)))
     return dst
 
 
