@@ -139,6 +139,30 @@ int mie_unsharp_amount(const void* src, void* dst, int src_dtype, int dst_dtype,
                        const float* wx, int kx, const float* wy, int ky, int border,
                        float amount, int clip, float lo, float hi, void* stream);
 
+/* ------------------------------------------------------------------ 3-D Gaussian / unsharp (whole volumes)
+ * skimage.filters.gaussian(image, sigma, mode, truncate) and skimage.filters.unsharp_mask(image, radius, amount) on a
+ * 3-D array: scipy.ndimage.gaussian_filter over all three axes of every (d, h, w) volume of the batch of n.
+ * wx / wy / wz: kx / ky / kz normalised 1-D weights (HOST arrays, copied into kernel parameters); each count odd, 1 ..
+ * MIE_MAX_TAPS (MIE_E_KERNEL otherwise); kz == 1 with weight 1.0 leaves z unfiltered (sigma_z == 0).  Pass order x,
+ * then y, then z, each acc = w[0]*x[0]; acc = fma(w[t], x[t], acc) in tap order — so with kz == 1 the result equals
+ * mie_gaussian2d / mie_unsharp_amount on every plane bit for bit.  Any border mode on any axis length, whatever the
+ * radius (every source index is mirrored / wrapped as often as needed): MIE_E_BORDER for an unknown mode only.
+ * Pixel mapping as mie_gaussian2d; dst_dtype is src_dtype or MIE_F32.  unsharp3d: out = fma(amount, x - blur, x),
+ * clamped to [0, 1] before quantisation when clip != 0; skimage's blur is mode 'reflect' (MIE_BORDER_SYMMETRIC),
+ * truncate 4.  Strides in elements; one launch, no workspace; n == 0 is a no-op.                               */
+int mie_gaussian3d(const void* src, void* dst, int src_dtype, int dst_dtype,
+                   int64_t n, int d, int h, int w,
+                   int64_t src_stride_n, int64_t src_stride_d, int64_t src_stride_h,
+                   int64_t dst_stride_n, int64_t dst_stride_d, int64_t dst_stride_h,
+                   const float* wx, int kx, const float* wy, int ky, const float* wz, int kz,
+                   int border, float lo, float hi, void* stream);
+int mie_unsharp3d(const void* src, void* dst, int src_dtype, int dst_dtype,
+                  int64_t n, int d, int h, int w,
+                  int64_t src_stride_n, int64_t src_stride_d, int64_t src_stride_h,
+                  int64_t dst_stride_n, int64_t dst_stride_d, int64_t dst_stride_h,
+                  const float* wx, int kx, const float* wy, int ky, const float* wz, int kz,
+                  int border, float amount, int clip, float lo, float hi, void* stream);
+
 /* ------------------------------------------------------------------ CLAHE
  * Replaces kornia.enhance.equalize_clahe(input, clip_limit, grid_size)
  * (reference pyproject.toml:8; SURVEY.md §8(a) A1) and, with

@@ -28,6 +28,7 @@ _E_VALUE = {-1, -3, -4, -5, -6, -7, -8, -9, -10, -12}  # -> ValueError
 
 _p, _i, _i64, _f, _d, _sz = C.c_void_p, C.c_int, C.c_int64, C.c_float, C.c_double, C.c_size_t
 _planes = [_i64, _i, _i, _i64, _i64, _i64, _i64]  # n, h, w, ssn, ssh, dsn, dsh
+_volumes = [_i64, _i, _i, _i, _i64, _i64, _i64, _i64, _i64, _i64]  # n, d, h, w, ssn, ssd, ssh, dsn, dsd, dsh
 _taps = [_p, _i, _p, _i]
 
 SIGNATURES = {
@@ -39,6 +40,8 @@ SIGNATURES = {
     "mie_gaussian2d": ([_p, _p, _i, _i, *_planes, *_taps, _i, _f, _f, _p], _i),
     "mie_unsharp": ([_p, _p, _i, _i, *_planes, *_taps, _i, _f, _f, _p], _i),
     "mie_unsharp_amount": ([_p, _p, _i, _i, *_planes, *_taps, _i, _f, _i, _f, _f, _p], _i),
+    "mie_gaussian3d": ([_p, _p, _i, _i, *_volumes, *_taps, *_taps[:2], _i, _f, _f, _p], _i),
+    "mie_unsharp3d": ([_p, _p, _i, _i, *_volumes, *_taps, *_taps[:2], _i, _f, _i, _f, _f, _p], _i),
     "mie_clahe_workspace_bytes": ([_i64, _i, _i, _i, _i], _sz),
     "mie_clahe_hist": ([_p, _i, _i64, _i, _i, _i64, _i64, _i, _i, _i, _f, _f, _p, _p], _i),
     "mie_clahe_luts": ([_p, _i, _i64, _i, _i, _i64, _i64, _i, _i, _d, _i, _f, _f, _p, _p], _i),

@@ -20,6 +20,12 @@ the SAME integer dtype unless out_dtype=torch.float32 — the natural contract f
 arithmetic is fp32 (skimage: float64 for integer input): agreement with scipy.ndimage is ~2e-7 abs on
 [0,1] data (tests/test_skimage_compat.py).
 
+gaussian / unsharp_mask filter every (H, W) plane on its own by default.  With volumetric=True they make skimage's
+call on a 3-D array instead: every (D, H, W) volume of a (D,H,W), (B,D,H,W) or (B,C,D,H,W) tensor is blurred along z
+as well, sigma / radius a scalar or (z, y, x).  One sm_100a kernel (csrc/gauss3d.cu) runs the x, y and z passes in that
+order, so a zero z sigma reproduces the per-plane result bit for bit; agreement with scipy.ndimage.gaussian_filter on
+3-D [0,1] data is to fp32 rounding (tests/test_gaussian3d.py).
+
     equalize_adapthist(image, kernel_size, clip_limit, nbins)  <- skimage.exposure.equalize_adapthist
     equalize_hist(image, nbins, mask)                          <- skimage.exposure.equalize_hist
     denoise_bilateral(image, win_size, sigma_color, sigma_spatial, bins, mode, cval)
@@ -68,26 +74,39 @@ def _mode(mode: str, cval: float) -> str:
 
 
 def gaussian(image: torch.Tensor, sigma=1, *, mode: str = "nearest", cval=0, preserve_range: bool = False,
-             truncate: float = 4.0, channel_axis=None, out=None, value_range=None, out_dtype=None) -> torch.Tensor:
+             truncate: float = 4.0, channel_axis=None, out=None, value_range=None, out_dtype=None,
+             volumetric: bool = False) -> torch.Tensor:
     """skimage.filters.gaussian on 2-D planes ((H,W), (C,H,W), (B,C,H,W): every plane on its own).
     `sigma`: scalar or (sigma_y, sigma_x).  `preserve_range` is accepted for signature compatibility:
-    integer tensors are returned in their own dtype and range either way (see the module docstring)."""
+    integer tensors are returned in their own dtype and range either way (see the module docstring).
+
+    volumetric=True: the last three dimensions of a (D,H,W), (B,D,H,W) or (B,C,D,H,W) tensor form ONE volume, as
+    skimage treats a 3-D array — blurred along z as well.  `sigma`: scalar or (sigma_z, sigma_y, sigma_x); an axis
+    with sigma 0 is not filtered, so sigma (0, s, s) gives the per-plane result bit for bit."""
     if channel_axis is not None:
         raise NotImplementedError("planes are filtered separately; channel_axis is not supported")
     if out is not None:
         raise NotImplementedError("out= is not supported")
+    if volumetric:
+        return _gaussian3d(image, sigma, _mode(mode, cval), truncate, value_range, out_dtype, None)
     sy, sx = (sigma if isinstance(sigma, (tuple, list)) else (sigma, sigma))
     return gaussian_blur2d(image, (_taps(sy, truncate), _taps(sx, truncate)), (float(sy), float(sx)), _mode(mode, cval),
                            value_range=value_range, out_dtype=out_dtype)
 
 
 def unsharp_mask(image: torch.Tensor, radius=1.0, amount=1.0, preserve_range: bool = False, *, channel_axis=None,
-                 value_range=None, out_dtype=None) -> torch.Tensor:
+                 value_range=None, out_dtype=None, volumetric: bool = False) -> torch.Tensor:
     """skimage.filters.unsharp_mask: image + amount * (image - gaussian(image, sigma=radius, mode='reflect')),
     clipped to [0, 1] on the normalised scale unless preserve_range (integer outputs saturate at the dtype's
-    range in both cases)."""
+    range in both cases).
+
+    volumetric=True: every (D, H, W) volume of a (D,H,W), (B,D,H,W) or (B,C,D,H,W) tensor is one 3-D image, blurred
+    over all three axes as skimage does for a 3-D array; `radius`: scalar or (r_z, r_y, r_x)."""
     if channel_axis is not None:
         raise NotImplementedError("planes are filtered separately; channel_axis is not supported")
+    if volumetric:
+        return _gaussian3d(image, radius, "symmetric", 4.0, value_range, out_dtype,
+                           (float(amount), 0 if preserve_range else 1))
     require_cuda(image)
     k = _taps(radius, 4.0)
     x, n, h, w = as_planes(image)
@@ -98,6 +117,50 @@ def unsharp_mask(image: torch.Tensor, radius=1.0, amount=1.0, preserve_range: bo
         check(lib().mie_unsharp_amount(x.data_ptr(), dst.data_ptr(), DTYPE_CODE[x.dtype], DTYPE_CODE[dst.dtype], n, h, w,
                                        h * w, w, h * w, w, wk.ctypes.data, k, wk.ctypes.data, k, BORDER["symmetric"],
                                        float(amount), 0 if preserve_range else 1, lo, hi, stream_ptr(x.device)))
+    return dst
+
+
+def _axis_weights(sigma, truncate: float) -> np.ndarray:
+    """1-D weights of one axis of a volume: sigma 0 leaves the axis unfiltered (scipy skips it)."""
+    s = float(sigma)
+    if s < 0.0 or s != s:
+        raise ValueError("sigma must be non-negative")
+    if s == 0.0:
+        return np.ones(1, np.float32)
+    k = _taps(s, truncate)
+    return get_gaussian_kernel1d(k, s)
+
+
+def _check_volume(image) -> None:
+    if not isinstance(image, torch.Tensor):
+        raise TypeError(f"input must be a torch.Tensor, got {type(image)}")
+    if not 3 <= image.dim() <= 5:
+        raise ValueError(f"volumetric=True expects (D,H,W), (B,D,H,W) or (B,C,D,H,W); got shape {tuple(image.shape)}")
+
+
+def _gaussian3d(image: torch.Tensor, sigma, border: str, truncate, value_range, out_dtype, unsharp) -> torch.Tensor:
+    """mie_gaussian3d / mie_unsharp3d (unsharp = (amount, clip)) on every (D, H, W) volume of `image`."""
+    _check_volume(image)
+    if isinstance(sigma, (tuple, list)):
+        if len(sigma) != 3:
+            raise ValueError(f"volumetric=True takes a scalar sigma or (sigma_z, sigma_y, sigma_x); got {sigma!r}")
+        sz, sy, sx = sigma
+    else:
+        sz = sy = sx = sigma
+    wz, wy, wx = (_axis_weights(s, truncate) for s in (sz, sy, sx))
+    require_cuda(image)
+    x = image.contiguous()
+    d, h, w = (int(s) for s in x.shape[-3:])
+    n = x.numel() // (d * h * w) if d * h * w else 0
+    lo, hi = value_range_of(x, value_range)
+    dst = _out_like(x, out_dtype)
+    args = (x.data_ptr(), dst.data_ptr(), DTYPE_CODE[x.dtype], DTYPE_CODE[dst.dtype], n, d, h, w, d * h * w, h * w, w,
+            d * h * w, h * w, w, wx.ctypes.data, wx.size, wy.ctypes.data, wy.size, wz.ctypes.data, wz.size, BORDER[border])
+    with torch.cuda.device(x.device):
+        if unsharp is None:
+            check(lib().mie_gaussian3d(*args, lo, hi, stream_ptr(x.device)))
+        else:
+            check(lib().mie_unsharp3d(*args, unsharp[0], unsharp[1], lo, hi, stream_ptr(x.device)))
     return dst
 
 
