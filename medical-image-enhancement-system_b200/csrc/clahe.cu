@@ -243,9 +243,12 @@ int mie_clahe(const void* src, void* dst, int src_dtype, int dst_dtype, int64_t 
         return clahe16_impl(src, dst, n, h, w, src_stride_n, src_stride_h, dst_stride_n, dst_stride_h, gh, gw,
                             clip_limit, workspace, workspace_bytes, (cudaStream_t)stream);
     }
+    // the destination is validated with the source, before the LUT pass is launched
+    int rc = check_planes(src, dst, n, h, w, src_stride_n, src_stride_h, dst_stride_n, dst_stride_h);
+    if (rc) return rc;
     if (!workspace) return MIE_E_NULL;
     if (workspace_bytes < mie_clahe_workspace_bytes(n, h, w, gh, gw)) return MIE_E_WORKSPACE;
-    int rc = clahe_luts_impl(src, src_dtype, n, h, w, src_stride_n, src_stride_h, gh, gw, clip_limit, semantics, lo,
+    rc = clahe_luts_impl(src, src_dtype, n, h, w, src_stride_n, src_stride_h, gh, gw, clip_limit, semantics, lo,
                              hi, nullptr, (uint8_t*)workspace, (cudaStream_t)stream);
     if (rc) return rc;
     if (semantics == MIE_CLAHE_KORNIA && dst && n > 0) {

@@ -10,6 +10,8 @@
 
 #include "window.cuh"
 
+#include <type_traits>
+
 namespace mie {
 
 // ---------------------------------------------------------------- histogram -> LUT, one WARP per tile
@@ -147,7 +149,25 @@ __device__ __forceinline__ float axis_weight(int y, int T) {
     return __fdiv_rn((float)(T - 1 - r), (float)(T - 1));
 }
 
-template <typename SrcT, typename DstT, bool WIN, bool IDX>
+// The four pixels of PixIO<DstT, false>::store4 (default range), stored one by one: same quantisation, no alignment.
+template <typename DstT>
+__device__ __forceinline__ void store4_scalar(DstT* p, const float* y) {
+    if constexpr (sizeof(DstT) == 4) {
+#pragma unroll
+        for (int k = 0; k < 4; ++k) p[k] = y[k];
+    } else if constexpr (sizeof(DstT) == 2) {
+        const uint32_t m = std::is_same<DstT, int16_t>::value ? 0x80008000u : 0u;   // as Fast<int16_t>::store4
+        const uint32_t a = Fast<uint16_t>::quant2_u16x2(y[0], y[1]) ^ m, b = Fast<uint16_t>::quant2_u16x2(y[2], y[3]) ^ m;
+        p[0] = (DstT)(a & 0xFFFFu); p[1] = (DstT)(a >> 16); p[2] = (DstT)(b & 0xFFFFu); p[3] = (DstT)(b >> 16);
+    } else {
+#pragma unroll
+        for (int k = 0; k < 4; ++k) p[k] = (uint8_t)Fast<uint8_t>::quant(y[k]);
+    }
+}
+
+// VEC_ST: one 4-pixel vector store per row and thread (destination rows 4-pixel aligned); otherwise the same four
+// pixels are stored one by one (a caller's destination crop at any element offset / row stride).
+template <typename SrcT, typename DstT, bool WIN, bool IDX, bool VEC_ST = true>
 __global__ void __launch_bounds__(1024)
 clahe_apply_fast_kernel(ApplyFastArgs a, const uint2* __restrict__ cells, WinCvt cv) {
     constexpr bool INT = sizeof(SrcT) != 4 && !WIN;
@@ -210,7 +230,8 @@ clahe_apply_fast_kernel(ApplyFastArgs a, const uint2* __restrict__ cells, WinCvt
                 y[k] = clahe_px(lds64_(tb + (__byte_perm(bits, 0u, 0x4440) << 3)), wxv[k], wyv);
             }
         }
-        PixIO<DstT, WIN>::store4(dp, y, cv);
+        if constexpr (VEC_ST) PixIO<DstT, WIN>::store4(dp, y, cv);
+        else store4_scalar(dp, y);
     }
 }
 
@@ -330,9 +351,14 @@ int launch_clahe_apply_index(const uint8_t* idx, void* dst, int dd, int64_t n, i
     if (blocks > 2147483647LL) return MIE_E_SHAPE;
     const size_t smem = (size_t)(g.gw + 1) * kBins * 8;
     const WinCvt cv = {};
+    // the vector store needs 4-pixel aligned destination rows; any other legal layout takes scalar stores
+    const int64_t va = 4 * kEsz[dd];
+    const bool vec = ((uintptr_t)dst % va) == 0 && (dsn * kEsz[dd]) % va == 0 && (dsh * kEsz[dd]) % va == 0;
+#define MIE_APPLY_IDX_V(D_, V_)                                                                            \
+    MIE_ENSURE_SMEM((clahe_apply_fast_kernel<uint8_t, D_, false, true, V_>), 80 * 1024);                   \
+    clahe_apply_fast_kernel<uint8_t, D_, false, true, V_><<<(unsigned)blocks, g.w / 4, smem, st>>>(a, (const uint2*)cells, cv)
 #define MIE_APPLY_IDX(D_)                                                                                  \
-    MIE_ENSURE_SMEM((clahe_apply_fast_kernel<uint8_t, D_, false, true>), 80 * 1024);                       \
-    clahe_apply_fast_kernel<uint8_t, D_, false, true><<<(unsigned)blocks, g.w / 4, smem, st>>>(a, (const uint2*)cells, cv)
+    if (vec) { MIE_APPLY_IDX_V(D_, true); } else { MIE_APPLY_IDX_V(D_, false); }
     switch (dd) {
         case MIE_U8: MIE_APPLY_IDX(uint8_t); break;
         case MIE_U16: MIE_APPLY_IDX(uint16_t); break;
@@ -340,6 +366,7 @@ int launch_clahe_apply_index(const uint8_t* idx, void* dst, int dd, int64_t n, i
         default: MIE_APPLY_IDX(float); break;
     }
 #undef MIE_APPLY_IDX
+#undef MIE_APPLY_IDX_V
     return check_launch();
 }
 
