@@ -422,7 +422,7 @@ static int launch_bilateral_packed(int k, const void* src, void* dst, int64_t ss
 int bilateral_impl(const void* src, void* dst, int sd, int dd, int64_t n, int h, int w, int64_t ssn, int64_t ssh,
                    int64_t dsn, int64_t dsh, const float* wspace, int ky, int kx, float sigma_color, int border,
                    float lo, float hi, cudaStream_t st) {
-    int rc = check_planes(src, dst, n, h, w, ssn, ssh, dsn, dsh);
+    int rc = check_planes({src, sd, ssn, ssh}, {dst, dd, dsn, dsh}, n, h, w);
     if (rc) return rc;
     rc = check_dtypes(sd, dd, lo, hi);
     if (rc) return rc;
@@ -453,8 +453,8 @@ int bilateral_impl(const void* src, void* dst, int sd, int dd, int64_t n, int h,
     return check_launch();
 }
 
-int launch_clahe_apply_index(const uint8_t* idx, void* dst, int dd, int64_t n, int64_t dsn, int64_t dsh, const ClaheGeom& g,
-                             const uint8_t* luts, void* cells, cudaStream_t st);   // clahe_fast.cu
+int launch_clahe_apply_index(const uint8_t* idx, const Image& d, int64_t n, const ClaheGeom& g, const uint8_t* luts,
+                             void* cells, cudaStream_t st);   // clahe_fast.cu
 size_t clahe_cells_bytes(int64_t n, int gh, int gw);
 
 static inline size_t bc_align(size_t v) { return (v + 255) & ~(size_t)255; }
@@ -495,7 +495,8 @@ int mie_bilateral_clahe(const void* src, void* dst, int src_dtype, int dst_dtype
                         const float* wspace, int k, float sigma_color, int border, int gh, int gw, double clip_limit,
                         float lo, float hi, int stages, void* workspace, size_t workspace_bytes, void* stream) {
     cudaStream_t st = (cudaStream_t)stream;
-    int rc = check_planes(src, dst, n, h, w, src_stride_n, src_stride_h, dst_stride_n, dst_stride_h);
+    const Image s{src, src_dtype, src_stride_n, src_stride_h}, d{dst, dst_dtype, dst_stride_n, dst_stride_h};
+    int rc = check_planes(s, d, n, h, w);
     if (rc) return rc;
     rc = check_dtypes(src_dtype, dst_dtype, lo, hi);
     if (rc) return rc;
@@ -557,7 +558,7 @@ int mie_bilateral_clahe(const void* src, void* dst, int src_dtype, int dst_dtype
         if (rc) return rc;
     }
     if (stages & 4)     // index plane -> CLAHE blend -> quantise
-        return launch_clahe_apply_index(idx, dst, dst_dtype, n, dst_stride_n, dst_stride_h, g, luts, cells, st);
+        return launch_clahe_apply_index(idx, d, n, g, luts, cells, st);
     return MIE_OK;
 }
 

@@ -260,7 +260,8 @@ int mie_chain_gauss_clahe_unsharp(const void* src, void* dst, int src_dtype, int
                                   int border, float lo, float hi, int stages, void* workspace,
                                   size_t workspace_bytes, void* stream) {
     cudaStream_t st = (cudaStream_t)stream;
-    int rc = check_planes(src, dst, n, h, w, src_stride_n, src_stride_h, dst_stride_n, dst_stride_h);
+    const Image s{src, src_dtype, src_stride_n, src_stride_h}, d{dst, dst_dtype, dst_stride_n, dst_stride_h};
+    int rc = check_planes(s, d, n, h, w);
     if (rc) return rc;
     rc = check_dtypes(src_dtype, dst_dtype, lo, hi);
     if (rc) return rc;
@@ -311,11 +312,10 @@ int mie_chain_gauss_clahe_unsharp(const void* src, void* dst, int src_dtype, int
     a.src = src; a.ssn = src_stride_n; a.ssh = src_stride_h; a.idx = plane; a.luts = luts; a.g = g;
     a.lp = make_lut_params(g, clip_limit, MIE_CLAHE_KORNIA);
     a.border = border; a.lo = lo; a.rg = hi - lo;
-    bool windowed = false;   // integer value_range window (window.cuh)
-    const bool fast_geo = fast_chain_ok(g, src_dtype, dst_dtype, src, src_stride_n, src_stride_h, dst, dst_stride_n,
-                                        dst_stride_h, kgx, kux, border, lo, hi, &windowed);
     WinCvt cv = {};
-    if (windowed) range_mode(src_dtype, lo, hi, &cv);
+    const int mode = fast_chain_mode(g, s, d, kgx, kux, border, lo, hi, &cv);
+    const bool fast = mode >= 0;
+    const WinCvt* win = mode == 1 ? &cv : nullptr;   // integer value_range window (window.cuh)
     ChainBArgs b;
     b.idx = plane; b.luts = luts; b.dst = dst; b.dsn = dst_stride_n; b.dsh = dst_stride_h; b.g = g;
     b.tiles_x = ceil_div(w, kTile); b.tiles_y = ceil_div(h, kTile); b.border = border; b.max_lut_tiles = lut_cap;
@@ -326,11 +326,9 @@ int mie_chain_gauss_clahe_unsharp(const void* src, void* dst, int src_dtype, int
     // block per 64x64 tile).  Measured crossover on B200: ~24 slices of 512x512 (benchmarks/
     // chain_latency_probe.py), i.e. about 1.5 band-blocks per SM.
     const bool enough_bands = n * (int64_t)g.gh >= 222;
-    const bool march = fast_geo && march_chain_ok(g, kgx, kux) &&
+    const bool march = fast && march_chain_ok(g, kgx, kux) &&
                        !(hints & MIE_CHAIN_PREFER_TILES) && (enough_bands || (hints & MIE_CHAIN_PREFER_MARCH)) &&
                        (int64_t)h * src_stride_h * 4 < (1LL << 31);  // 32-bit source-row offsets
-    const bool fast = fast_geo;
-    const WinCvt* win = windowed ? &cv : nullptr;
     if (fast) {
         if (stages & MIE_CHAIN_STAGE_A) {
             rc = march ? launch_chain_a_march(a, src_dtype, tgx, tgy, n, st, win)

@@ -290,31 +290,13 @@ chain_b_fast_kernel(ChainBArgs a, const uint2* __restrict__ cells, AxisWeights a
 }
 
 // ================================================================ host side
-static bool default_range(int dtype, float lo, float hi) {
-    switch (dtype) {
-        case MIE_U8: return lo == 0.0f && hi == 255.0f;
-        case MIE_U16: return lo == 0.0f && hi == 65535.0f;
-        case MIE_I16: return lo == -32768.0f && hi == 32767.0f;
-        default: return true;
-    }
-}
-
-bool fast_chain_ok(const ClaheGeom& g, int sd, int dd, const void* src, int64_t ssn, int64_t ssh, const void* dst,
-                   int64_t dsn, int64_t dsh, int kg, int ku, int border, float lo, float hi, bool* windowed) {
-    static const int esz[4] = {1, 2, 2, 4};
-    if (g.th != kTile || g.tw != kTile || g.hp != g.h || g.wp != g.w) return false;
-    if (kg < 3 || kg > 9 || ku < 3 || ku > 9) return false;
-    if (border == MIE_BORDER_CIRCULAR || border == MIE_BORDER_SYMMETRIC) return false;
-    if (windowed) *windowed = false;
-    if (!default_range(sd, lo, hi) || !default_range(dd, lo, hi)) {
-        WinCvt cv;
-        if (!windowed || range_mode(sd, lo, hi, &cv) != 1) return false;
-        *windowed = true;
-    }
-    // 16-byte aligned rows for the vector loads / stores
-    if (((uintptr_t)src % 16) || ((ssn * esz[sd]) % 16) || ((ssh * esz[sd]) % 16)) return false;
-    if (((uintptr_t)dst % 16) || ((dsn * esz[dd]) % 16) || ((dsh * esz[dd]) % 16)) return false;
-    return true;
+int fast_chain_mode(const ClaheGeom& g, const Image& s, const Image& d, int kg, int ku, int border, float lo, float hi,
+                    WinCvt* cv) {
+    if (g.th != kTile || g.tw != kTile || g.hp != g.h || g.wp != g.w) return -1;
+    if (kg < 3 || kg > 9 || ku < 3 || ku > 9) return -1;
+    if (border == MIE_BORDER_CIRCULAR || border == MIE_BORDER_SYMMETRIC) return -1;
+    if (!s.aligned(16) || !d.aligned(16)) return -1;   // 16-byte aligned rows for the vector loads / stores
+    return range_mode(s.dtype, lo, hi, cv);
 }
 
 template <typename SrcT, bool WIN>

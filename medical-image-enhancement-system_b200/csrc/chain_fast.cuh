@@ -55,12 +55,11 @@ struct ChainBArgs {
 
 struct WinCvt;   // window.cuh
 
-// Defined in chain_fast.cu.  `fast_chain_ok` tells whether the tuned kernels cover the request.
-// `windowed` (optional): set when the range is not the dtype's default but an integer window the windowed
-// conversion of window.cuh can take.
-bool fast_chain_ok(const ClaheGeom& g, int src_dtype, int dst_dtype, const void* src, int64_t ssn, int64_t ssh,
-                   const void* dst, int64_t dsn, int64_t dsh, int kg, int ku, int border, float lo, float hi,
-                   bool* windowed = nullptr);
+// Defined in chain_fast.cu.  `fast_chain_mode` returns -1 when the tuned kernels do not cover the request, else
+// the range mode of window.cuh: 0 for the dtype's default range, 1 for an integer window the windowed conversion
+// can take (*cv filled in).  The destination dtype is the source's or float32.
+int fast_chain_mode(const ClaheGeom& g, const Image& s, const Image& d, int kg, int ku, int border, float lo, float hi,
+                    WinCvt* cv);
 int launch_chain_a_fast(const ChainAArgs& a, int src_dtype, const Taps& wx, const Taps& wy, int R, int64_t n,
                         cudaStream_t st, const WinCvt* win = nullptr);
 size_t chain_cells_bytes(int64_t n, int gh, int gw);

@@ -5,19 +5,18 @@
 // (per-warp sub-histograms, warp-uniform fast path for constant regions such as
 // CT air), then clips, redistributes and scans in-block.
 #include "clahe.cuh"
+#include "window.cuh"
 
 namespace mie {
 
 // clahe_fast.cu
-bool clahe_lut_fast_ok(const ClaheGeom& g, int sd, const void* src, int64_t ssn, int64_t ssh, float lo, float hi);
-int launch_clahe_lut_fast(const void* src, int sd, int64_t n, int64_t ssn, int64_t ssh, const ClaheGeom& g,
-                          const LutParams& lp, uint32_t* hist, uint8_t* luts, float lo, float hi, cudaStream_t st);
+int clahe_lut_fast_mode(const ClaheGeom& g, const Image& s, float lo, float hi, WinCvt* cv);
+int launch_clahe_lut_fast(const Image& s, int64_t n, const ClaheGeom& g, const LutParams& lp, uint32_t* hist,
+                          uint8_t* luts, int mode, const WinCvt& cv, cudaStream_t st);
 size_t clahe_cells_bytes(int64_t n, int gh, int gw);
-bool clahe_apply_fast_ok(const ClaheGeom& g, int sd, int dd, const void* src, const void* dst, int64_t ssn,
-                         int64_t ssh, int64_t dsn, int64_t dsh, float lo, float hi);
-int launch_clahe_apply_fast(const void* src, void* dst, int sd, int dd, int64_t n, int64_t ssn, int64_t ssh,
-                            int64_t dsn, int64_t dsh, const ClaheGeom& g, const uint8_t* luts, void* cells,
-                            float lo, float hi, cudaStream_t st);
+int clahe_apply_fast_mode(const ClaheGeom& g, const Image& s, const Image& d, float lo, float hi, WinCvt* cv);
+int launch_clahe_apply_fast(const Image& s, const Image& d, int64_t n, const ClaheGeom& g, const uint8_t* luts,
+                            void* cells, int mode, const WinCvt& cv, cudaStream_t st);
 
 // ---------------------------------------------------------------- LUT kernel
 template <typename SrcT, int SEM>
@@ -121,12 +120,13 @@ clahe_apply_kernel(const SrcT* __restrict__ src, DstT* __restrict__ dst, int64_t
 }
 
 // ---------------------------------------------------------------- host side
-static int clahe_common_checks(const void* src, int sd, int64_t n, int h, int w, int64_t ssn, int64_t ssh, int gh,
-                               int gw, int semantics, float lo, float hi, ClaheGeom* g) {
+static int clahe_common_checks(const Image& s, int64_t n, int h, int w, int gh, int gw, int semantics, float lo, float hi,
+                               ClaheGeom* g) {
+    const int sd = s.dtype;
     if (n < 0 || h <= 0 || w <= 0) return MIE_E_SHAPE;
-    if (n > 0 && !src) return MIE_E_NULL;
+    if (n > 0 && !s.p) return MIE_E_NULL;
     if (!valid_dtype(sd)) return MIE_E_DTYPE;
-    if (ssh < w || (n > 1 && ssn < (int64_t)(h - 1) * ssh + w)) return MIE_E_STRIDE;
+    if (!plane_strides_ok(s, n, h, w)) return MIE_E_STRIDE;
     if (semantics != MIE_CLAHE_KORNIA && semantics != MIE_CLAHE_OPENCV) return MIE_E_UNSUPPORTED;
     if (semantics == MIE_CLAHE_OPENCV && sd != MIE_U8) return MIE_E_UNSUPPORTED;  // uint16: mie_clahe / mie_clahe16_luts
     if (semantics == MIE_CLAHE_KORNIA && sd != MIE_F32 && !(hi > lo)) return MIE_E_RANGE;
@@ -151,14 +151,18 @@ static int launch_lut(const void* src, int64_t n, int64_t ssn, int64_t ssh, cons
 int clahe_luts_impl(const void* src, int sd, int64_t n, int h, int w, int64_t ssn, int64_t ssh, int gh, int gw,
                     double clip_limit, int semantics, float lo, float hi, uint32_t* hist, uint8_t* luts,
                     cudaStream_t st) {
+    const Image s{src, sd, ssn, ssh};
     ClaheGeom g;
-    int rc = clahe_common_checks(src, sd, n, h, w, ssn, ssh, gh, gw, semantics, lo, hi, &g);
+    int rc = clahe_common_checks(s, n, h, w, gh, gw, semantics, lo, hi, &g);
     if (rc) return rc;
     if ((int64_t)g.th * g.tw >= (1 << 24)) return MIE_E_SHAPE;  // counts are carried in fp32-exact range
     const LutParams lp = make_lut_params(g, clip_limit, semantics);
     const float rg = hi - lo;
-    if (semantics == MIE_CLAHE_KORNIA && clahe_lut_fast_ok(g, sd, src, ssn, ssh, lo, hi))
-        return launch_clahe_lut_fast(src, sd, n, ssn, ssh, g, lp, hist, luts, lo, hi, st);
+    if (semantics == MIE_CLAHE_KORNIA) {
+        WinCvt cv = {};
+        const int mode = clahe_lut_fast_mode(g, s, lo, hi, &cv);
+        if (mode >= 0) return launch_clahe_lut_fast(s, n, g, lp, hist, luts, mode, cv, st);
+    }
     MIE_DISPATCH_SRC(sd, return launch_lut<SrcT>(src, n, ssn, ssh, g, lo, rg, lp, semantics, hist, luts, st));
     return MIE_OK;
 }
@@ -167,13 +171,13 @@ int clahe_apply_impl(const void* src, void* dst, int sd, int dd, int64_t n, int 
                      int64_t dsn, int64_t dsh, int gh, int gw, int semantics, float lo, float hi, const uint8_t* luts,
                      cudaStream_t st) {
     ClaheGeom g;
-    int rc = clahe_common_checks(src, sd, n, h, w, ssn, ssh, gh, gw, semantics, lo, hi, &g);
+    int rc = clahe_common_checks({src, sd, ssn, ssh}, n, h, w, gh, gw, semantics, lo, hi, &g);
     if (rc) return rc;
     if (!dst || !luts) return MIE_E_NULL;
     rc = check_dtypes(sd, dd, 0.f, 1.f);
     if (rc) return rc;
     if (semantics == MIE_CLAHE_OPENCV && dd != sd) return MIE_E_DTYPE;
-    if (dsh < w || (n > 1 && dsn < (int64_t)(h - 1) * dsh + w)) return MIE_E_STRIDE;
+    if (!plane_strides_ok({dst, dd, dsn, dsh}, n, h, w)) return MIE_E_STRIDE;
     if (n == 0) return MIE_OK;
     if (n > 65535) return MIE_E_SHAPE;
     const float rg = hi - lo;
@@ -236,31 +240,32 @@ int mie_clahe(const void* src, void* dst, int src_dtype, int dst_dtype, int64_t 
               int64_t src_stride_n, int64_t src_stride_h, int64_t dst_stride_n, int64_t dst_stride_h, int gh, int gw,
               double clip_limit, int semantics, float lo, float hi, void* workspace, size_t workspace_bytes,
               void* stream) {
+    const Image s{src, src_dtype, src_stride_n, src_stride_h}, d{dst, dst_dtype, dst_stride_n, dst_stride_h};
     if (semantics == MIE_CLAHE_OPENCV && src_dtype == MIE_U16) {  // 65 536-bin mode (clahe16.cu)
         if (dst_dtype != MIE_U16) return MIE_E_DTYPE;
-        int rc16 = check_planes(src, dst, n, h, w, src_stride_n, src_stride_h, dst_stride_n, dst_stride_h);
+        int rc16 = check_planes(s, d, n, h, w);
         if (rc16) return rc16;
         return clahe16_impl(src, dst, n, h, w, src_stride_n, src_stride_h, dst_stride_n, dst_stride_h, gh, gw,
                             clip_limit, workspace, workspace_bytes, (cudaStream_t)stream);
     }
     // the destination is validated with the source, before the LUT pass is launched
-    int rc = check_planes(src, dst, n, h, w, src_stride_n, src_stride_h, dst_stride_n, dst_stride_h);
+    int rc = check_planes(s, d, n, h, w);
     if (rc) return rc;
     if (!workspace) return MIE_E_NULL;
     if (workspace_bytes < mie_clahe_workspace_bytes(n, h, w, gh, gw)) return MIE_E_WORKSPACE;
     rc = clahe_luts_impl(src, src_dtype, n, h, w, src_stride_n, src_stride_h, gh, gw, clip_limit, semantics, lo,
                              hi, nullptr, (uint8_t*)workspace, (cudaStream_t)stream);
     if (rc) return rc;
-    if (semantics == MIE_CLAHE_KORNIA && dst && n > 0) {
+    // clahe_luts_impl has validated the source, the range and the geometry; clahe_apply_fast_mode accepts only a
+    // destination dtype of the source's or float32
+    if (semantics == MIE_CLAHE_KORNIA && n > 0 && n <= 65535) {
         ClaheGeom g;
-        if (make_clahe_geom(h, w, gh, gw, semantics, &g) == MIE_OK && check_dtypes(src_dtype, dst_dtype, lo, hi) == MIE_OK &&
-            check_planes(src, dst, n, h, w, src_stride_n, src_stride_h, dst_stride_n, dst_stride_h) == MIE_OK &&
-            n <= 65535 &&
-            clahe_apply_fast_ok(g, src_dtype, dst_dtype, src, dst, src_stride_n, src_stride_h, dst_stride_n,
-                                dst_stride_h, lo, hi))
-            return launch_clahe_apply_fast(src, dst, src_dtype, dst_dtype, n, src_stride_n, src_stride_h, dst_stride_n,
-                                           dst_stride_h, g, (const uint8_t*)workspace,
-                                           (uint8_t*)workspace + clahe_lut_region(n, gh, gw), lo, hi,
+        make_clahe_geom(h, w, gh, gw, semantics, &g);
+        WinCvt cv = {};
+        const int mode = clahe_apply_fast_mode(g, s, d, lo, hi, &cv);
+        if (mode >= 0)
+            return launch_clahe_apply_fast(s, d, n, g, (const uint8_t*)workspace,
+                                           (uint8_t*)workspace + clahe_lut_region(n, gh, gw), mode, cv,
                                            (cudaStream_t)stream);
     }
     return clahe_apply_impl(src, dst, src_dtype, dst_dtype, n, h, w, src_stride_n, src_stride_h, dst_stride_n,

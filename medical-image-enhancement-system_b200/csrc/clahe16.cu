@@ -503,7 +503,7 @@ int clahe16_luts_impl(const void* src, int64_t n, int h, int w, int64_t ssn, int
                       double clip_limit, uint16_t* luts, cudaStream_t st, uint32_t* vmax = nullptr) {
     if (n < 0 || h <= 0 || w <= 0) return MIE_E_SHAPE;
     if (n > 0 && (!src || !luts)) return MIE_E_NULL;
-    if (ssh < w || (n > 1 && ssn < (int64_t)(h - 1) * ssh + w)) return MIE_E_STRIDE;
+    if (!plane_strides_ok({src, MIE_U16, ssn, ssh}, n, h, w)) return MIE_E_STRIDE;
     ClaheGeom g;
     int rc = make_clahe_geom(h, w, gh, gw, MIE_CLAHE_OPENCV, &g);
     if (rc) return rc;

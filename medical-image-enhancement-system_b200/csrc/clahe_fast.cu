@@ -236,38 +236,34 @@ clahe_apply_fast_kernel(ApplyFastArgs a, const uint2* __restrict__ cells, WinCvt
 }
 
 // ---------------------------------------------------------------- host side
-static const int kEsz[4] = {1, 2, 2, 4};
 static bool int_rules_disabled() {   // keep the float conversion of the input (cross-check of the integer bin rules)
     return kernel_policy(MIE_POLICY_CLAHE_FLOAT_RULES);
 }
 static bool fast_disabled() { return kernel_policy(MIE_POLICY_GENERIC_CLAHE); }
 
-bool clahe_lut_fast_ok(const ClaheGeom& g, int sd, const void* src, int64_t ssn, int64_t ssh, float lo, float hi) {
-    if (fast_disabled()) return false;
-    if (g.hp != g.h || g.wp != g.w || (g.tw & 7)) return false;
-    WinCvt cv;
-    if (range_mode(sd, lo, hi, &cv) < 0) return false;
-    if (((uintptr_t)src % 16) || ((ssn * kEsz[sd]) % 16) || ((ssh * kEsz[sd]) % 16)) return false;
-    if (((int64_t)g.tw * kEsz[sd]) % 16) return false;   // tile origins 16-byte aligned for load8
-    return true;
+// The range mode of window.cuh (0, or 1 with *cv filled in) when the tuned LUT kernels cover the request, else -1.
+int clahe_lut_fast_mode(const ClaheGeom& g, const Image& s, float lo, float hi, WinCvt* cv) {
+    if (fast_disabled()) return -1;
+    if (g.hp != g.h || g.wp != g.w || (g.tw & 7)) return -1;
+    if (!s.aligned(16)) return -1;
+    if (((int64_t)g.tw * s.bytes()) % 16) return -1;   // tile origins 16-byte aligned for load8
+    return range_mode(s.dtype, lo, hi, cv);
 }
 
-int launch_clahe_lut_fast(const void* src, int sd, int64_t n, int64_t ssn, int64_t ssh, const ClaheGeom& g,
-                          const LutParams& lp, uint32_t* hist, uint8_t* luts, float lo, float hi, cudaStream_t st) {
+int launch_clahe_lut_fast(const Image& s, int64_t n, const ClaheGeom& g, const LutParams& lp, uint32_t* hist,
+                          uint8_t* luts, int mode, const WinCvt& cv, cudaStream_t st) {
     const int64_t tiles = n * g.gh * g.gw;
     if (tiles == 0) return MIE_OK;
     if (tiles > 2147483647LL) return MIE_E_SHAPE;
-    WinCvt cv = {};
-    const int mode = range_mode(sd, lo, hi, &cv);
-    if (mode < 0) return MIE_E_UNSUPPORTED;   // callers test clahe_lut_fast_ok first
+    const int sd = s.dtype;
     const int wpb = 8;
     const int64_t blocks = (tiles + wpb - 1) / wpb;
 #define MIE_LUT_FAST(WIN_, IDX_)                                                                                  \
     if (tiles < 4 * 148) /* small job: spread every tile over a whole block */                                   \
-        clahe_lut_block_kernel<SrcT, WIN_, IDX_><<<(unsigned)tiles, 256, 0, st>>>((const SrcT*)src, ssn, ssh, g, lp,  \
+        clahe_lut_block_kernel<SrcT, WIN_, IDX_><<<(unsigned)tiles, 256, 0, st>>>((const SrcT*)s.p, s.sn, s.sh, g, lp, \
                                                                                hist, luts, cv);                   \
     else                                                                                                          \
-        clahe_lut_fast_kernel<SrcT, WIN_, IDX_><<<(unsigned)blocks, 32 * wpb, 0, st>>>((const SrcT*)src, ssn, ssh, g, \
+        clahe_lut_fast_kernel<SrcT, WIN_, IDX_><<<(unsigned)blocks, 32 * wpb, 0, st>>>((const SrcT*)s.p, s.sn, s.sh, g, \
                                                                                     lp, hist, luts, tiles, cv)
     if (mode == 1) { MIE_DISPATCH_SRC(sd, MIE_LUT_FAST(true, false)); }
     else if (sd != MIE_F32 && int_rules_ok(sd) && !int_rules_disabled()) { MIE_DISPATCH_SRC(sd, MIE_LUT_FAST(false, true)); }
@@ -278,26 +274,20 @@ int launch_clahe_lut_fast(const void* src, int sd, int64_t n, int64_t ssn, int64
 
 size_t clahe_cells_bytes(int64_t n, int gh, int gw) { return chain_cells_bytes(n, gh, gw); }
 
-bool clahe_apply_fast_ok(const ClaheGeom& g, int sd, int dd, const void* src, const void* dst, int64_t ssn,
-                         int64_t ssh, int64_t dsn, int64_t dsh, float lo, float hi) {
-    if (fast_disabled()) return false;
-    if (g.hp != g.h || g.wp != g.w || (g.tw & 7) || (g.w & 3) || g.w > 4096 || g.gw > 32) return false;
-    if (dd != sd && dd != MIE_F32) return false;
-    WinCvt cv;
-    if (range_mode(sd, lo, hi, &cv) < 0) return false;
-    if (((uintptr_t)src % 16) || ((ssn * kEsz[sd]) % 16) || ((ssh * kEsz[sd]) % 16)) return false;
-    if (((uintptr_t)dst % 16) || ((dsn * kEsz[dd]) % 16) || ((dsh * kEsz[dd]) % 16)) return false;
-    return true;
+// As clahe_lut_fast_mode, for the tuned interpolation kernel.
+int clahe_apply_fast_mode(const ClaheGeom& g, const Image& s, const Image& d, float lo, float hi, WinCvt* cv) {
+    if (fast_disabled()) return -1;
+    if (g.hp != g.h || g.wp != g.w || (g.tw & 7) || (g.w & 3) || g.w > 4096 || g.gw > 32) return -1;
+    if (d.dtype != s.dtype && d.dtype != MIE_F32) return -1;
+    if (!s.aligned(16) || !d.aligned(16)) return -1;
+    return range_mode(s.dtype, lo, hi, cv);
 }
 
 // luts -> cell tables (in `cells`, clahe_cells_bytes) -> interpolation
-int launch_clahe_apply_fast(const void* src, void* dst, int sd, int dd, int64_t n, int64_t ssn, int64_t ssh,
-                            int64_t dsn, int64_t dsh, const ClaheGeom& g, const uint8_t* luts, void* cells,
-                            float lo, float hi, cudaStream_t st) {
+int launch_clahe_apply_fast(const Image& s, const Image& d, int64_t n, const ClaheGeom& g, const uint8_t* luts,
+                            void* cells, int mode, const WinCvt& cv, cudaStream_t st) {
     if (n == 0) return MIE_OK;
-    WinCvt cv = {};
-    const int mode = range_mode(sd, lo, hi, &cv);
-    if (mode < 0) return MIE_E_UNSUPPORTED;   // callers test clahe_apply_fast_ok first
+    const int sd = s.dtype, dd = d.dtype;
     // small jobs are launch-latency bound (a single 512x512 slice: ~4 us per launch): skip the packing launch
     const bool in_kernel_cells = n * (int64_t)g.gh * g.gw < 4 * 148;
     if (!in_kernel_cells) {
@@ -306,7 +296,7 @@ int launch_clahe_apply_fast(const void* src, void* dst, int sd, int dd, int64_t 
     }
     ApplyFastArgs a;
     a.luts = in_kernel_cells ? luts : nullptr;
-    a.src = src; a.dst = dst; a.ssn = ssn; a.ssh = ssh; a.dsn = dsn; a.dsh = dsh; a.g = g;
+    a.src = s.p; a.dst = d.out(); a.ssn = s.sn; a.ssh = s.sh; a.dsn = d.sn; a.dsh = d.sh; a.g = g;
     int rows = g.th / 2;                        // rows of a block stay inside one cell row
     for (int d = 32; d >= 1; --d)
         if ((g.th / 2) % d == 0) { rows = d; break; }
@@ -334,14 +324,14 @@ int launch_clahe_apply_fast(const void* src, void* dst, int sd, int dd, int64_t 
 
 // Interpolation pass of the fused bilateral -> CLAHE chain: the source is the 1-byte lookup-index plane (the index IS
 // the byte: Codes<uint8_t>), the destination any pixel dtype in its default range.
-int launch_clahe_apply_index(const uint8_t* idx, void* dst, int dd, int64_t n, int64_t dsn, int64_t dsh, const ClaheGeom& g,
-                             const uint8_t* luts, void* cells, cudaStream_t st) {
+int launch_clahe_apply_index(const uint8_t* idx, const Image& d, int64_t n, const ClaheGeom& g, const uint8_t* luts,
+                             void* cells, cudaStream_t st) {
     if (n == 0) return MIE_OK;
     int rc = launch_pack_cells(luts, cells, n, g.gh, g.gw, st);
     if (rc) return rc;
     ApplyFastArgs a;
     a.luts = nullptr;
-    a.src = idx; a.dst = dst; a.ssn = (int64_t)g.h * g.w; a.ssh = g.w; a.dsn = dsn; a.dsh = dsh; a.g = g;
+    a.src = idx; a.dst = d.out(); a.ssn = (int64_t)g.h * g.w; a.ssh = g.w; a.dsn = d.sn; a.dsh = d.sh; a.g = g;
     int rows = g.th / 2;
     for (int d = 32; d >= 1; --d)
         if ((g.th / 2) % d == 0) { rows = d; break; }
@@ -352,14 +342,13 @@ int launch_clahe_apply_index(const uint8_t* idx, void* dst, int dd, int64_t n, i
     const size_t smem = (size_t)(g.gw + 1) * kBins * 8;
     const WinCvt cv = {};
     // the vector store needs 4-pixel aligned destination rows; any other legal layout takes scalar stores
-    const int64_t va = 4 * kEsz[dd];
-    const bool vec = ((uintptr_t)dst % va) == 0 && (dsn * kEsz[dd]) % va == 0 && (dsh * kEsz[dd]) % va == 0;
+    const bool vec = d.aligned(4 * d.bytes());
 #define MIE_APPLY_IDX_V(D_, V_)                                                                            \
     MIE_ENSURE_SMEM((clahe_apply_fast_kernel<uint8_t, D_, false, true, V_>), 80 * 1024);                   \
     clahe_apply_fast_kernel<uint8_t, D_, false, true, V_><<<(unsigned)blocks, g.w / 4, smem, st>>>(a, (const uint2*)cells, cv)
 #define MIE_APPLY_IDX(D_)                                                                                  \
     if (vec) { MIE_APPLY_IDX_V(D_, true); } else { MIE_APPLY_IDX_V(D_, false); }
-    switch (dd) {
+    switch (d.dtype) {
         case MIE_U8: MIE_APPLY_IDX(uint8_t); break;
         case MIE_U16: MIE_APPLY_IDX(uint16_t); break;
         case MIE_I16: MIE_APPLY_IDX(int16_t); break;

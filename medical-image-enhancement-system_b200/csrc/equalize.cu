@@ -433,14 +433,14 @@ static int equalize_fused_plan(int h, int w, int esz, int* rows_per_cta) {
 }
 
 template <typename SrcT, typename DstT>
-static int launch_equalize_fused(const void* src, void* dst, int64_t n, int h, int w, int64_t ssn, int64_t ssh,
-                                 int64_t dsn, int64_t dsh, float lo, float rg, int cs, int rows, cudaStream_t st) {
+static int launch_equalize_fused(const Image& s, const Image& d, int64_t n, int h, int w, float lo, float rg, int cs,
+                                 int rows, cudaStream_t st) {
     const size_t smem = (size_t)rows * w * sizeof(SrcT);
     // Small planes (148 of them, one per resident cluster, stay L2-resident): no slab at all — the mapping pass reads the
     // pixels a second time through L2, nothing limits the occupancy (8 CTAs per SM instead of 3), and CTAs in different
     // phases hide each other's latencies: 0.0617 ms against 0.0688 ms with slabs on the config-2 batch.
     const size_t plane_bytes = (size_t)h * w * sizeof(SrcT);
-    if (ssh == w && 148 * plane_bytes <= ((size_t)96 << 20) && !kernel_policy(MIE_POLICY_EQUALIZE_SLAB)) {
+    if (s.sh == w && 148 * plane_bytes <= ((size_t)96 << 20) && !kernel_policy(MIE_POLICY_EQUALIZE_SLAB)) {
         int c8 = 8;
         while (c8 > 1 && ceil_div(h, c8) < 8) c8 >>= 1;
         cudaLaunchConfig_t c2 = {};
@@ -452,8 +452,8 @@ static int launch_equalize_fused(const void* src, void* dst, int64_t n, int h, i
         a2[0].id = cudaLaunchAttributeClusterDimension;
         a2[0].val.clusterDim.x = (unsigned)c8; a2[0].val.clusterDim.y = 1; a2[0].val.clusterDim.z = 1;
         c2.attrs = a2; c2.numAttrs = 1;
-        cudaError_t e2 = cudaLaunchKernelEx(&c2, equalize_fused_cluster_kernel<SrcT, DstT, false>, (const SrcT*)src, (DstT*)dst,
-                                            ssn, ssh, dsn, dsh, h, w, ceil_div(h, c8), lo, rg);
+        cudaError_t e2 = cudaLaunchKernelEx(&c2, equalize_fused_cluster_kernel<SrcT, DstT, false>, (const SrcT*)s.p, (DstT*)d.out(),
+                                            s.sn, s.sh, d.sn, d.sh, h, w, ceil_div(h, c8), lo, rg);
         return e2 == cudaSuccess ? check_launch() : (int)e2;
     }
     MIE_ENSURE_SMEM((equalize_fused_cluster_kernel<SrcT, DstT>), 200 * 1024);
@@ -469,21 +469,16 @@ static int launch_equalize_fused(const void* src, void* dst, int64_t n, int h, i
     at[0].val.clusterDim.z = 1;
     cfg.attrs = at;
     cfg.numAttrs = 1;
-    cudaError_t e = cudaLaunchKernelEx(&cfg, equalize_fused_cluster_kernel<SrcT, DstT>, (const SrcT*)src, (DstT*)dst, ssn,
-                                       ssh, dsn, dsh, h, w, rows, lo, rg);
+    cudaError_t e = cudaLaunchKernelEx(&cfg, equalize_fused_cluster_kernel<SrcT, DstT>, (const SrcT*)s.p, (DstT*)d.out(),
+                                       s.sn, s.sh, d.sn, d.sh, h, w, rows, lo, rg);
     return e == cudaSuccess ? check_launch() : (int)e;
 }
 
-static bool equalize_fast_ok(int sd, int dd, const void* src, const void* dst, int w, int64_t ssn, int64_t ssh,
-                             int64_t dsn, int64_t dsh, float lo, float hi) {
-    const bool off = kernel_policy(MIE_POLICY_GENERIC_EQUALIZE);
-    static const int esz[4] = {1, 2, 2, 4};
-    WinCvt cv;
-    if (off || (w & 7) || range_mode(sd, lo, hi, &cv) < 0) return false;
-    const int sa = 8 * esz[sd], da = dd == MIE_F32 ? 16 : 8 * esz[dd];
-    if (((uintptr_t)src % sa) || ((ssn * esz[sd]) % sa) || ((ssh * esz[sd]) % sa)) return false;
-    if (((uintptr_t)dst % da) || ((dsn * esz[dd]) % da) || ((dsh * esz[dd]) % da)) return false;
-    return true;
+// The range mode of window.cuh (0, or 1 with *cv filled in) when the tuned kernels cover the request, else -1.
+static int equalize_fast_mode(const Image& s, const Image& d, int w, float lo, float hi, WinCvt* cv) {
+    if (kernel_policy(MIE_POLICY_GENERIC_EQUALIZE) || (w & 7)) return -1;
+    if (!s.aligned(8 * s.bytes()) || !d.aligned(d.dtype == MIE_F32 ? 16 : 8 * d.bytes())) return -1;
+    return range_mode(s.dtype, lo, hi, cv);
 }
 
 }  // namespace mie
@@ -498,7 +493,8 @@ int mie_equalize(const void* src, void* dst, int src_dtype, int dst_dtype, int64
                  int64_t src_stride_n, int64_t src_stride_h, int64_t dst_stride_n, int64_t dst_stride_h, float lo,
                  float hi, void* workspace, size_t workspace_bytes, void* stream) {
     cudaStream_t st = (cudaStream_t)stream;
-    int rc = check_planes(src, dst, n, h, w, src_stride_n, src_stride_h, dst_stride_n, dst_stride_h);
+    const Image s{src, src_dtype, src_stride_n, src_stride_h}, d{dst, dst_dtype, dst_stride_n, dst_stride_h};
+    int rc = check_planes(s, d, n, h, w);
     if (rc) return rc;
     rc = check_dtypes(src_dtype, dst_dtype, lo, hi);
     if (rc) return rc;
@@ -509,33 +505,30 @@ int mie_equalize(const void* src, void* dst, int src_dtype, int dst_dtype, int64
     if (workspace_bytes < mie_equalize_workspace_bytes(n)) return MIE_E_WORKSPACE;
     EqPlaneState* state = (EqPlaneState*)workspace;
     const float rg = hi - lo;
-    if (equalize_fast_ok(src_dtype, dst_dtype, src, dst, w, src_stride_n, src_stride_h, dst_stride_n, dst_stride_h, lo,
-                         hi)) {
+    WinCvt cv = {};
+    const int mode = equalize_fast_mode(s, d, w, lo, hi, &cv);
+    if (mode >= 0) {
         // ~8 blocks per SM in flight; at least 8 rows per block so the 256 global atomics per block stay rare
         int bpp = (int)((8 * 148 + n - 1) / n);
         int rows = ceil_div(h, bpp < 1 ? 1 : bpp);
         if (rows < 8) rows = 8;
         if (rows > 64) rows = 64;
         dim3 grid((unsigned)ceil_div(h, rows), (unsigned)n);
-        WinCvt cv = {};
         // float planes (kornia's native input) may hold values outside [0, 1] or NaN: they take the range-checked
         // code path of the windowed kernels (PixIO<float, true> is a plain load)
-        const bool win = range_mode(src_dtype, lo, hi, &cv) == 1 || src_dtype == MIE_F32;
+        const bool win = mode == 1 || src_dtype == MIE_F32;
         const bool no_int = kernel_policy(MIE_POLICY_EQUALIZE_FLOAT_RULES);
         const bool idx = !win && !no_int && int_rules_ok(src_dtype);
         // one launch, one HBM round trip, when the integer rules apply and a cluster's shared memory holds the plane
         // (bulk copies move whole rows: 16-byte granularity)
-        static const int esz[4] = {1, 2, 2, 4};
         int frows = 0;
-        const int eb = esz[src_dtype];
-        const int fcs = idx && !kernel_policy(MIE_POLICY_EQUALIZE_THREE_PASS) && ((int64_t)w * eb) % 16 == 0 &&
-                                ((uintptr_t)src % 16) == 0 && (src_stride_n * eb) % 16 == 0 && (src_stride_h * eb) % 16 == 0
-                            ? equalize_fused_plan(h, w, eb, &frows)
+        const int fcs = idx && !kernel_policy(MIE_POLICY_EQUALIZE_THREE_PASS) && ((int64_t)w * s.bytes()) % 16 == 0 &&
+                                s.aligned(16)
+                            ? equalize_fused_plan(h, w, s.bytes(), &frows)
                             : 0;
         if (fcs) {
             MIE_DISPATCH_SRC_DST(src_dtype, dst_dtype,
-                                 return (launch_equalize_fused<SrcT, DstT>(src, dst, n, h, w, src_stride_n, src_stride_h,
-                                                                           dst_stride_n, dst_stride_h, lo, rg, fcs, frows, st)));
+                                 return (launch_equalize_fused<SrcT, DstT>(s, d, n, h, w, lo, rg, fcs, frows, st)));
         }
         cudaError_t me = cudaMemsetAsync(state, 0, (size_t)n * sizeof(EqPlaneState), st);
         if (me != cudaSuccess) return (int)me;

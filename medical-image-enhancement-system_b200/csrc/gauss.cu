@@ -2,15 +2,15 @@
 // Replaces kornia.filters.gaussian_blur2d / kornia.filters.unsharp_mask
 // (reference pyproject.toml:8; SURVEY.md §8(a) A3, A4).
 #include "stencil.cuh"
+#include "window.cuh"
 
 namespace mie {
 
 // gauss_march.cu
-bool gauss_march_ok(const void* src, const void* dst, int sd, int dd, int h, int w, int64_t ssn, int64_t ssh,
-                    int64_t dsn, int64_t dsh, int kx, int ky, int border, float lo, float hi);
-int launch_gauss_march(const void* src, void* dst, int sd, int dd, int64_t n, int h, int w, int64_t ssn, int64_t ssh,
-                       int64_t dsn, int64_t dsh, const Taps& wx, const Taps& wy, int border, int unsharp,
-                       float lo, float hi, cudaStream_t st);
+int gauss_march_mode(const Image& s, const Image& d, int h, int w, int kx, int ky, int border, float lo, float hi,
+                     WinCvt* cv);
+int launch_gauss_march(const Image& s, const Image& d, int64_t n, int h, int w, const Taps& wx, const Taps& wy,
+                       int border, int unsharp, int mode, const WinCvt& cv, cudaStream_t st);
 
 struct GaussArgs {
     const void* src;
@@ -175,7 +175,8 @@ int check_taps(const float* wx, int kx, const float* wy, int ky, int border, int
 int gauss_impl(const void* src, void* dst, int sd, int dd, int64_t n, int h, int w, int64_t ssn, int64_t ssh,
                int64_t dsn, int64_t dsh, const float* wxp, int kx, const float* wyp, int ky, int border, float lo,
                float hi, int unsharp, bool internal, cudaStream_t st, float amount, int clip) {
-    int rc = check_planes(src, dst, n, h, w, ssn, ssh, dsn, dsh);
+    const Image s{src, sd, ssn, ssh}, d{dst, dd, dsn, dsh};
+    int rc = check_planes(s, d, n, h, w);
     if (rc) return rc;
     if (!valid_dtype(sd) || !valid_dtype(dd)) return MIE_E_DTYPE;
     if (!(internal && sd == MIE_F32) && dd != sd && dd != MIE_F32) return MIE_E_DTYPE;
@@ -189,9 +190,11 @@ int gauss_impl(const void* src, void* dst, int sd, int dd, int64_t n, int h, int
         wy.w[i] = i < ky ? wyp[i] : 0.f;
     }
     // common geometry (square 9-tap kernel, W % 128 == 0, H % 64 == 0): marching kernel (gauss_march.cu)
-    if ((!unsharp || (amount == 1.0f && !clip)) &&
-        gauss_march_ok(src, dst, sd, dd, h, w, ssn, ssh, dsn, dsh, kx, ky, border, lo, hi))
-        return launch_gauss_march(src, dst, sd, dd, n, h, w, ssn, ssh, dsn, dsh, wx, wy, border, unsharp, lo, hi, st);
+    if (!unsharp || (amount == 1.0f && !clip)) {
+        WinCvt cv = {};
+        const int mode = gauss_march_mode(s, d, h, w, kx, ky, border, lo, hi, &cv);
+        if (mode >= 0) return launch_gauss_march(s, d, n, h, w, wx, wy, border, unsharp, mode, cv, st);
+    }
     GaussArgs a;
     a.src = src; a.dst = dst; a.ssn = ssn; a.ssh = ssh; a.dsn = dsn; a.dsh = dsh;
     a.h = h; a.w = w; a.tiles_x = a.tiles_y = 0; a.border = border; a.unsharp = unsharp;

@@ -221,13 +221,9 @@ static int gauss3d_impl(const void* src, void* dst, int sd, int dd, int64_t n, i
                         int64_t ssd, int64_t ssh, int64_t dsn, int64_t dsd, int64_t dsh, const float* wxp, int kx,
                         const float* wyp, int ky, const float* wzp, int kz, int border, int unsharp, float amount,
                         int clip, float lo, float hi, cudaStream_t st) {
-    if (n < 0 || d <= 0 || h <= 0 || w <= 0) return MIE_E_SHAPE;
-    if (n > 0 && (!src || !dst)) return MIE_E_NULL;
-    const int64_t src_vol = (int64_t)(d - 1) * ssd + (int64_t)(h - 1) * ssh + w;
-    const int64_t dst_vol = (int64_t)(d - 1) * dsd + (int64_t)(h - 1) * dsh + w;
-    if (ssh < w || (d > 1 && ssd < (int64_t)(h - 1) * ssh + w) || (n > 1 && ssn < src_vol)) return MIE_E_STRIDE;
-    if (dsh < w || (d > 1 && dsd < (int64_t)(h - 1) * dsh + w) || (n > 1 && dsn < dst_vol)) return MIE_E_STRIDE;
-    int rc = check_dtypes(sd, dd, lo, hi);
+    int rc = check_volumes({src, sd, ssn, ssh}, ssd, {dst, dd, dsn, dsh}, dsd, n, d, h, w);
+    if (rc) return rc;
+    rc = check_dtypes(sd, dd, lo, hi);
     if (rc) return rc;
     if (!wxp || !wyp || !wzp) return MIE_E_NULL;
     if (bad_taps(kx) || bad_taps(ky) || bad_taps(kz)) return MIE_E_KERNEL;

@@ -160,21 +160,17 @@ gauss_march_kernel(GaussMarchArgs a, Taps wx, Taps wy, WinCvt cv) {
     }
 }
 
-bool gauss_march_ok(const void* src, const void* dst, int sd, int dd, int h, int w, int64_t ssn, int64_t ssh,
-                    int64_t dsn, int64_t dsh, int kx, int ky, int border, float lo, float hi) {
-    static const int esz[4] = {1, 2, 2, 4};
-    const bool off = kernel_policy(MIE_POLICY_GENERIC_GAUSS);
-    if (off) return false;
-    if (kx != 9 || ky != 9) return false;
-    if (w % 128 != 0 || w > 1024 || h % kTile != 0) return false;
-    if (border == MIE_BORDER_CIRCULAR || border == MIE_BORDER_SYMMETRIC) return false;
-    if (dd != sd && dd != MIE_F32) return false;
-    WinCvt cv;
-    if (range_mode(sd, lo, hi, &cv) < 0) return false;   // default range, or an integer window the host has verified
-    if (((uintptr_t)src % 16) || ((ssn * esz[sd]) % 16) || ((ssh * esz[sd]) % 16)) return false;
-    if (((uintptr_t)dst % 16) || ((dsn * esz[dd]) % 16) || ((dsh * esz[dd]) % 16)) return false;
-    if ((int64_t)h * ssh * 4 >= (1LL << 31)) return false;  // 32-bit source-row offsets
-    return true;
+// The range mode of window.cuh (0, or 1 with *cv filled in) when the marching kernel covers the request, else -1.
+int gauss_march_mode(const Image& s, const Image& d, int h, int w, int kx, int ky, int border, float lo, float hi,
+                     WinCvt* cv) {
+    if (kernel_policy(MIE_POLICY_GENERIC_GAUSS)) return -1;
+    if (kx != 9 || ky != 9) return -1;
+    if (w % 128 != 0 || w > 1024 || h % kTile != 0) return -1;
+    if (border == MIE_BORDER_CIRCULAR || border == MIE_BORDER_SYMMETRIC) return -1;
+    if (d.dtype != s.dtype && d.dtype != MIE_F32) return -1;
+    if (!s.aligned(16) || !d.aligned(16)) return -1;
+    if ((int64_t)h * s.sh * 4 >= (1LL << 31)) return -1;  // 32-bit source-row offsets
+    return range_mode(s.dtype, lo, hi, cv);   // default range, or an integer window the host has verified
 }
 
 template <typename SrcT, typename DstT, int BORDER, bool WIN>
@@ -207,20 +203,16 @@ static int launch_gm(const GaussMarchArgs& a, const Taps& wx, const Taps& wy, in
     }
 }
 
-int launch_gauss_march(const void* src, void* dst, int sd, int dd, int64_t n, int h, int w, int64_t ssn, int64_t ssh,
-                       int64_t dsn, int64_t dsh, const Taps& wx, const Taps& wy, int border, int unsharp,
-                       float lo, float hi, cudaStream_t st) {
-    WinCvt cv = {};
-    const int mode = range_mode(sd, lo, hi, &cv);
-    if (mode < 0) return MIE_E_UNSUPPORTED;   // callers test gauss_march_ok first
+int launch_gauss_march(const Image& s, const Image& d, int64_t n, int h, int w, const Taps& wx, const Taps& wy,
+                       int border, int unsharp, int mode, const WinCvt& cv, cudaStream_t st) {
     GaussMarchArgs a;
-    a.src = src; a.dst = dst; a.ssn = ssn; a.ssh = ssh; a.dsn = dsn; a.dsh = dsh; a.h = h; a.w = w;
+    a.src = s.p; a.dst = d.out(); a.ssn = s.sn; a.ssh = s.sh; a.dsn = d.sn; a.dsh = d.sh; a.h = h; a.w = w;
     const int64_t blocks = n * (h / kTile);
     if (blocks > 2147483647LL) return MIE_E_SHAPE;
     if (mode == 1) {
-        MIE_DISPATCH_SRC_DST(sd, dd, return (launch_gm<SrcT, DstT, true>(a, wx, wy, border, unsharp, (unsigned)blocks, cv, st)));
+        MIE_DISPATCH_SRC_DST(s.dtype, d.dtype, return (launch_gm<SrcT, DstT, true>(a, wx, wy, border, unsharp, (unsigned)blocks, cv, st)));
     } else {
-        MIE_DISPATCH_SRC_DST(sd, dd, return (launch_gm<SrcT, DstT, false>(a, wx, wy, border, unsharp, (unsigned)blocks, cv, st)));
+        MIE_DISPATCH_SRC_DST(s.dtype, d.dtype, return (launch_gm<SrcT, DstT, false>(a, wx, wy, border, unsharp, (unsigned)blocks, cv, st)));
     }
     return MIE_OK;
 }

@@ -849,32 +849,28 @@ median3x3_f32_kernel(const float* __restrict__ src, float* __restrict__ dst, int
     }
 }
 
-static int try_median3x3_f32(const void* src, void* dst, int64_t n, int h, int w, int64_t ssn, int64_t ssh, int64_t dsn,
-                             int64_t dsh, int border, cudaStream_t st) {
+static int try_median3x3_f32(const Image& s, const Image& d, int64_t n, int h, int w, int border, cudaStream_t st) {
     const bool off = kernel_policy(MIE_POLICY_GENERIC_MEDIAN);
     if (off || (w & 3) || h < 2) return -1;
-    if (((uintptr_t)src % 16) || ((ssn * 4) % 16) || ((ssh * 4) % 16)) return -1;
-    if (((uintptr_t)dst % 16) || ((dsn * 4) % 16) || ((dsh * 4) % 16)) return -1;
+    if (!s.aligned(16) || !d.aligned(16)) return -1;
     const int strips = ceil_div(w, 128);
     int rows = 32;
     while (rows > 8 && n * strips * ceil_div(h, rows) < 8 * 148 * 4) rows >>= 1;
     const int bands = ceil_div(h, rows);
     const int64_t blocks = (n * strips * bands + 7) / 8;
     if (blocks > 2147483647LL) return MIE_E_SHAPE;
-    median3x3_f32_kernel<<<(unsigned)blocks, 256, 0, st>>>((const float*)src, (float*)dst, ssn, ssh, dsn, dsh, n, h, w,
-                                                          strips, bands, rows, border);
+    median3x3_f32_kernel<<<(unsigned)blocks, 256, 0, st>>>((const float*)s.p, (float*)d.out(), s.sn, s.sh, d.sn, d.sh, n,
+                                                          h, w, strips, bands, rows, border);
     return check_launch();
 }
 
 // 0 = launched, < 0 = not applicable (caller falls back to the generic kernel), > 0 = CUDA error
 template <typename T>
-static int try_median_packed(const void* src, void* dst, int64_t n, int h, int w, int64_t ssn, int64_t ssh,
-                                int64_t dsn, int64_t dsh, int border, cudaStream_t st, int k = 3) {
+static int try_median_packed(const Image& s, const Image& d, int64_t n, int h, int w, int border, int k,
+                             cudaStream_t st) {
     const bool off = kernel_policy(MIE_POLICY_GENERIC_MEDIAN);
     if (off || (w & 7) || h < k - 1) return -1;
-    constexpr int esz = (int)sizeof(T), al = 8 * esz;   // one 8-pixel vector per lane and row
-    if (((uintptr_t)src % al) || ((ssn * esz) % al) || ((ssh * esz) % al)) return -1;
-    if (((uintptr_t)dst % al) || ((dsn * esz) % al) || ((dsh * esz) % al)) return -1;
+    if (!s.aligned(8 * sizeof(T)) || !d.aligned(8 * sizeof(T))) return -1;   // one 8-pixel vector per lane and row
     const int strips = ceil_div(w, 256);
     int rows = 32;                                 // 2 halo rows per band: 6 % extra loads
     while (rows > 8 && n * strips * ceil_div(h, rows) < 8 * 148 * 4) rows >>= 1;   // small jobs: more warps
@@ -883,23 +879,24 @@ static int try_median_packed(const void* src, void* dst, int64_t n, int h, int w
     const int64_t blocks = (warps + 7) / 8;
     if (blocks > 2147483647LL) return MIE_E_SHAPE;
     if (k == 5)
-        median5x5_packed_kernel<T><<<(unsigned)blocks, 256, 0, st>>>((const T*)src, (T*)dst, ssn, ssh, dsn, dsh, n, h, w,
-                                                                    strips, bands, rows, border);
+        median5x5_packed_kernel<T><<<(unsigned)blocks, 256, 0, st>>>((const T*)s.p, (T*)d.out(), s.sn, s.sh, d.sn, d.sh, n,
+                                                                    h, w, strips, bands, rows, border);
     else
-        median3x3_packed_kernel<T><<<(unsigned)blocks, 256, 0, st>>>((const T*)src, (T*)dst, ssn, ssh, dsn, dsh, n, h, w,
-                                                                    strips, bands, rows, border);
+        median3x3_packed_kernel<T><<<(unsigned)blocks, 256, 0, st>>>((const T*)s.p, (T*)d.out(), s.sn, s.sh, d.sn, d.sh, n,
+                                                                    h, w, strips, bands, rows, border);
     return check_launch();
 }
 
 template <typename T>
-static int launch_median3d(const void* src, void* dst, int d, int h, int w, int64_t ssd, int64_t ssh, int64_t dsd,
-                           int64_t dsh, const void* lo, const void* hi, int border, cudaStream_t st) {
+static int launch_median3d(const Image& s, const Image& o, int d, int h, int w, const void* lo, const void* hi,
+                           int border, cudaStream_t st) {
+    const void* src = s.p;
+    void* dst = o.out();
+    const int64_t ssd = s.sn, ssh = s.sh, dsd = o.sn, dsh = o.sh;
     const int zchunk = d >= 64 ? 32 : (d >= 16 ? 8 : d);
     if constexpr (sizeof(T) == 2) {
         const bool off = kernel_policy(MIE_POLICY_GENERIC_MEDIAN);
-        const bool words_ok = !(w & 1) && !(ssd & 1) && !(ssh & 1) && !(dsd & 1) && !(dsh & 1) &&
-                              !((uintptr_t)src & 3) && !((uintptr_t)dst & 3) && !((uintptr_t)lo & 3) &&
-                              !((uintptr_t)hi & 3);
+        const bool words_ok = !(w & 1) && s.aligned(4) && o.aligned(4) && !((uintptr_t)lo & 3) && !((uintptr_t)hi & 3);
         if (!off && words_ok) {
             const int tiles_x = ceil_div(w, 64), tiles_y = ceil_div(h, 8);
             dim3 grid((unsigned)(tiles_x * tiles_y), (unsigned)ceil_div(d, zchunk));
@@ -931,25 +928,24 @@ extern "C" {
 int mie_median2d(const void* src, void* dst, int dtype, int64_t n, int h, int w, int64_t src_stride_n,
                  int64_t src_stride_h, int64_t dst_stride_n, int64_t dst_stride_h, int ky, int kx, int border,
                  void* stream) {
-    int rc = check_planes(src, dst, n, h, w, src_stride_n, src_stride_h, dst_stride_n, dst_stride_h);
+    const Image s{src, dtype, src_stride_n, src_stride_h}, d{dst, dtype, dst_stride_n, dst_stride_h};
+    int rc = check_planes(s, d, n, h, w);
     if (rc) return rc;
     if (border != MIE_BORDER_CONSTANT && border != MIE_BORDER_REPLICATE && border != MIE_BORDER_REFLECT &&
         border != MIE_BORDER_SYMMETRIC)
         return MIE_E_BORDER;
     if (ky <= 0 || kx <= 0 || !(ky & 1) || !(kx & 1)) return MIE_E_KERNEL;
     if (n == 0) return MIE_OK;
+    if (!valid_dtype(dtype)) return MIE_E_DTYPE;   // before the tuned paths, which pick their kernel by dtype
     cudaStream_t st = (cudaStream_t)stream;
     if (ky == 3 && kx == 3 && dtype == MIE_F32) {
-        rc = try_median3x3_f32(src, dst, n, h, w, src_stride_n, src_stride_h, dst_stride_n, dst_stride_h, border, st);
+        rc = try_median3x3_f32(s, d, n, h, w, border, st);
         if (rc >= 0) return rc;
     }
     if (ky == kx && (ky == 3 || ky == 5) && dtype != MIE_F32) {   // packed marching kernels (8 / 16-bit pixels)
-        rc = dtype == MIE_U16 ? try_median_packed<uint16_t>(src, dst, n, h, w, src_stride_n, src_stride_h,
-                                                               dst_stride_n, dst_stride_h, border, st, ky)
-           : dtype == MIE_I16 ? try_median_packed<int16_t>(src, dst, n, h, w, src_stride_n, src_stride_h,
-                                                              dst_stride_n, dst_stride_h, border, st, ky)
-                              : try_median_packed<uint8_t>(src, dst, n, h, w, src_stride_n, src_stride_h,
-                                                              dst_stride_n, dst_stride_h, border, st, ky);
+        rc = dtype == MIE_U16   ? try_median_packed<uint16_t>(s, d, n, h, w, border, ky, st)
+             : dtype == MIE_I16 ? try_median_packed<int16_t>(s, d, n, h, w, border, ky, st)
+                                : try_median_packed<uint8_t>(s, d, n, h, w, border, ky, st);
         if (rc >= 0) return rc;
     }
     MIE_DISPATCH_SRC(dtype, return dispatch_median2d<SrcT>(ky, kx, src, dst, n, h, w, src_stride_n, src_stride_h,
@@ -960,13 +956,13 @@ int mie_median2d(const void* src, void* dst, int dtype, int64_t n, int h, int w,
 int mie_median3d(const void* src, void* dst, int dtype, int d, int h, int w, int64_t src_stride_d,
                  int64_t src_stride_h, int64_t dst_stride_d, int64_t dst_stride_h, const void* halo_lo,
                  const void* halo_hi, int border, void* stream) {
-    int rc = check_planes(src, dst, d, h, w, src_stride_d, src_stride_h, dst_stride_d, dst_stride_h);
+    const Image s{src, dtype, src_stride_d, src_stride_h}, o{dst, dtype, dst_stride_d, dst_stride_h};
+    int rc = check_planes(s, o, d, h, w);
     if (rc) return rc;
     if (border != MIE_BORDER_CONSTANT && border != MIE_BORDER_REPLICATE) return MIE_E_BORDER;
     if (d == 0) return MIE_OK;
     cudaStream_t st = (cudaStream_t)stream;
-    MIE_DISPATCH_SRC(dtype, return launch_median3d<SrcT>(src, dst, d, h, w, src_stride_d, src_stride_h, dst_stride_d,
-                                                        dst_stride_h, halo_lo, halo_hi, border, st));
+    MIE_DISPATCH_SRC(dtype, return launch_median3d<SrcT>(s, o, d, h, w, halo_lo, halo_hi, border, st));
     return MIE_OK;
 }
 

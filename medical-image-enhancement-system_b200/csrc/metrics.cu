@@ -266,7 +266,8 @@ size_t mie_metric_workspace_bytes(int64_t n, int h, int w, int ws) {
 int mie_sqdiff_sums(const void* a, const void* b, int dtype, int64_t n, int h, int w, int64_t a_stride_n,
                     int64_t a_stride_h, int64_t b_stride_n, int64_t b_stride_h, double* out, void* workspace,
                     size_t workspace_bytes, void* stream) {
-    int rc = check_planes(a, b, n, h, w, a_stride_n, a_stride_h, b_stride_n, b_stride_h);
+    const Image A{a, dtype, a_stride_n, a_stride_h}, B{b, dtype, b_stride_n, b_stride_h};
+    int rc = check_planes(A, B, n, h, w);
     if (rc) return rc;
     if (!valid_dtype(dtype)) return MIE_E_DTYPE;
     if (n == 0) return MIE_OK;
@@ -277,11 +278,7 @@ int mie_sqdiff_sums(const void* a, const void* b, int dtype, int64_t n, int h, i
     const int rows = sqdiff_rows_per_block(n, h);
     const int count = ceil_div(h, rows);
     dim3 grid((unsigned)count, (unsigned)n);
-    static const int esz_[4] = {1, 2, 2, 4};
-    const int eb = esz_[dtype];
-    const bool vec = dtype != MIE_F32 && ((int64_t)w * eb) % 16 == 0 && ((uintptr_t)a % 16) == 0 && ((uintptr_t)b % 16) == 0 &&
-                     (a_stride_n * eb) % 16 == 0 && (a_stride_h * eb) % 16 == 0 && (b_stride_n * eb) % 16 == 0 &&
-                     (b_stride_h * eb) % 16 == 0;
+    const bool vec = dtype != MIE_F32 && ((int64_t)w * A.bytes()) % 16 == 0 && A.aligned(16) && B.aligned(16);
 #define MIE_SQDIFF(T)                                                                                          \
     if (vec && sizeof(T) != 4)                                                                                 \
         sqdiff_vec_kernel<T><<<grid, 256, 0, st>>>((const T*)a, (const T*)b, a_stride_n, a_stride_h, b_stride_n,   \
@@ -311,7 +308,7 @@ int mie_sqdiff_sums(const void* a, const void* b, int dtype, int64_t n, int h, i
 int mie_ssim_sums(const void* a, const void* b, int dtype, int64_t n, int h, int w, int64_t a_stride_n,
                   int64_t a_stride_h, int64_t b_stride_n, int64_t b_stride_h, int ws, double c1, double c2,
                   double* out, void* workspace, size_t workspace_bytes, void* stream) {
-    int rc = check_planes(a, b, n, h, w, a_stride_n, a_stride_h, b_stride_n, b_stride_h);
+    int rc = check_planes({a, dtype, a_stride_n, a_stride_h}, {b, dtype, b_stride_n, b_stride_h}, n, h, w);
     if (rc) return rc;
     if (!valid_dtype(dtype)) return MIE_E_DTYPE;
     if (ws < 1 || ws > kSsimMaxWs || ws > h || ws > w) return MIE_E_KERNEL;

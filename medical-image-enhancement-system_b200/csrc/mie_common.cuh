@@ -132,18 +132,44 @@ inline int check_launch() {
     return e == cudaSuccess ? MIE_OK : (int)e;
 }
 
-struct PlaneArgs {
-    int64_t n;
-    int h, w;
-    int64_t ssn, ssh, dsn, dsh;
+// One image operand of a C-ABI call: plane i at p + i*sn, row y at + y*sh (strides in elements, include/mie.h).
+// bytes() and aligned() need a valid dtype code.
+struct Image {
+    const void* p;
+    int dtype;
+    int64_t sn, sh;
+    int bytes() const {
+        static const int kEsz[4] = {1, 2, 2, 4};
+        return kEsz[dtype];
+    }
+    // base, plane stride and row stride all multiples of b bytes (vector loads and stores of b bytes)
+    bool aligned(int b) const { return (uintptr_t)p % b == 0 && sn * bytes() % b == 0 && sh * bytes() % b == 0; }
+    void* out() const { return const_cast<void*>(p); }
 };
 
-inline int check_planes(const void* src, const void* dst, int64_t n, int h, int w,
-                        int64_t ssn, int64_t ssh, int64_t dsn, int64_t dsh, bool need_dst = true) {
+// Rows no shorter than the width, and plane i + 1 starting after plane i's last row.
+inline bool plane_strides_ok(const Image& x, int64_t n, int h, int w) {
+    return x.sh >= w && (n <= 1 || x.sn >= (int64_t)(h - 1) * x.sh + w);
+}
+
+inline int check_planes(const Image& s, const Image& d, int64_t n, int h, int w) {
     if (n < 0 || h <= 0 || w <= 0) return MIE_E_SHAPE;
-    if (n > 0 && (!src || (need_dst && !dst))) return MIE_E_NULL;  // empty batches carry null pointers
-    if (ssh < w || (n > 1 && ssn < (int64_t)(h - 1) * ssh + w)) return MIE_E_STRIDE;
-    if (need_dst && (dsh < w || (n > 1 && dsn < (int64_t)(h - 1) * dsh + w))) return MIE_E_STRIDE;
+    if (n > 0 && (!s.p || !d.p)) return MIE_E_NULL;  // empty batches carry null pointers
+    if (!plane_strides_ok(s, n, h, w) || !plane_strides_ok(d, n, h, w)) return MIE_E_STRIDE;
+    return MIE_OK;
+}
+
+// Batches of volumes: sn is the volume stride, slice z of a volume starts at + z*slice_stride.
+inline bool volume_strides_ok(const Image& x, int64_t slice_stride, int64_t n, int depth, int h, int w) {
+    const int64_t slice = (int64_t)(h - 1) * x.sh + w;
+    return x.sh >= w && (depth <= 1 || slice_stride >= slice) &&
+           (n <= 1 || x.sn >= (int64_t)(depth - 1) * slice_stride + slice);
+}
+
+inline int check_volumes(const Image& s, int64_t ssd, const Image& d, int64_t dsd, int64_t n, int depth, int h, int w) {
+    if (n < 0 || depth <= 0 || h <= 0 || w <= 0) return MIE_E_SHAPE;
+    if (n > 0 && (!s.p || !d.p)) return MIE_E_NULL;
+    if (!volume_strides_ok(s, ssd, n, depth, h, w) || !volume_strides_ok(d, dsd, n, depth, h, w)) return MIE_E_STRIDE;
     return MIE_OK;
 }
 

@@ -223,7 +223,7 @@ nlm_march_kernel(const SrcT* __restrict__ src, DstT* __restrict__ dst, int64_t s
 int nlm_impl(const void* src, void* dst, int sd, int dd, int64_t n, int h, int w, int64_t ssn, int64_t ssh,
              int64_t dsn, int64_t dsh, int patch_size, int patch_distance, float hpar, float sigma, float lo, float hi,
              cudaStream_t st) {
-    int rc = check_planes(src, dst, n, h, w, ssn, ssh, dsn, dsh);
+    int rc = check_planes({src, sd, ssn, ssh}, {dst, dd, dsn, dsh}, n, h, w);
     if (rc) return rc;
     rc = check_dtypes(sd, dd, lo, hi);
     if (rc) return rc;
@@ -365,7 +365,7 @@ nlm_slow_kernel(const SrcT* __restrict__ src, DstT* __restrict__ dst, int64_t ss
 static int nlm_slow_impl(const void* src, void* dst, int sd, int dd, int64_t n, int h, int w, int64_t ssn, int64_t ssh,
                          int64_t dsn, int64_t dsh, int patch_size, int patch_distance, double hpar, double sigma, float lo,
                          float hi, cudaStream_t st) {
-    int rc = check_planes(src, dst, n, h, w, ssn, ssh, dsn, dsh);
+    int rc = check_planes({src, sd, ssn, ssh}, {dst, dd, dsn, dsh}, n, h, w);
     if (rc) return rc;
     if (!valid_dtype(sd) || !(dd == sd || dd == MIE_F32 || dd == MIE_F64)) return MIE_E_DTYPE;
     if (sd != MIE_F32 && !(hi > lo)) return MIE_E_RANGE;

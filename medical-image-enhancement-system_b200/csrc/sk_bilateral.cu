@@ -112,7 +112,7 @@ extern "C" int mie_sk_denoise_bilateral(const void* src, void* dst, int src_dtyp
                                         const double* color_luts, const double* range_lut, const int* ranges,
                                         void* stream) {
     cudaStream_t st = (cudaStream_t)stream;
-    int rc = check_planes(src, dst, n, h, w, src_stride_n, src_stride_h, dst_stride_n, dst_stride_h);
+    int rc = check_planes({src, src_dtype, src_stride_n, src_stride_h}, {dst, dst_dtype, dst_stride_n, dst_stride_h}, n, h, w);
     if (rc) return rc;
     if (src_dtype != MIE_U8 && src_dtype != MIE_U16 && src_dtype != MIE_I16) return MIE_E_DTYPE;
     if (dst_dtype != MIE_F32 && dst_dtype != MIE_F64) return MIE_E_DTYPE;

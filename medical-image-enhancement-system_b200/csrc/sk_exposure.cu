@@ -581,7 +581,7 @@ int mie_sk_equalize_adapthist(const void* src, void* dst, int src_dtype, int dst
                               int kr, int kc, double clip_limit, int nbins, void* workspace, size_t workspace_bytes,
                               void* stream) {
     cudaStream_t st = (cudaStream_t)stream;
-    int rc = check_planes(src, dst, n, h, w, src_stride_n, src_stride_h, dst_stride_n, dst_stride_h);
+    int rc = check_planes({src, src_dtype, src_stride_n, src_stride_h}, {dst, dst_dtype, dst_stride_n, dst_stride_h}, n, h, w);
     if (rc) return rc;
     if (!valid_dtype(src_dtype) || (dst_dtype != MIE_F32 && dst_dtype != MIE_F64)) return MIE_E_DTYPE;
     if (kr <= 0 || kc <= 0) return MIE_E_KERNEL;
@@ -646,14 +646,9 @@ int mie_sk_equalize_adapthist3d(const void* src, void* dst, int src_dtype, int d
                                 int64_t dst_stride_n, int64_t dst_stride_d, int64_t dst_stride_h,
                                 int kd, int kr, int kc, double clip_limit, int nbins, void* workspace, size_t workspace_bytes,
                                 void* stream) {
-    if (n < 0 || d <= 0 || h <= 0 || w <= 0) return MIE_E_SHAPE;
-    if (n > 0 && (!src || !dst)) return MIE_E_NULL;
-    const int64_t src_vol = (int64_t)(d - 1) * src_stride_d + (int64_t)(h - 1) * src_stride_h + w;
-    const int64_t dst_vol = (int64_t)(d - 1) * dst_stride_d + (int64_t)(h - 1) * dst_stride_h + w;
-    if (src_stride_h < w || (d > 1 && src_stride_d < (int64_t)(h - 1) * src_stride_h + w) || (n > 1 && src_stride_n < src_vol))
-        return MIE_E_STRIDE;
-    if (dst_stride_h < w || (d > 1 && dst_stride_d < (int64_t)(h - 1) * dst_stride_h + w) || (n > 1 && dst_stride_n < dst_vol))
-        return MIE_E_STRIDE;
+    const int rc = check_volumes({src, src_dtype, src_stride_n, src_stride_h}, src_stride_d,
+                                 {dst, dst_dtype, dst_stride_n, dst_stride_h}, dst_stride_d, n, d, h, w);
+    if (rc) return rc;
     if (!valid_dtype(src_dtype) || (dst_dtype != MIE_F32 && dst_dtype != MIE_F64)) return MIE_E_DTYPE;
     if (kd <= 0 || kr <= 0 || kc <= 0) return MIE_E_KERNEL;
     if (nbins <= 0 || nbins > kSkMaxBins) return MIE_E_UNSUPPORTED;
@@ -719,7 +714,7 @@ int mie_sk_equalize_hist(const void* src, void* dst, int src_dtype, int dst_dtyp
                          int64_t src_stride_n, int64_t src_stride_h, int64_t dst_stride_n, int64_t dst_stride_h,
                          void* workspace, size_t workspace_bytes, void* stream) {
     cudaStream_t st = (cudaStream_t)stream;
-    int rc = check_planes(src, dst, n, h, w, src_stride_n, src_stride_h, dst_stride_n, dst_stride_h);
+    int rc = check_planes({src, src_dtype, src_stride_n, src_stride_h}, {dst, dst_dtype, dst_stride_n, dst_stride_h}, n, h, w);
     if (rc) return rc;
     if (src_dtype != MIE_U8 && src_dtype != MIE_U16 && src_dtype != MIE_I16) return MIE_E_DTYPE;
     if (dst_dtype != MIE_F32 && dst_dtype != MIE_F64) return MIE_E_DTYPE;

@@ -148,6 +148,25 @@ def test_newer_entry_points_reject_bad_arguments_before_any_launch():
                                            65535.0, 3 | 4, fake, 0, None) == 0
 
 
+def test_median2d_rejects_unknown_dtype_codes_before_the_tuned_kernels():
+    """The 3x3 / 5x5 tuned median kernels are chosen by dtype: an unknown code must be refused before that choice,
+    as it is for the generic 7x7 path.  With a GPU the pointers are a real buffer, so a wrongly launched kernel
+    stays inside it."""
+    from mie_b200 import _ffi
+
+    L = _ffi.lib()
+    if torch.cuda.is_available():
+        bufs = [torch.zeros(64 * 64 * 4, dtype=torch.uint8, device="cuda") for _ in range(2)]
+        src, dst = (b.data_ptr() for b in bufs)
+    else:
+        src = dst = 0x10000
+    for dtype in (4, 7, -1):
+        for k in (3, 5, 7):
+            assert L.mie_median2d(src, dst, dtype, 1, 64, 64, 4096, 64, 4096, 64, k, k, 0, None) == -2, (dtype, k)
+    if torch.cuda.is_available():
+        torch.cuda.synchronize()
+
+
 def test_round2_advice_validation_paths():
     """ADVICE round 1: a misaligned workspace is refused (MIE_E_ALIGN) instead of faulting in a 32-bit / 128-bit
     access, and the 65 536-bin CLAHE validates the grid before it enters a division (was SIGFPE through the C ABI)."""
