@@ -371,6 +371,40 @@ int mie_sk_equalize_adapthist3d(const void* src, void* dst, int src_dtype, int d
                                 int64_t dst_stride_n, int64_t dst_stride_d, int64_t dst_stride_h,
                                 int kd, int kr, int kc, double clip_limit, int nbins,
                                 void* workspace, size_t workspace_bytes, void* stream);
+/* mie_sk_denoise_tv_chambolle / mie_sk_denoise_tv_chambolle3d: skimage.restoration.denoise_tv_chambolle(image, weight,
+ * eps, max_num_iter) on every (h, w) plane (ndim 2, tau = 1/4) or every (d, h, w) volume (ndim 3, tau = 1/6) of the
+ * batch; a (1, h, w) volume is therefore not a plane.  src u8 / u16 / i16 are computed in float64 on the img_as_float
+ * scale (unsigned v / max, int16 (2 v + 1) / 65535), src f32 in float32; dst F64 or F32 (rounded once).
+ * RECALLED semantics (upstream _denoise_tv_chambolle_nd; numpy twin tests/sk_tv_chambolle_twin.py), per pass i with
+ * p = 0 on entry to pass 0, array axes a in order, every step one correctly rounded operation (no fma):
+ *   d   = -(p0 + p1 [+ p2]), then d += p_a(x - e_a) where x_a >= 1, axis by axis;  out = image + d (pass 0: out = image)
+ *   g_a = out(x + e_a) - out(x), 0 where x_a = n_a - 1;  norm = sqrt(g0^2 + g1^2 [+ g2^2])
+ *   E   = (sum d^2 + weight * sum norm) / image.size;  p = (p - tau * g_a) / (1 + norm * (tau / weight))
+ *   pass 0 sets E_init = E_previous = E; pass i > 0 stops if |E_previous - E| < eps * E_init, else E_previous = E.
+ * The result is out of the last pass run (its p update is discarded): max_num_iter = 1 returns the float image, and a
+ * constant image (E_init = 0) runs every pass and comes back unchanged.  In float32, tau and tau / weight (a float64
+ * quotient) are rounded to float32 and weight * sum, eps * E_init are float32 products.  The two energy sums are taken
+ * in float64 in a fixed order (numpy sums pairwise); they feed only the stopping test.  Every image stops on its own.
+ * weight must be finite and > 0 (MIE_E_RANGE), max_num_iter >= 1 (MIE_E_SHAPE).  iters: DEVICE int32[n] receiving the
+ * passes run per image, or NULL.  One launch per pass up to max_num_iter - 1 whatever the stopping point (a stopped
+ * image's CTAs return at once), then one finishing launch; no host synchronisation and no allocation: all state lives in
+ * the workspace (>= the query, 256-byte aligned) and is re-initialised by every call, so the call can be captured into
+ * a CUDA graph.  The workspace holds two float copies of p: 2 * ndim * n * voxels * sizeof(float type) bytes plus a
+ * little state. */
+size_t mie_sk_tv_chambolle_workspace_bytes(int64_t n, int h, int w, int src_dtype);
+size_t mie_sk_tv_chambolle3d_workspace_bytes(int64_t n, int d, int h, int w, int src_dtype);
+int mie_sk_denoise_tv_chambolle(const void* src, void* dst, int src_dtype, int dst_dtype,
+                                int64_t n, int h, int w,
+                                int64_t src_stride_n, int64_t src_stride_h,
+                                int64_t dst_stride_n, int64_t dst_stride_h,
+                                double weight, double eps, int max_num_iter, int* iters,
+                                void* workspace, size_t workspace_bytes, void* stream);
+int mie_sk_denoise_tv_chambolle3d(const void* src, void* dst, int src_dtype, int dst_dtype,
+                                  int64_t n, int d, int h, int w,
+                                  int64_t src_stride_n, int64_t src_stride_d, int64_t src_stride_h,
+                                  int64_t dst_stride_n, int64_t dst_stride_d, int64_t dst_stride_h,
+                                  double weight, double eps, int max_num_iter, int* iters,
+                                  void* workspace, size_t workspace_bytes, void* stream);
 size_t mie_sk_equalize_hist_workspace_bytes(int64_t n, int src_dtype);
 int mie_sk_equalize_hist(const void* src, void* dst, int src_dtype, int dst_dtype,
                          int64_t n, int h, int w,

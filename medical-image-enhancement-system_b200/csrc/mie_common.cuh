@@ -55,6 +55,14 @@ struct Px<int16_t> : PxInt<int16_t, -32768, 32767> {
     static constexpr int code = MIE_I16;
 };
 
+// skimage.util.img_as_float of an integer code (float64): unsigned v / max, int16 (2 v + 1) / 65535.
+template <typename T>
+__device__ __forceinline__ double skb_as_float(int v) {
+    if constexpr (sizeof(T) == 1) return __ddiv_rn((double)v, 255.0);
+    else if constexpr (T(-1) > T(0)) return __ddiv_rn((double)v, 65535.0);
+    else return __ddiv_rn(__dadd_rn(__dmul_rn((double)v, 2.0), 1.0), 65535.0);
+}
+
 // ---------------------------------------------------------------- borders
 // Returns the source index for coordinate i of an axis of length n, or -1 for
 // MIE_BORDER_CONSTANT outside the image.  Reflect = mirror without repeating
@@ -87,6 +95,7 @@ __host__ __device__ __forceinline__ int border_index(int i, int n, int mode) {
 }
 
 __host__ __device__ __forceinline__ int ceil_div(int a, int b) { return (a + b - 1) / b; }
+inline size_t align256(size_t v) { return (v + 255) & ~(size_t)255; }
 
 // ---------------------------------------------------------------- CLAHE geometry
 struct ClaheGeom {

@@ -11,13 +11,6 @@
 
 namespace mie {
 
-template <typename T>
-__device__ __forceinline__ double skb_as_float(int v) {
-    if constexpr (sizeof(T) == 1) return __ddiv_rn((double)v, 255.0);
-    else if constexpr (T(-1) > T(0)) return __ddiv_rn((double)v, 65535.0);
-    else return __ddiv_rn(__dadd_rn(__dmul_rn((double)v, 2.0), 1.0), 65535.0);
-}
-
 // mode: 0 constant, 1 edge, 2 symmetric, 3 reflect, 4 wrap (numpy.pad names)
 __device__ __forceinline__ int skb_border(int i, int n, int mode) {
     if (i >= 0 && i < n) return i;

@@ -561,8 +561,6 @@ sk_eqhist_apply_kernel(const T* __restrict__ src, DstT* __restrict__ dst, int64_
     dst[n * dsn + (int64_t)y * dsh + x] = (DstT)__ddiv_rn((double)hh[v - r.mn], total);
 }
 
-static inline size_t align256(size_t v) { return (v + 255) & ~(size_t)255; }
-
 }  // namespace mie
 
 using namespace mie;

@@ -30,12 +30,14 @@ order, so a zero z sigma reproduces the per-plane result bit for bit; agreement 
     equalize_hist(image, nbins, mask)                          <- skimage.exposure.equalize_hist
     denoise_bilateral(image, win_size, sigma_color, sigma_spatial, bins, mode, cval)
                                                                <- skimage.restoration.denoise_bilateral
+    denoise_tv_chambolle(image, weight, eps, max_num_iter)     <- skimage.restoration.denoise_tv_chambolle
 
-These three have different algorithms from their kornia counterparts (SURVEY.md Appendix B3/B4) and their own
-kernels (csrc/sk_exposure.cu, csrc/sk_bilateral.cu).  They keep skimage's numerics — float64 arithmetic and a float64
+These four have different algorithms from their kornia counterparts (SURVEY.md Appendix B3/B4) and their own
+kernels (csrc/sk_exposure.cu, csrc/sk_bilateral.cu, csrc/sk_tv.cu).  They keep skimage's numerics — float64 arithmetic and a float64
 result in [0, 1] for integer images (out_dtype=torch.float32 rounds it once) — and skimage's per-image semantics:
 every (H, W) plane of the input is one image.  equalize_adapthist(..., volumetric=True) is skimage's call on a 3-D
-array instead: every (D, H, W) volume is one image with 3-D contextual regions.  RECALLED semantics, restated in oracle/skimage_twin.py (numpy,
+array instead: every (D, H, W) volume is one image with 3-D contextual regions, and denoise_tv_chambolle(...,
+volumetric=True) runs the 3-D algorithm on every volume.  RECALLED semantics, restated in oracle/skimage_twin.py (numpy,
 array-level) and oracle/mie_oracle.c (per pixel), which agree bit for bit; tests/test_live_pins.py compares all of it
 with the real package when it is importable.
 """
@@ -50,7 +52,7 @@ from ._ffi import BORDER, DTYPE_CODE, MIE_F32, MIE_F64, as_planes, check, lib, r
 from .filters import MAX_TAPS, _out_like, denoise_nl_means, gaussian_blur2d, get_gaussian_kernel1d, median  # noqa: F401
 
 __all__ = ["gaussian", "unsharp_mask", "median", "denoise_nl_means", "SCIPY_MODES", "equalize_adapthist", "equalize_hist",
-           "denoise_bilateral"]
+           "denoise_bilateral", "denoise_tv_chambolle"]
 
 SCIPY_MODES = {"nearest": "replicate", "reflect": "symmetric", "mirror": "reflect", "constant": "constant",
                "wrap": "circular"}
@@ -324,4 +326,53 @@ def denoise_bilateral(image: torch.Tensor, win_size=None, sigma_color=None, sigm
         check(lib().mie_sk_denoise_bilateral(x.data_ptr(), dst.data_ptr(), DTYPE_CODE[x.dtype], _OUT_CODE[dst.dtype], n, h, w,
                                              h * w, w, h * w, w, win_size, int(bins), _PAD_MODES[mode], float(cval),
                                              d_luts.data_ptr(), d_spatial.data_ptr(), ranges.data_ptr(), stream_ptr(x.device)))
+    return dst
+
+
+def denoise_tv_chambolle(image: torch.Tensor, weight: float = 0.1, eps: float = 2e-4, max_num_iter: int = 200, *,
+                         channel_axis=None, out_dtype=None, volumetric: bool = False) -> torch.Tensor:
+    """skimage.restoration.denoise_tv_chambolle on every (H, W) plane of `image` ((H,W), (C,H,W), (B,C,H,W)), each
+    plane one 2-D image with its own energy and stopping point.
+
+    volumetric=True: every (D, H, W) volume of a (D,H,W), (B,D,H,W) or (B,C,D,H,W) tensor is one 3-D image, as skimage
+    treats a 3-D array.  Integer images are computed in float64 on the img_as_float scale, float32 images in float32;
+    returns that float dtype, or `out_dtype`.  The iteration runs on the device with no host synchronisation."""
+    return _denoise_tv_chambolle(image, weight, eps, max_num_iter, channel_axis, out_dtype, volumetric, None)
+
+
+def _denoise_tv_chambolle(image, weight, eps, max_num_iter, channel_axis, out_dtype, volumetric, iters):
+    """denoise_tv_chambolle; `iters`: None or a CUDA int32 tensor of one entry per image receiving the passes run."""
+    if channel_axis is not None:
+        raise NotImplementedError("planes are denoised separately; channel_axis is not supported")
+    if not float(weight) > 0.0 or not math.isfinite(float(weight)):
+        raise ValueError("weight must be a positive finite number")
+    if int(max_num_iter) < 1:
+        raise ValueError("max_num_iter must be at least 1")
+    if volumetric:
+        _check_volume(image)
+    require_cuda(image)
+    L = lib()
+    if volumetric:
+        x = image.contiguous()
+        d, h, w = (int(s) for s in x.shape[-3:])
+        n = x.numel() // (d * h * w) if d * h * w else 0
+        nbytes = L.mie_sk_tv_chambolle3d_workspace_bytes(n, d, h, w, DTYPE_CODE[x.dtype])
+    else:
+        x, n, h, w = as_planes(image)
+        nbytes = L.mie_sk_tv_chambolle_workspace_bytes(n, h, w, DTYPE_CODE[x.dtype])
+    dst = _sk_out(x, out_dtype, torch.float32 if x.dtype == torch.float32 else torch.float64)
+    if iters is not None and (iters.dtype != torch.int32 or iters.numel() != n or iters.device != x.device):
+        raise ValueError(f"iters must be an int32 tensor of {n} entries on {x.device}")
+    ws = torch.empty(max(nbytes, 1), dtype=torch.uint8, device=x.device)
+    it = None if iters is None else iters.data_ptr()
+    with torch.cuda.device(x.device):
+        if volumetric:
+            check(L.mie_sk_denoise_tv_chambolle3d(x.data_ptr(), dst.data_ptr(), DTYPE_CODE[x.dtype], _OUT_CODE[dst.dtype],
+                                                  n, d, h, w, d * h * w, h * w, w, d * h * w, h * w, w, float(weight),
+                                                  float(eps), int(max_num_iter), it, ws.data_ptr(), ws.numel(),
+                                                  stream_ptr(x.device)))
+        else:
+            check(L.mie_sk_denoise_tv_chambolle(x.data_ptr(), dst.data_ptr(), DTYPE_CODE[x.dtype], _OUT_CODE[dst.dtype],
+                                                n, h, w, h * w, w, h * w, w, float(weight), float(eps), int(max_num_iter),
+                                                it, ws.data_ptr(), ws.numel(), stream_ptr(x.device)))
     return dst
