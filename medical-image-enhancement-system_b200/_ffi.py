@@ -65,8 +65,7 @@ SIGNATURES = {
     "mie_sk_adapthist_workspace_bytes": ([_i64, _i, _i, _i, _i, _i], _sz),
     "mie_sk_equalize_adapthist": ([_p, _p, _i, _i, *_planes, _i, _i, _d, _i, _p, _sz, _p], _i),
     "mie_sk_adapthist3d_workspace_bytes": ([_i64, _i, _i, _i, _i, _i, _i, _i], _sz),
-    "mie_sk_equalize_adapthist3d": ([_p, _p, _i, _i, _i64, _i, _i, _i, _i64, _i64, _i64, _i64, _i64, _i64,
-                                     _i, _i, _i, _d, _i, _p, _sz, _p], _i),
+    "mie_sk_equalize_adapthist3d": ([_p, _p, _i, _i, *_volumes, _i, _i, _i, _d, _i, _p, _sz, _p], _i),
     "mie_sk_equalize_hist_workspace_bytes": ([_i64, _i], _sz),
     "mie_sk_equalize_hist": ([_p, _p, _i, _i, *_planes, _p, _sz, _p], _i),
     "mie_sk_denoise_bilateral": ([_p, _p, _i, _i, *_planes, _i, _i, _i, _d, _p, _p, _p, _p], _i),
@@ -150,6 +149,13 @@ def stream_ptr(device: torch.device) -> int:
     return torch.cuda.current_stream(device).cuda_stream
 
 
+def call(device: torch.device, name: str, *args) -> None:
+    """Enqueue ABI entry point `name` on `device`'s current stream: every entry point that launches work takes its
+    stream as the last argument.  A non-zero return code raises (see check)."""
+    with torch.cuda.device(device):
+        check(getattr(lib(), name)(*args, stream_ptr(device)))
+
+
 def require_cuda(t: torch.Tensor, name: str = "input") -> None:
     if not isinstance(t, torch.Tensor):
         raise TypeError(f"{name} must be a torch.Tensor, got {type(t)}")
@@ -196,3 +202,63 @@ def as_planes(t: torch.Tensor):
     h, w = t.shape[-2:]
     n = t.numel() // (h * w) if h * w else 0
     return t, n, h, w
+
+
+def as_volumes(t):
+    """(D,H,W) | (B,D,H,W) | (B,C,D,H,W) -> dense tensor + (n, d, h, w): every (D, H, W) volume is one 3-D image, as
+    skimage treats a 3-D array.  Checks the argument only: the caller checks the device and dtype (require_cuda)."""
+    if not isinstance(t, torch.Tensor):
+        raise TypeError(f"input must be a torch.Tensor, got {type(t)}")
+    if not 3 <= t.dim() <= 5:
+        raise ValueError(f"volumetric=True expects (D,H,W), (B,D,H,W) or (B,C,D,H,W); got shape {tuple(t.shape)}")
+    t = t.contiguous()
+    d, h, w = (int(s) for s in t.shape[-3:])
+    n = t.numel() // (d * h * w) if d * h * w else 0
+    return t, n, d, h, w
+
+
+def plane_layout(n: int, h: int, w: int) -> tuple:
+    """The `_planes` arguments of n dense (h, w) planes, the destination in the source's layout.  Entry points that
+    read a source only take the first five."""
+    return n, h, w, h * w, w, h * w, w
+
+
+def volume_layout(n: int, d: int, h: int, w: int) -> tuple:
+    """The `_volumes` arguments of n dense (d, h, w) volumes, the destination in the source's layout."""
+    return n, d, h, w, d * h * w, h * w, w, d * h * w, h * w, w
+
+
+def _dtype_names(dtypes) -> str:
+    return " or ".join(str(dt) for dt in dict.fromkeys(dtypes))
+
+
+def new_out(x: torch.Tensor, out_dtype, allowed=None, default=None) -> torch.Tensor:
+    """Output of `x`'s shape on its device in `out_dtype` (None: `default`, itself defaulting to x's dtype), which
+    must be one of `allowed` (default: x's dtype or float32, the rule of the kornia-signature operators)."""
+    allowed = (x.dtype, torch.float32) if allowed is None else allowed
+    dt = (x.dtype if default is None else default) if out_dtype is None else out_dtype
+    if dt not in allowed:
+        raise TypeError(f"out_dtype must be {_dtype_names(allowed)}")
+    return torch.empty(x.shape, dtype=dt, device=x.device)
+
+
+def check_out(x: torch.Tensor, out: torch.Tensor, allowed=None) -> torch.Tensor:
+    """A caller's output for `x`: contiguous, of x's shape, on x's device, dtype one of `allowed` (as in new_out)."""
+    allowed = (x.dtype, torch.float32) if allowed is None else allowed
+    if out.shape != x.shape or not out.is_contiguous() or out.device != x.device or out.dtype not in allowed:
+        raise ValueError(f"out must be a contiguous tensor of the input's shape on its device, dtype "
+                         f"{_dtype_names(allowed)}")
+    return out
+
+
+def use_workspace(device: torch.device, nbytes: int, workspace: torch.Tensor = None) -> torch.Tensor:
+    """The uint8 scratch memory of a call that needs `nbytes`: a fresh buffer, or the caller's `workspace` after
+    checking it.  The kernels use `nbytes` dense bytes from its first byte, store 32-bit words and load 16-byte
+    pieces (MIE_E_ALIGN), so a caller's buffer must be contiguous and 256-byte aligned like a fresh allocation."""
+    if workspace is None:
+        return torch.empty(max(nbytes, 1), dtype=torch.uint8, device=device)
+    if workspace.dtype != torch.uint8 or not workspace.is_contiguous() or workspace.numel() < nbytes or \
+            workspace.device != device or workspace.data_ptr() % 256:
+        raise ValueError(f"workspace must be a contiguous, 256-byte aligned uint8 tensor of >= {nbytes} bytes on the "
+                         "input's device (a fresh torch.empty is; a sliced view such as ws[1:] is not)")
+    return workspace

@@ -10,9 +10,11 @@ from __future__ import annotations
 
 from dataclasses import dataclass
 
+import numpy as np
 import torch
 
-from ._ffi import DTYPE_CODE, as_planes, check, lib, require_cuda, stream_ptr, value_range_of
+from ._ffi import (DTYPE_CODE, as_planes, call, check_out, lib, new_out, plane_layout, require_cuda, use_workspace,
+                   value_range_of)
 from .enhance import _check_clahe_args
 from .filters import _border, _check_kernel, _pair_float, _pair_int, get_gaussian_kernel1d
 
@@ -57,33 +59,15 @@ def enhance_chain(input: torch.Tensor, config: ChainConfig = ChainConfig(), *, o
     require_cuda(input)
     x, n, h, w = as_planes(input)
     lo, hi = value_range_of(x, cfg.value_range)
-    if out is None:
-        dt = x.dtype if out_dtype is None else out_dtype
-        if dt != x.dtype and dt != torch.float32:
-            raise TypeError("out_dtype must be the input dtype or torch.float32")
-        out = torch.empty(x.shape, dtype=dt, device=x.device)
-    elif out.shape != x.shape or not out.is_contiguous() or out.device != x.device or \
-            (out.dtype != x.dtype and out.dtype != torch.float32):
-        raise ValueError("out must be a contiguous tensor of the input's shape on its device (same dtype or float32)")
+    out = new_out(x, out_dtype) if out is None else check_out(x, out)
     gh, gw = int(cfg.grid_size[0]), int(cfg.grid_size[1])
-    L = lib()
-    need = L.mie_chain_workspace_bytes(n, h, w, gh, gw)
-    if workspace is None:
-        workspace = torch.empty(max(need, 1), dtype=torch.uint8, device=x.device)
-    elif workspace.dtype != torch.uint8 or workspace.numel() < need or workspace.device != x.device:
-        raise ValueError(f"workspace must be a uint8 tensor of >= {need} bytes on the input's device")
-    elif workspace.data_ptr() % 256 or not workspace.is_contiguous():
-        # the kernels store 32-bit index words and load LUTs / cell tables as 16-byte pieces (MIE_E_ALIGN)
-        raise ValueError("workspace must be contiguous and 256-byte aligned (a fresh torch.empty is; a sliced view "
-                         "such as ws[1:] is not)")
+    workspace = use_workspace(x.device, lib().mie_chain_workspace_bytes(n, h, w, gh, gw), workspace)
     wgx, wgy = get_gaussian_kernel1d(gkx, gsx), get_gaussian_kernel1d(gky, gsy)
     wux, wuy = get_gaussian_kernel1d(ukx, usx), get_gaussian_kernel1d(uky, usy)
-    with torch.cuda.device(x.device):
-        check(L.mie_chain_gauss_clahe_unsharp(
-            x.data_ptr(), out.data_ptr(), DTYPE_CODE[x.dtype], DTYPE_CODE[out.dtype], n, h, w, h * w, w, h * w, w,
-            wgx.ctypes.data, gkx, wgy.ctypes.data, gky, gh, gw, float(cfg.clip_limit),
-            wux.ctypes.data, ukx, wuy.ctypes.data, uky, _border(cfg.border_type), lo, hi, int(stages),
-            workspace.data_ptr(), workspace.numel(), stream_ptr(x.device)))
+    call(x.device, "mie_chain_gauss_clahe_unsharp", x.data_ptr(), out.data_ptr(), DTYPE_CODE[x.dtype],
+         DTYPE_CODE[out.dtype], *plane_layout(n, h, w), wgx.ctypes.data, gkx, wgy.ctypes.data, gky, gh, gw,
+         float(cfg.clip_limit), wux.ctypes.data, ukx, wuy.ctypes.data, uky, _border(cfg.border_type), lo, hi,
+         int(stages), workspace.data_ptr(), workspace.numel())
     return out
 
 
@@ -108,10 +92,8 @@ class ChainPlan:
             out = torch.empty(input.shape, dtype=dt, device=input.device)
         self.out = out
         gh, gw = int(config.grid_size[0]), int(config.grid_size[1])
-        if workspace is None:  # a stage-2-only plan must be given the workspace its stage-1 twin filled
-            workspace = torch.empty(max(chain_workspace_bytes(n, h, w, (gh, gw)), 1), dtype=torch.uint8,
-                                    device=input.device)
-        self.workspace = workspace
+        # a stage-2-only plan must be given the workspace its stage-1 twin filled
+        self.workspace = use_workspace(input.device, chain_workspace_bytes(n, h, w, (gh, gw)), workspace)
         self._graph = None
         self._direct()  # validates the arguments and performs the one-time kernel attribute setup
         if graph and n > 0:
@@ -204,31 +186,14 @@ def bilateral_clahe(input: torch.Tensor, kernel_size=9, sigma_color=0.1, sigma_s
     sy, sx = _pair_float(sigma_space, "sigma_space")
     x, n, h, w = as_planes(input)
     lo, hi = value_range_of(x, value_range)
-    if out is None:
-        dt = x.dtype if out_dtype is None else out_dtype
-        if dt != x.dtype and dt != torch.float32:
-            raise TypeError("out_dtype must be the input dtype or torch.float32")
-        out = torch.empty(x.shape, dtype=dt, device=x.device)
-    elif out.shape != x.shape or not out.is_contiguous() or out.device != x.device or \
-            (out.dtype != x.dtype and out.dtype != torch.float32):
-        raise ValueError("out must be a contiguous tensor of the input's shape on its device (same dtype or float32)")
+    out = new_out(x, out_dtype) if out is None else check_out(x, out)
     gh, gw = int(grid_size[0]), int(grid_size[1])
-    L = lib()
-    need = L.mie_bilateral_clahe_workspace_bytes(n, h, w, gh, gw)
-    if workspace is None:
-        workspace = torch.empty(max(need, 1), dtype=torch.uint8, device=x.device)
-    elif workspace.dtype != torch.uint8 or workspace.numel() < need or workspace.device != x.device or \
-            workspace.data_ptr() % 256:
-        raise ValueError(f"workspace must be a 256-byte aligned uint8 tensor of >= {need} bytes on the input's device")
-    import numpy as np
-
+    workspace = use_workspace(x.device, lib().mie_bilateral_clahe_workspace_bytes(n, h, w, gh, gw), workspace)
     wsp = np.ascontiguousarray(
         (get_gaussian_kernel1d(k, sy)[:, None] * get_gaussian_kernel1d(k, sx)[None, :]).astype(np.float32))
-    with torch.cuda.device(x.device):
-        check(L.mie_bilateral_clahe(x.data_ptr(), out.data_ptr(), DTYPE_CODE[x.dtype], DTYPE_CODE[out.dtype], n, h, w,
-                                    h * w, w, h * w, w, wsp.ctypes.data, k, float(sigma_color), _border(border_type), gh, gw,
-                                    float(clip_limit), lo, hi, int(stages), workspace.data_ptr(), workspace.numel(),
-                                    stream_ptr(x.device)))
+    call(x.device, "mie_bilateral_clahe", x.data_ptr(), out.data_ptr(), DTYPE_CODE[x.dtype], DTYPE_CODE[out.dtype],
+         *plane_layout(n, h, w), wsp.ctypes.data, k, float(sigma_color), _border(border_type), gh, gw,
+         float(clip_limit), lo, hi, int(stages), workspace.data_ptr(), workspace.numel())
     return out
 
 
@@ -242,8 +207,7 @@ class BilateralClahePlan:
         x, n, h, w = as_planes(input)
         self.out = out if out is not None else torch.empty_like(input)
         grid = kwargs.get("grid_size", (16, 16))
-        self.workspace = torch.empty(max(bilateral_clahe_workspace_bytes(n, h, w, grid), 1), dtype=torch.uint8,
-                                     device=input.device)
+        self.workspace = use_workspace(input.device, bilateral_clahe_workspace_bytes(n, h, w, grid))
 
     def run(self, stages: int = 7) -> torch.Tensor:
         return bilateral_clahe(self.input, out=self.out, workspace=self.workspace, stages=stages, **self.kwargs)

@@ -12,12 +12,10 @@ on the way out.  float32 tensors behave like kornia ([0,1] in, float out).
 """
 from __future__ import annotations
 
-import ctypes as C
-
 import torch
 
-from . import _ffi
-from ._ffi import CLAHE_KORNIA, CLAHE_OPENCV, DTYPE_CODE, as_planes, check, lib, require_cuda, stream_ptr, value_range_of
+from ._ffi import (CLAHE_KORNIA, CLAHE_OPENCV, DTYPE_CODE, as_planes, call, lib, new_out, plane_layout, require_cuda,
+                   use_workspace, value_range_of)
 
 __all__ = ["equalize_clahe", "equalize", "clahe_histograms", "clahe_luts", "clahe_apply", "clahe16_luts"]
 
@@ -43,13 +41,6 @@ def _check_clahe_args(clip_limit, grid_size):
         raise ValueError(f"Input grid_size elements must be positive. Got {grid_size}")
 
 
-def _out_like(x: torch.Tensor, out_dtype) -> torch.Tensor:
-    dt = x.dtype if out_dtype is None else out_dtype
-    if dt != x.dtype and dt != torch.float32:
-        raise TypeError("out_dtype must be the input dtype or torch.float32")
-    return torch.empty(x.shape, dtype=dt, device=x.device)
-
-
 def equalize_clahe(input: torch.Tensor, clip_limit: float = 40.0, grid_size: tuple = (8, 8),
                    slow_and_differentiable: bool = False, *, value_range=None, semantics: str = "kornia",
                    out_dtype=None) -> torch.Tensor:
@@ -66,19 +57,17 @@ def equalize_clahe(input: torch.Tensor, clip_limit: float = 40.0, grid_size: tup
     require_cuda(input)
     x, n, h, w = as_planes(input)
     lo, hi = value_range_of(x, value_range)
-    dst = _out_like(x, out_dtype)
+    dst = new_out(x, out_dtype)
     gh, gw = int(grid_size[0]), int(grid_size[1])
     L = lib()
-    with torch.cuda.device(x.device):
-        if semantics == "opencv" and x.dtype == torch.uint16:
-            per_image = L.mie_clahe16_lut_bytes(gh, gw)
-            ws_bytes = per_image * max(1, min(n, CLAHE16_WORKSPACE_BYTES // max(per_image, 1))) + 256   # + the value bound
-        else:
-            ws_bytes = L.mie_clahe_workspace_bytes(n, h, w, gh, gw)
-        ws = torch.empty(max(ws_bytes, 1), dtype=torch.uint8, device=x.device)
-        check(L.mie_clahe(x.data_ptr(), dst.data_ptr(), DTYPE_CODE[x.dtype], DTYPE_CODE[dst.dtype], n, h, w,
-                          h * w, w, h * w, w, gh, gw, float(clip_limit), _SEMANTICS[semantics], lo, hi,
-                          ws.data_ptr(), ws.numel(), stream_ptr(x.device)))
+    if semantics == "opencv" and x.dtype == torch.uint16:
+        per_image = L.mie_clahe16_lut_bytes(gh, gw)
+        ws_bytes = per_image * max(1, min(n, CLAHE16_WORKSPACE_BYTES // max(per_image, 1))) + 256   # + the value bound
+    else:
+        ws_bytes = L.mie_clahe_workspace_bytes(n, h, w, gh, gw)
+    ws = use_workspace(x.device, ws_bytes)
+    call(x.device, "mie_clahe", x.data_ptr(), dst.data_ptr(), DTYPE_CODE[x.dtype], DTYPE_CODE[dst.dtype],
+         *plane_layout(n, h, w), gh, gw, float(clip_limit), _SEMANTICS[semantics], lo, hi, ws.data_ptr(), ws.numel())
     return dst
 
 
@@ -89,9 +78,8 @@ def clahe_histograms(input: torch.Tensor, grid_size=(8, 8), *, value_range=None,
     lo, hi = value_range_of(x, value_range)
     gh, gw = int(grid_size[0]), int(grid_size[1])
     hist = torch.empty(x.shape[:-2] + (gh, gw, 256), dtype=torch.int32, device=x.device)
-    with torch.cuda.device(x.device):
-        check(lib().mie_clahe_hist(x.data_ptr(), DTYPE_CODE[x.dtype], n, h, w, h * w, w, gh, gw,
-                                   _SEMANTICS[semantics], lo, hi, hist.data_ptr(), stream_ptr(x.device)))
+    call(x.device, "mie_clahe_hist", x.data_ptr(), DTYPE_CODE[x.dtype], *plane_layout(n, h, w)[:5], gh, gw,
+         _SEMANTICS[semantics], lo, hi, hist.data_ptr())
     return hist
 
 
@@ -103,9 +91,8 @@ def clahe_luts(input: torch.Tensor, clip_limit: float = 40.0, grid_size=(8, 8), 
     lo, hi = value_range_of(x, value_range)
     gh, gw = int(grid_size[0]), int(grid_size[1])
     luts = torch.empty(x.shape[:-2] + (gh, gw, 256), dtype=torch.uint8, device=x.device)
-    with torch.cuda.device(x.device):
-        check(lib().mie_clahe_luts(x.data_ptr(), DTYPE_CODE[x.dtype], n, h, w, h * w, w, gh, gw, float(clip_limit),
-                                   _SEMANTICS[semantics], lo, hi, luts.data_ptr(), stream_ptr(x.device)))
+    call(x.device, "mie_clahe_luts", x.data_ptr(), DTYPE_CODE[x.dtype], *plane_layout(n, h, w)[:5], gh, gw,
+         float(clip_limit), _SEMANTICS[semantics], lo, hi, luts.data_ptr())
     return luts
 
 
@@ -117,9 +104,8 @@ def clahe16_luts(input: torch.Tensor, clip_limit: float = 40.0, grid_size=(8, 8)
         raise TypeError("clahe16_luts takes uint16 tensors")
     gh, gw = int(grid_size[0]), int(grid_size[1])
     luts = torch.empty(x.shape[:-2] + (gh, gw, 65536), dtype=torch.uint16, device=x.device)
-    with torch.cuda.device(x.device):
-        check(lib().mie_clahe16_luts(x.data_ptr(), n, h, w, h * w, w, gh, gw, float(clip_limit), luts.data_ptr(),
-                                     stream_ptr(x.device)))
+    call(x.device, "mie_clahe16_luts", x.data_ptr(), *plane_layout(n, h, w)[:5], gh, gw, float(clip_limit),
+         luts.data_ptr())
     return luts
 
 
@@ -133,11 +119,9 @@ def clahe_apply(input: torch.Tensor, luts: torch.Tensor, grid_size=(8, 8), *, va
     luts = luts.contiguous()
     if luts.dtype != torch.uint8 or luts.numel() != n * gh * gw * 256 or luts.device != x.device:
         raise ValueError("luts must be a uint8 tensor of n*gh*gw*256 entries on the input's device")
-    dst = _out_like(x, out_dtype)
-    with torch.cuda.device(x.device):
-        check(lib().mie_clahe_apply(x.data_ptr(), dst.data_ptr(), DTYPE_CODE[x.dtype], DTYPE_CODE[dst.dtype], n, h, w,
-                                    h * w, w, h * w, w, gh, gw, _SEMANTICS[semantics], lo, hi, luts.data_ptr(),
-                                    stream_ptr(x.device)))
+    dst = new_out(x, out_dtype)
+    call(x.device, "mie_clahe_apply", x.data_ptr(), dst.data_ptr(), DTYPE_CODE[x.dtype], DTYPE_CODE[dst.dtype],
+         *plane_layout(n, h, w), gh, gw, _SEMANTICS[semantics], lo, hi, luts.data_ptr())
     return dst
 
 
@@ -146,11 +130,8 @@ def equalize(input: torch.Tensor, *, value_range=None, out_dtype=None) -> torch.
     require_cuda(input)
     x, n, h, w = as_planes(input)
     lo, hi = value_range_of(x, value_range)
-    dst = _out_like(x, out_dtype)
-    L = lib()
-    with torch.cuda.device(x.device):
-        ws_bytes = L.mie_equalize_workspace_bytes(n)
-        ws = torch.empty(max(ws_bytes, 1), dtype=torch.uint8, device=x.device)
-        check(L.mie_equalize(x.data_ptr(), dst.data_ptr(), DTYPE_CODE[x.dtype], DTYPE_CODE[dst.dtype], n, h, w,
-                             h * w, w, h * w, w, lo, hi, ws.data_ptr(), ws.numel(), stream_ptr(x.device)))
+    dst = new_out(x, out_dtype)
+    ws = use_workspace(x.device, lib().mie_equalize_workspace_bytes(n))
+    call(x.device, "mie_equalize", x.data_ptr(), dst.data_ptr(), DTYPE_CODE[x.dtype], DTYPE_CODE[dst.dtype],
+         *plane_layout(n, h, w), lo, hi, ws.data_ptr(), ws.numel())
     return dst

@@ -13,7 +13,8 @@ from __future__ import annotations
 import numpy as np
 import torch
 
-from ._ffi import BORDER, DTYPE_CODE, MIE_F64, as_planes, check, lib, require_cuda, stream_ptr, value_range_of
+from ._ffi import (BORDER, DTYPE_CODE, MIE_F64, as_planes, call, check_out, new_out, plane_layout, require_cuda,
+                   value_range_of)
 
 __all__ = ["get_gaussian_kernel1d", "gaussian_blur2d", "unsharp_mask", "median_blur", "bilateral_blur", "median"]
 
@@ -72,13 +73,6 @@ def _border(border_type: str) -> int:
     return BORDER[border_type]
 
 
-def _out_like(x, out_dtype):
-    dt = x.dtype if out_dtype is None else out_dtype
-    if dt != x.dtype and dt != torch.float32:
-        raise TypeError("out_dtype must be the input dtype or torch.float32")
-    return torch.empty(x.shape, dtype=dt, device=x.device)
-
-
 def _separable(fn_name, input, kernel_size, sigma, border_type, value_range, out_dtype):
     ky, kx = _pair_int(kernel_size, "kernel_size")
     _check_kernel(ky, kx)
@@ -87,12 +81,10 @@ def _separable(fn_name, input, kernel_size, sigma, border_type, value_range, out
     require_cuda(input)
     x, n, h, w = as_planes(input)
     lo, hi = value_range_of(x, value_range)
-    dst = _out_like(x, out_dtype)
+    dst = new_out(x, out_dtype)
     wx, wy = get_gaussian_kernel1d(kx, sx), get_gaussian_kernel1d(ky, sy)
-    with torch.cuda.device(x.device):
-        check(getattr(lib(), fn_name)(x.data_ptr(), dst.data_ptr(), DTYPE_CODE[x.dtype], DTYPE_CODE[dst.dtype],
-                                      n, h, w, h * w, w, h * w, w, wx.ctypes.data, kx, wy.ctypes.data, ky,
-                                      _border(border_type), lo, hi, stream_ptr(x.device)))
+    call(x.device, fn_name, x.data_ptr(), dst.data_ptr(), DTYPE_CODE[x.dtype], DTYPE_CODE[dst.dtype],
+         *plane_layout(n, h, w), wx.ctypes.data, kx, wy.ctypes.data, ky, _border(border_type), lo, hi)
     return dst
 
 
@@ -116,9 +108,8 @@ def median_blur(input: torch.Tensor, kernel_size, *, border_type: str = "constan
     ky, kx = _pair_int(kernel_size, "kernel_size")
     x, n, h, w = as_planes(input)
     dst = torch.empty_like(x)
-    with torch.cuda.device(x.device):
-        check(lib().mie_median2d(x.data_ptr(), dst.data_ptr(), DTYPE_CODE[x.dtype], n, h, w, h * w, w, h * w, w,
-                                 ky, kx, _border(border_type), stream_ptr(x.device)))
+    call(x.device, "mie_median2d", x.data_ptr(), dst.data_ptr(), DTYPE_CODE[x.dtype], *plane_layout(n, h, w), ky, kx,
+         _border(border_type))
     return dst
 
 
@@ -136,13 +127,11 @@ def bilateral_blur(input: torch.Tensor, kernel_size, sigma_color, sigma_space, b
         sigma_color = float(sigma_color.flatten()[0])
     x, n, h, w = as_planes(input)
     lo, hi = value_range_of(x, value_range)
-    dst = _out_like(x, out_dtype)
+    dst = new_out(x, out_dtype)
     wsp = np.ascontiguousarray(
         (get_gaussian_kernel1d(ky, sy)[:, None] * get_gaussian_kernel1d(kx, sx)[None, :]).astype(np.float32))
-    with torch.cuda.device(x.device):
-        check(lib().mie_bilateral(x.data_ptr(), dst.data_ptr(), DTYPE_CODE[x.dtype], DTYPE_CODE[dst.dtype], n, h, w,
-                                  h * w, w, h * w, w, wsp.ctypes.data, ky, kx, float(sigma_color),
-                                  _border(border_type), lo, hi, stream_ptr(x.device)))
+    call(x.device, "mie_bilateral", x.data_ptr(), dst.data_ptr(), DTYPE_CODE[x.dtype], DTYPE_CODE[dst.dtype],
+         *plane_layout(n, h, w), wsp.ctypes.data, ky, kx, float(sigma_color), _border(border_type), lo, hi)
     return dst
 
 
@@ -164,21 +153,14 @@ def denoise_nl_means(image: torch.Tensor, patch_size: int = 7, patch_distance: i
     x, n, hh, ww = as_planes(image)
     lo, hi = value_range_of(x, value_range)
     if not fast_mode:
-        dt = x.dtype if out_dtype is None else out_dtype
-        if dt not in (x.dtype, torch.float32, torch.float64):
-            raise TypeError("out_dtype must be the input dtype, torch.float32 or torch.float64")
-        dst = torch.empty(x.shape, dtype=dt, device=x.device)
-        code = MIE_F64 if dt == torch.float64 else DTYPE_CODE[dt]
-        with torch.cuda.device(x.device):
-            check(lib().mie_nlm_slow(x.data_ptr(), dst.data_ptr(), DTYPE_CODE[x.dtype], code, n, hh, ww,
-                                     hh * ww, ww, hh * ww, ww, int(patch_size), int(patch_distance), float(h),
-                                     float(sigma), lo, hi, stream_ptr(x.device)))
+        dst = new_out(x, out_dtype, (x.dtype, torch.float32, torch.float64))
+        code = MIE_F64 if dst.dtype == torch.float64 else DTYPE_CODE[dst.dtype]
+        call(x.device, "mie_nlm_slow", x.data_ptr(), dst.data_ptr(), DTYPE_CODE[x.dtype], code, *plane_layout(n, hh, ww),
+             int(patch_size), int(patch_distance), float(h), float(sigma), lo, hi)
         return dst
-    dst = _out_like(x, out_dtype)
-    with torch.cuda.device(x.device):
-        check(lib().mie_nlm(x.data_ptr(), dst.data_ptr(), DTYPE_CODE[x.dtype], DTYPE_CODE[dst.dtype], n, hh, ww,
-                            hh * ww, ww, hh * ww, ww, int(patch_size), int(patch_distance), float(h), float(sigma),
-                            lo, hi, stream_ptr(x.device)))
+    dst = new_out(x, out_dtype)
+    call(x.device, "mie_nlm", x.data_ptr(), dst.data_ptr(), DTYPE_CODE[x.dtype], DTYPE_CODE[dst.dtype],
+         *plane_layout(n, hh, ww), int(patch_size), int(patch_distance), float(h), float(sigma), lo, hi)
     return dst
 
 
@@ -207,27 +189,23 @@ def median(image: torch.Tensor, footprint=None, out=None, mode: str = "nearest",
             raise NotImplementedError("only the default all-ones 3^ndim footprint is supported")
     border = BORDER[_MEDIAN_MODES[mode]]
     x = image.contiguous()
-    dst = out if out is not None else torch.empty_like(x)
-    if out is not None and (out.shape != x.shape or out.dtype != x.dtype or not out.is_contiguous()):
-        raise ValueError("out must be a contiguous tensor of the input's shape and dtype")
+    dst = torch.empty_like(x) if out is None else check_out(x, out, (x.dtype,))
     if out is not None and out.untyped_storage().data_ptr() == x.untyped_storage().data_ptr():
         lo, hi = max(out.data_ptr(), x.data_ptr()), min(out.data_ptr() + out.numel() * out.element_size(),
                                                         x.data_ptr() + x.numel() * x.element_size())
         if lo < hi:
             raise ValueError("out must not overlap the input: the median kernels read neighbours they have not written yet")
-    with torch.cuda.device(x.device):
-        if x.dim() == 2:
-            h, w = x.shape
-            check(lib().mie_median2d(x.data_ptr(), dst.data_ptr(), DTYPE_CODE[x.dtype], 1, h, w, h * w, w, h * w, w,
-                                     3, 3, border, stream_ptr(x.device)))
-        else:
-            d, h, w = x.shape
-            for hp in (halo_lo, halo_hi):
-                if hp is not None and (hp.shape != (h, w) or hp.dtype != x.dtype or not hp.is_contiguous()
-                                       or (hp.device != x.device and not (peer_halos and hp.is_cuda))):
-                    raise ValueError("halo planes must be contiguous (H, W) tensors of the volume's dtype on its device")
-            check(lib().mie_median3d(x.data_ptr(), dst.data_ptr(), DTYPE_CODE[x.dtype], d, h, w, h * w, w, h * w, w,
-                                     halo_lo.data_ptr() if halo_lo is not None else None,
-                                     halo_hi.data_ptr() if halo_hi is not None else None, border,
-                                     stream_ptr(x.device)))
+    if x.dim() == 2:
+        call(x.device, "mie_median2d", x.data_ptr(), dst.data_ptr(), DTYPE_CODE[x.dtype], *plane_layout(1, *x.shape),
+             3, 3, border)
+    else:
+        d, h, w = x.shape
+        for hp in (halo_lo, halo_hi):
+            if hp is not None and (hp.shape != (h, w) or hp.dtype != x.dtype or not hp.is_contiguous()
+                                   or (hp.device != x.device and not (peer_halos and hp.is_cuda))):
+                raise ValueError("halo planes must be contiguous (H, W) tensors of the volume's dtype on its device")
+        # one volume of d dense planes: mie_median3d takes (d, h, w) and the plane strides
+        call(x.device, "mie_median3d", x.data_ptr(), dst.data_ptr(), DTYPE_CODE[x.dtype], *plane_layout(d, h, w),
+             halo_lo.data_ptr() if halo_lo is not None else None, halo_hi.data_ptr() if halo_hi is not None else None,
+             border)
     return dst

@@ -16,6 +16,7 @@ from typing import Callable, Optional
 
 import torch
 
+from ._ffi import use_workspace
 from .chain import ChainConfig, chain_workspace_bytes, enhance_chain
 
 __all__ = ["HostSlicePipeline", "HostVolumePipeline", "pin", "enhance_chain_host", "median3d_clahe_host"]
@@ -47,7 +48,7 @@ class HostSlicePipeline:
             self.x = [torch.empty(shape, dtype=dtype, device=self.device) for _ in range(depth)]
             self.y = [torch.empty(shape, dtype=self.out_dtype, device=self.device) for _ in range(depth)]
             ws = chain_workspace_bytes(self.chunk, self.h, self.w, config.grid_size)
-            self.ws = [torch.empty(max(ws, 1), dtype=torch.uint8, device=self.device) for _ in range(depth)]
+            self.ws = [use_workspace(self.device, ws) for _ in range(depth)]
             self.ev_in = [torch.cuda.Event() for _ in range(depth)]
             self.ev_comp = [torch.cuda.Event() for _ in range(depth)]
             self.ev_out = [torch.cuda.Event() for _ in range(depth)]

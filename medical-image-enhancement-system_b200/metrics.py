@@ -15,7 +15,7 @@ from __future__ import annotations
 import numpy as np
 import torch
 
-from ._ffi import DTYPE_CODE, as_planes, check, lib, require_cuda, stream_ptr
+from ._ffi import DTYPE_CODE, as_planes, call, lib, plane_layout, require_cuda, use_workspace
 
 __all__ = ["mse", "rmse", "psnr", "ssim", "mae"]
 
@@ -47,12 +47,10 @@ def _max_of(t: torch.Tensor, MAX):
 
 def _sqdiff_sums(GT, P) -> tuple[np.ndarray, int]:
     a, b, n, h, w = _initial_check(GT, P)
-    L = lib()
-    with torch.cuda.device(a.device):
-        out = torch.empty((max(n, 1), 2), dtype=torch.float64, device=a.device)
-        ws = torch.empty(max(L.mie_metric_workspace_bytes(n, h, w, 0), 1), dtype=torch.uint8, device=a.device)
-        check(L.mie_sqdiff_sums(a.data_ptr(), b.data_ptr(), DTYPE_CODE[a.dtype], n, h, w, h * w, w, h * w, w,
-                                out.data_ptr(), ws.data_ptr(), ws.numel(), stream_ptr(a.device)))
+    out = torch.empty((max(n, 1), 2), dtype=torch.float64, device=a.device)
+    ws = use_workspace(a.device, lib().mie_metric_workspace_bytes(n, h, w, 0))
+    call(a.device, "mie_sqdiff_sums", a.data_ptr(), b.data_ptr(), DTYPE_CODE[a.dtype], *plane_layout(n, h, w),
+         out.data_ptr(), ws.data_ptr(), ws.numel())
     return out[:n].cpu().numpy(), h * w
 
 
@@ -108,13 +106,10 @@ def ssim(GT: torch.Tensor, P: torch.Tensor, ws: int = 11, K1: float = 0.01, K2: 
     if ws < 1 or ws > min(h, w):
         raise ValueError(f"window size {ws} does not fit a {h}x{w} image")
     c1, c2 = (K1 * mx) ** 2, (K2 * mx) ** 2
-    L = lib()
-    with torch.cuda.device(a.device):
-        out = torch.empty((max(n, 1), 2), dtype=torch.float64, device=a.device)
-        wsb = torch.empty(max(L.mie_metric_workspace_bytes(n, h, w, ws), 1), dtype=torch.uint8, device=a.device)
-        check(L.mie_ssim_sums(a.data_ptr(), b.data_ptr(), DTYPE_CODE[a.dtype], n, h, w, h * w, w, h * w, w, ws,
-                              float(c1), float(c2), out.data_ptr(), wsb.data_ptr(), wsb.numel(),
-                              stream_ptr(a.device)))
+    out = torch.empty((max(n, 1), 2), dtype=torch.float64, device=a.device)
+    wsb = use_workspace(a.device, lib().mie_metric_workspace_bytes(n, h, w, ws))
+    call(a.device, "mie_ssim_sums", a.data_ptr(), b.data_ptr(), DTYPE_CODE[a.dtype], *plane_layout(n, h, w), ws,
+         float(c1), float(c2), out.data_ptr(), wsb.data_ptr(), wsb.numel())
     vals = out[:n].cpu().numpy() / float((h - ws + 1) * (w - ws + 1))
     if per_plane:
         return torch.from_numpy(np.ascontiguousarray(vals[:, 0])), torch.from_numpy(np.ascontiguousarray(vals[:, 1]))

@@ -48,8 +48,9 @@ import math
 import numpy as np
 import torch
 
-from ._ffi import BORDER, DTYPE_CODE, MIE_F32, MIE_F64, as_planes, check, lib, require_cuda, stream_ptr, value_range_of
-from .filters import MAX_TAPS, _out_like, denoise_nl_means, gaussian_blur2d, get_gaussian_kernel1d, median  # noqa: F401
+from ._ffi import (BORDER, DTYPE_CODE, MIE_F32, MIE_F64, as_planes, as_volumes, call, lib, new_out, plane_layout,
+                   require_cuda, use_workspace, value_range_of, volume_layout)
+from .filters import MAX_TAPS, denoise_nl_means, gaussian_blur2d, get_gaussian_kernel1d, median  # noqa: F401
 
 __all__ = ["gaussian", "unsharp_mask", "median", "denoise_nl_means", "SCIPY_MODES", "equalize_adapthist", "equalize_hist",
            "denoise_bilateral", "denoise_tv_chambolle"]
@@ -113,12 +114,11 @@ def unsharp_mask(image: torch.Tensor, radius=1.0, amount=1.0, preserve_range: bo
     k = _taps(radius, 4.0)
     x, n, h, w = as_planes(image)
     lo, hi = value_range_of(x, value_range)
-    dst = _out_like(x, out_dtype)
+    dst = new_out(x, out_dtype)
     wk = get_gaussian_kernel1d(k, float(radius))
-    with torch.cuda.device(x.device):
-        check(lib().mie_unsharp_amount(x.data_ptr(), dst.data_ptr(), DTYPE_CODE[x.dtype], DTYPE_CODE[dst.dtype], n, h, w,
-                                       h * w, w, h * w, w, wk.ctypes.data, k, wk.ctypes.data, k, BORDER["symmetric"],
-                                       float(amount), 0 if preserve_range else 1, lo, hi, stream_ptr(x.device)))
+    call(x.device, "mie_unsharp_amount", x.data_ptr(), dst.data_ptr(), DTYPE_CODE[x.dtype], DTYPE_CODE[dst.dtype],
+         *plane_layout(n, h, w), wk.ctypes.data, k, wk.ctypes.data, k, BORDER["symmetric"], float(amount),
+         0 if preserve_range else 1, lo, hi)
     return dst
 
 
@@ -133,16 +133,9 @@ def _axis_weights(sigma, truncate: float) -> np.ndarray:
     return get_gaussian_kernel1d(k, s)
 
 
-def _check_volume(image) -> None:
-    if not isinstance(image, torch.Tensor):
-        raise TypeError(f"input must be a torch.Tensor, got {type(image)}")
-    if not 3 <= image.dim() <= 5:
-        raise ValueError(f"volumetric=True expects (D,H,W), (B,D,H,W) or (B,C,D,H,W); got shape {tuple(image.shape)}")
-
-
 def _gaussian3d(image: torch.Tensor, sigma, border: str, truncate, value_range, out_dtype, unsharp) -> torch.Tensor:
     """mie_gaussian3d / mie_unsharp3d (unsharp = (amount, clip)) on every (D, H, W) volume of `image`."""
-    _check_volume(image)
+    x, n, d, h, w = as_volumes(image)
     if isinstance(sigma, (tuple, list)):
         if len(sigma) != 3:
             raise ValueError(f"volumetric=True takes a scalar sigma or (sigma_z, sigma_y, sigma_x); got {sigma!r}")
@@ -150,19 +143,15 @@ def _gaussian3d(image: torch.Tensor, sigma, border: str, truncate, value_range, 
     else:
         sz = sy = sx = sigma
     wz, wy, wx = (_axis_weights(s, truncate) for s in (sz, sy, sx))
-    require_cuda(image)
-    x = image.contiguous()
-    d, h, w = (int(s) for s in x.shape[-3:])
-    n = x.numel() // (d * h * w) if d * h * w else 0
+    require_cuda(x)
     lo, hi = value_range_of(x, value_range)
-    dst = _out_like(x, out_dtype)
-    args = (x.data_ptr(), dst.data_ptr(), DTYPE_CODE[x.dtype], DTYPE_CODE[dst.dtype], n, d, h, w, d * h * w, h * w, w,
-            d * h * w, h * w, w, wx.ctypes.data, wx.size, wy.ctypes.data, wy.size, wz.ctypes.data, wz.size, BORDER[border])
-    with torch.cuda.device(x.device):
-        if unsharp is None:
-            check(lib().mie_gaussian3d(*args, lo, hi, stream_ptr(x.device)))
-        else:
-            check(lib().mie_unsharp3d(*args, unsharp[0], unsharp[1], lo, hi, stream_ptr(x.device)))
+    dst = new_out(x, out_dtype)
+    args = (x.data_ptr(), dst.data_ptr(), DTYPE_CODE[x.dtype], DTYPE_CODE[dst.dtype], *volume_layout(n, d, h, w),
+            wx.ctypes.data, wx.size, wy.ctypes.data, wy.size, wz.ctypes.data, wz.size, BORDER[border])
+    if unsharp is None:
+        call(x.device, "mie_gaussian3d", *args, lo, hi)
+    else:
+        call(x.device, "mie_unsharp3d", *args, unsharp[0], unsharp[1], lo, hi)
     return dst
 
 
@@ -171,11 +160,9 @@ _OUT_CODE = {torch.float32: MIE_F32, torch.float64: MIE_F64}
 _PAD_MODES = {"constant": 0, "edge": 1, "symmetric": 2, "reflect": 3, "wrap": 4}
 
 
-def _sk_out(x: torch.Tensor, out_dtype, default):
-    dt = default if out_dtype is None else out_dtype
-    if dt not in _OUT_CODE:
-        raise TypeError("out_dtype must be torch.float32 or torch.float64")
-    return torch.empty(x.shape, dtype=dt, device=x.device)
+def _float_default(x: torch.Tensor) -> torch.dtype:
+    """skimage's result dtype: float32 for float32 images, float64 (img_as_float) for integer images."""
+    return torch.float32 if x.dtype == torch.float32 else torch.float64
 
 
 def _sk_kernel_size(shape, kernel_size):
@@ -208,38 +195,25 @@ def equalize_adapthist(image: torch.Tensor, kernel_size=None, clip_limit: float 
         raise ValueError("kernel_size entries must be positive")
     if not 0 < int(nbins) <= 4096:
         raise NotImplementedError("nbins must be in 1..4096")
-    dst = _sk_out(x, out_dtype, torch.float32 if x.dtype == torch.float32 else torch.float64)
-    L = lib()
-    ws = torch.empty(max(L.mie_sk_adapthist_workspace_bytes(n, h, w, kr, kc, int(nbins)), 1), dtype=torch.uint8, device=x.device)
-    with torch.cuda.device(x.device):
-        check(L.mie_sk_equalize_adapthist(x.data_ptr(), dst.data_ptr(), DTYPE_CODE[x.dtype], _OUT_CODE[dst.dtype], n, h, w,
-                                          h * w, w, h * w, w, kr, kc, float(clip_limit), int(nbins), ws.data_ptr(), ws.numel(),
-                                          stream_ptr(x.device)))
+    dst = new_out(x, out_dtype, _OUT_CODE, _float_default(x))
+    ws = use_workspace(x.device, lib().mie_sk_adapthist_workspace_bytes(n, h, w, kr, kc, int(nbins)))
+    call(x.device, "mie_sk_equalize_adapthist", x.data_ptr(), dst.data_ptr(), DTYPE_CODE[x.dtype], _OUT_CODE[dst.dtype],
+         *plane_layout(n, h, w), kr, kc, float(clip_limit), int(nbins), ws.data_ptr(), ws.numel())
     return dst
 
 
 def _equalize_adapthist3d(image: torch.Tensor, kernel_size, clip_limit, nbins, out_dtype) -> torch.Tensor:
-    if not isinstance(image, torch.Tensor):
-        raise TypeError(f"input must be a torch.Tensor, got {type(image)}")
-    if not 3 <= image.dim() <= 5:
-        raise ValueError(f"volumetric=True expects (D,H,W), (B,D,H,W) or (B,C,D,H,W); got shape {tuple(image.shape)}")
-    d, h, w = (int(s) for s in image.shape[-3:])
+    x, n, d, h, w = as_volumes(image)
     kd, kr, kc = _sk_kernel_size((d, h, w), kernel_size)
     if kd <= 0 or kr <= 0 or kc <= 0:
         raise ValueError("kernel_size entries must be positive")
     if not 0 < int(nbins) <= 4096:
         raise NotImplementedError("nbins must be in 1..4096")
-    require_cuda(image)
-    x = image.contiguous()
-    n = x.numel() // (d * h * w) if d * h * w else 0
-    dst = _sk_out(x, out_dtype, torch.float32 if x.dtype == torch.float32 else torch.float64)
-    L = lib()
-    ws = torch.empty(max(L.mie_sk_adapthist3d_workspace_bytes(n, d, h, w, kd, kr, kc, int(nbins)), 1), dtype=torch.uint8,
-                     device=x.device)
-    with torch.cuda.device(x.device):
-        check(L.mie_sk_equalize_adapthist3d(x.data_ptr(), dst.data_ptr(), DTYPE_CODE[x.dtype], _OUT_CODE[dst.dtype], n, d, h,
-                                            w, d * h * w, h * w, w, d * h * w, h * w, w, kd, kr, kc, float(clip_limit),
-                                            int(nbins), ws.data_ptr(), ws.numel(), stream_ptr(x.device)))
+    require_cuda(x)
+    dst = new_out(x, out_dtype, _OUT_CODE, _float_default(x))
+    ws = use_workspace(x.device, lib().mie_sk_adapthist3d_workspace_bytes(n, d, h, w, kd, kr, kc, int(nbins)))
+    call(x.device, "mie_sk_equalize_adapthist3d", x.data_ptr(), dst.data_ptr(), DTYPE_CODE[x.dtype], _OUT_CODE[dst.dtype],
+         *volume_layout(n, d, h, w), kd, kr, kc, float(clip_limit), int(nbins), ws.data_ptr(), ws.numel())
     return dst
 
 
@@ -253,12 +227,10 @@ def equalize_hist(image: torch.Tensor, nbins: int = 256, mask=None, *, out_dtype
         raise NotImplementedError("equalize_hist is built for integer images (uint8 / uint16 / int16); float images use "
                                   "numpy.histogram's edge rules upstream")
     x, n, h, w = as_planes(image)
-    dst = _sk_out(x, out_dtype, torch.float64)
-    L = lib()
-    ws = torch.empty(max(L.mie_sk_equalize_hist_workspace_bytes(n, DTYPE_CODE[x.dtype]), 1), dtype=torch.uint8, device=x.device)
-    with torch.cuda.device(x.device):
-        check(L.mie_sk_equalize_hist(x.data_ptr(), dst.data_ptr(), DTYPE_CODE[x.dtype], _OUT_CODE[dst.dtype], n, h, w,
-                                     h * w, w, h * w, w, ws.data_ptr(), ws.numel(), stream_ptr(x.device)))
+    dst = new_out(x, out_dtype, _OUT_CODE, torch.float64)
+    ws = use_workspace(x.device, lib().mie_sk_equalize_hist_workspace_bytes(n, DTYPE_CODE[x.dtype]))
+    call(x.device, "mie_sk_equalize_hist", x.data_ptr(), dst.data_ptr(), DTYPE_CODE[x.dtype], _OUT_CODE[dst.dtype],
+         *plane_layout(n, h, w), ws.data_ptr(), ws.numel())
     return dst
 
 
@@ -291,7 +263,7 @@ def denoise_bilateral(image: torch.Tensor, win_size=None, sigma_color=None, sigm
     if win_size is None:
         win_size = max(5, 2 * int(math.ceil(3 * sigma_spatial)) + 1)
     win_size = int(win_size)
-    dst = _sk_out(x, out_dtype, torch.float64)
+    dst = new_out(x, out_dtype, _OUT_CODE, torch.float64)
     if n == 0:
         return dst
     planes = x.reshape(n, h * w)
@@ -322,10 +294,9 @@ def denoise_bilateral(image: torch.Tensor, win_size=None, sigma_color=None, sigm
     spatial = np.exp(-0.5 * (np.hypot(rr, cc) ** 2 / float(sigma_spatial) ** 2)).ravel()
     d_luts = torch.from_numpy(np.ascontiguousarray(luts)).to(x.device)
     d_spatial = torch.from_numpy(np.ascontiguousarray(spatial)).to(x.device)
-    with torch.cuda.device(x.device):
-        check(lib().mie_sk_denoise_bilateral(x.data_ptr(), dst.data_ptr(), DTYPE_CODE[x.dtype], _OUT_CODE[dst.dtype], n, h, w,
-                                             h * w, w, h * w, w, win_size, int(bins), _PAD_MODES[mode], float(cval),
-                                             d_luts.data_ptr(), d_spatial.data_ptr(), ranges.data_ptr(), stream_ptr(x.device)))
+    call(x.device, "mie_sk_denoise_bilateral", x.data_ptr(), dst.data_ptr(), DTYPE_CODE[x.dtype], _OUT_CODE[dst.dtype],
+         *plane_layout(n, h, w), win_size, int(bins), _PAD_MODES[mode], float(cval), d_luts.data_ptr(),
+         d_spatial.data_ptr(), ranges.data_ptr())
     return dst
 
 
@@ -348,31 +319,21 @@ def _denoise_tv_chambolle(image, weight, eps, max_num_iter, channel_axis, out_dt
         raise ValueError("weight must be a positive finite number")
     if int(max_num_iter) < 1:
         raise ValueError("max_num_iter must be at least 1")
-    if volumetric:
-        _check_volume(image)
-    require_cuda(image)
     L = lib()
     if volumetric:
-        x = image.contiguous()
-        d, h, w = (int(s) for s in x.shape[-3:])
-        n = x.numel() // (d * h * w) if d * h * w else 0
+        x, n, d, h, w = as_volumes(image)
+        require_cuda(x)
+        entry, layout = "mie_sk_denoise_tv_chambolle3d", volume_layout(n, d, h, w)
         nbytes = L.mie_sk_tv_chambolle3d_workspace_bytes(n, d, h, w, DTYPE_CODE[x.dtype])
     else:
+        require_cuda(image)
         x, n, h, w = as_planes(image)
+        entry, layout = "mie_sk_denoise_tv_chambolle", plane_layout(n, h, w)
         nbytes = L.mie_sk_tv_chambolle_workspace_bytes(n, h, w, DTYPE_CODE[x.dtype])
-    dst = _sk_out(x, out_dtype, torch.float32 if x.dtype == torch.float32 else torch.float64)
+    dst = new_out(x, out_dtype, _OUT_CODE, _float_default(x))
     if iters is not None and (iters.dtype != torch.int32 or iters.numel() != n or iters.device != x.device):
         raise ValueError(f"iters must be an int32 tensor of {n} entries on {x.device}")
-    ws = torch.empty(max(nbytes, 1), dtype=torch.uint8, device=x.device)
-    it = None if iters is None else iters.data_ptr()
-    with torch.cuda.device(x.device):
-        if volumetric:
-            check(L.mie_sk_denoise_tv_chambolle3d(x.data_ptr(), dst.data_ptr(), DTYPE_CODE[x.dtype], _OUT_CODE[dst.dtype],
-                                                  n, d, h, w, d * h * w, h * w, w, d * h * w, h * w, w, float(weight),
-                                                  float(eps), int(max_num_iter), it, ws.data_ptr(), ws.numel(),
-                                                  stream_ptr(x.device)))
-        else:
-            check(L.mie_sk_denoise_tv_chambolle(x.data_ptr(), dst.data_ptr(), DTYPE_CODE[x.dtype], _OUT_CODE[dst.dtype],
-                                                n, h, w, h * w, w, h * w, w, float(weight), float(eps), int(max_num_iter),
-                                                it, ws.data_ptr(), ws.numel(), stream_ptr(x.device)))
+    ws = use_workspace(x.device, nbytes)
+    call(x.device, entry, x.data_ptr(), dst.data_ptr(), DTYPE_CODE[x.dtype], _OUT_CODE[dst.dtype], *layout, float(weight),
+         float(eps), int(max_num_iter), None if iters is None else iters.data_ptr(), ws.data_ptr(), ws.numel())
     return dst
