@@ -405,6 +405,51 @@ int mie_sk_denoise_tv_chambolle3d(const void* src, void* dst, int src_dtype, int
                                   int64_t dst_stride_n, int64_t dst_stride_d, int64_t dst_stride_h,
                                   double weight, double eps, int max_num_iter, int* iters,
                                   void* workspace, size_t workspace_bytes, void* stream);
+/* mie_sk_structural_similarity / mie_sk_structural_similarity3d: skimage.metrics.structural_similarity(im1, im2,
+ * win_size, data_range, gaussian_weights, K1, K2, sigma, use_sample_covariance) on every (h, w) plane (ndim 2) or every
+ * (d, h, w) volume (ndim 3) of the batch; a (1, h, w) volume is therefore not a plane (a 7x7x7 window needs d >= 7).
+ * RECALLED semantics (upstream skimage/metrics/_structural_similarity.py, 0.26; numpy twin tests/sk_ssim_twin.py):
+ *   F = float32 for f32 sources, float64 for u8 / u16 / i16 sources (RAW values, not img_as_float);
+ *   filter = uniform_filter(size = win_size) or, gaussian_weights, gaussian(sigma, truncate = 3.5, mode = 'reflect');
+ *   ux, uy, uxx, uyy, uxy = filter(a), filter(b), filter(a*a), filter(b*b), filter(a*b), products in F;
+ *   vx = cov_norm (uxx - ux ux), vy = cov_norm (uyy - uy uy), vxy = cov_norm (uxy - ux uy);
+ *   A1 = 2 ux uy + c1, A2 = 2 vxy + c2, B1 = ux^2 + uy^2 + c1, B2 = vx + vy + c2;  S = (A1 A2) / (B1 B2), all in F;
+ *   mssim = mean(S cropped by (win_size - 1) / 2 on every side of every axis), in float64.
+ * The caller computes cov_norm = NP / (NP - 1) with NP = win_size^ndim (1.0 without the sample covariance), c1 = (K1 R)^2
+ * and c2 = (K2 R)^2 as upstream does in Python; for f32 sources they are rounded to float32, as NumPy 2 does.
+ * scipy.ndimage's arithmetic (checked against scipy 1.18.1), which makes the map bit-exact: the 1-D pass runs along
+ * axis 0, then 1, then 2, each line extended by half-sample symmetric reflection (d c b a | a b c d | d c b a, repeated
+ * as often as needed) into float64, results rounded to F between passes.
+ *   box (taps == NULL): tmp = sum of the first win_size extended samples, out[0] = tmp / win_size, then for i >= 1
+ *        tmp += ext[i + win_size - 1] - ext[i - 1] and out[i] = tmp / win_size — a running sum over the whole line;
+ *   Gaussian (taps = HOST float64 weights exp(-0.5 x^2 / sigma^2) / sum, x = -r .. r, ntaps = 2r + 1 odd, copied at
+ *        call time): tmp = ext[c] w[r], then tmp += (ext[c + j] + ext[c - j]) w[j + r] for j = -r .. -1; no fma.
+ *        win_size then only sets the crop and NP; the taps may reach beyond an axis.
+ * map: NULL, or the S map (dst layout: its own strides), MIE_F64 for integer sources and MIE_F32 for f32 (MIE_E_DTYPE
+ * otherwise).  mssim: DEVICE double[n], one value per image.  MIE_E_KERNEL for win_size or ntaps even, < 1 or
+ * > MIE_MAX_TAPS; MIE_E_SHAPE for an image axis shorter than win_size.  The workspace (>= the query, 256-byte aligned)
+ * does not grow with n or d beyond a fixed bound: the batch runs in chunks whose float buffers stay below 640 MiB
+ * (plus 40 h w bytes for volumes, where a long volume's box z-pass carries its running sums between chunks).  Four
+ * launches per chunk (three for planes), the per-image sums in a fixed order (same bits on every run); no host
+ * synchronisation and no allocation, so the call can be captured into a CUDA graph.  n == 0 is a no-op. */
+size_t mie_sk_structural_similarity_workspace_bytes(int64_t n, int h, int w, int src_dtype);
+size_t mie_sk_structural_similarity3d_workspace_bytes(int64_t n, int d, int h, int w, int src_dtype);
+int mie_sk_structural_similarity(const void* a, const void* b, void* map, int src_dtype, int map_dtype,
+                                 int64_t n, int h, int w,
+                                 int64_t a_stride_n, int64_t a_stride_h,
+                                 int64_t b_stride_n, int64_t b_stride_h,
+                                 int64_t map_stride_n, int64_t map_stride_h,
+                                 int win_size, const double* taps, int ntaps,
+                                 double cov_norm, double c1, double c2, double* mssim,
+                                 void* workspace, size_t workspace_bytes, void* stream);
+int mie_sk_structural_similarity3d(const void* a, const void* b, void* map, int src_dtype, int map_dtype,
+                                   int64_t n, int d, int h, int w,
+                                   int64_t a_stride_n, int64_t a_stride_d, int64_t a_stride_h,
+                                   int64_t b_stride_n, int64_t b_stride_d, int64_t b_stride_h,
+                                   int64_t map_stride_n, int64_t map_stride_d, int64_t map_stride_h,
+                                   int win_size, const double* taps, int ntaps,
+                                   double cov_norm, double c1, double c2, double* mssim,
+                                   void* workspace, size_t workspace_bytes, void* stream);
 size_t mie_sk_equalize_hist_workspace_bytes(int64_t n, int src_dtype);
 int mie_sk_equalize_hist(const void* src, void* dst, int src_dtype, int dst_dtype,
                          int64_t n, int h, int w,

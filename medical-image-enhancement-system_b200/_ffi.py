@@ -73,6 +73,12 @@ SIGNATURES = {
     "mie_sk_tv_chambolle3d_workspace_bytes": ([_i64, _i, _i, _i, _i], _sz),
     "mie_sk_denoise_tv_chambolle": ([_p, _p, _i, _i, *_planes, _d, _d, _i, _p, _p, _sz, _p], _i),
     "mie_sk_denoise_tv_chambolle3d": ([_p, _p, _i, _i, *_volumes, _d, _d, _i, _p, _p, _sz, _p], _i),
+    "mie_sk_structural_similarity_workspace_bytes": ([_i64, _i, _i, _i], _sz),
+    "mie_sk_structural_similarity3d_workspace_bytes": ([_i64, _i, _i, _i, _i], _sz),
+    "mie_sk_structural_similarity": (
+        [_p, _p, _p, _i, _i, *_planes, _i64, _i64, _i, _p, _i, _d, _d, _d, _p, _p, _sz, _p], _i),
+    "mie_sk_structural_similarity3d": (
+        [_p, _p, _p, _i, _i, *_volumes, _i64, _i64, _i64, _i, _p, _i, _d, _d, _d, _p, _p, _sz, _p], _i),
     "mie_halo_exchange_available": ([], _i),
     "mie_halo_exchange_z": ([_p, _i, _i, _p, _p, _p, _p, _sz, _p], _i),
     "mie_enable_peer_access": ([_i], _i),

@@ -19,27 +19,6 @@ namespace mie {
 template <typename T> struct MetAcc { using type = long long; };
 template <> struct MetAcc<float> { using type = double; };
 
-template <typename A>
-__device__ __forceinline__ A warp_tree(A v) {
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-    return v;
-}
-// Sum over the 256 threads of a block, fixed order; result valid in thread 0.
-template <typename A>
-__device__ __forceinline__ A block_tree_256(A v, A* s8) {
-    v = warp_tree(v);
-    __syncthreads();
-    if ((threadIdx.x & 31) == 0) s8[threadIdx.x >> 5] = v;
-    __syncthreads();
-    A t = 0;
-    if (threadIdx.x == 0) {
-#pragma unroll
-        for (int i = 0; i < 8; ++i) t += s8[i];
-    }
-    return t;
-}
-
 // ---------------------------------------------------------------- sum (a-b)^2, sum |a-b|
 template <typename T>
 __global__ void __launch_bounds__(256)

@@ -9,6 +9,8 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include <type_traits>
+
 #include "../../include/mie.h"
 
 namespace mie {
@@ -61,6 +63,44 @@ __device__ __forceinline__ double skb_as_float(int v) {
     if constexpr (sizeof(T) == 1) return __ddiv_rn((double)v, 255.0);
     else if constexpr (T(-1) > T(0)) return __ddiv_rn((double)v, 65535.0);
     else return __ddiv_rn(__dadd_rn(__dmul_rn((double)v, 2.0), 1.0), 65535.0);
+}
+
+// One correctly rounded operation each, never contracted to fma: the scikit-image kernels follow numpy's element-wise
+// order with them, in the image's float type SkFloat<T> (float64 for integer images, float32 for float32 images).
+__device__ __forceinline__ float rn_add(float a, float b) { return __fadd_rn(a, b); }
+__device__ __forceinline__ double rn_add(double a, double b) { return __dadd_rn(a, b); }
+__device__ __forceinline__ float rn_sub(float a, float b) { return __fsub_rn(a, b); }
+__device__ __forceinline__ double rn_sub(double a, double b) { return __dsub_rn(a, b); }
+__device__ __forceinline__ float rn_mul(float a, float b) { return __fmul_rn(a, b); }
+__device__ __forceinline__ double rn_mul(double a, double b) { return __dmul_rn(a, b); }
+__device__ __forceinline__ float rn_div(float a, float b) { return __fdiv_rn(a, b); }
+__device__ __forceinline__ double rn_div(double a, double b) { return __ddiv_rn(a, b); }
+__device__ __forceinline__ float rn_sqrt(float a) { return __fsqrt_rn(a); }
+__device__ __forceinline__ double rn_sqrt(double a) { return __dsqrt_rn(a); }
+
+template <typename T>
+using SkFloat = typename std::conditional<std::is_same<T, float>::value, float, double>::type;
+
+// Fixed-order sums: a warp butterfly, then the 8 warp totals of a 256-thread block in index order (thread 0 holds the
+// block's sum), so a reduction gives the same bits on every run.
+template <typename A>
+__device__ __forceinline__ A warp_tree(A v) {
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+    return v;
+}
+template <typename A>
+__device__ __forceinline__ A block_tree_256(A v, A* s8) {
+    v = warp_tree(v);
+    __syncthreads();
+    if ((threadIdx.x & 31) == 0) s8[threadIdx.x >> 5] = v;
+    __syncthreads();
+    A t = 0;
+    if (threadIdx.x == 0) {
+#pragma unroll
+        for (int i = 0; i < 8; ++i) t += s8[i];
+    }
+    return t;
 }
 
 // ---------------------------------------------------------------- borders

@@ -21,21 +21,6 @@
 
 namespace mie {
 
-__device__ __forceinline__ float tv_add(float a, float b) { return __fadd_rn(a, b); }
-__device__ __forceinline__ double tv_add(double a, double b) { return __dadd_rn(a, b); }
-__device__ __forceinline__ float tv_sub(float a, float b) { return __fsub_rn(a, b); }
-__device__ __forceinline__ double tv_sub(double a, double b) { return __dsub_rn(a, b); }
-__device__ __forceinline__ float tv_mul(float a, float b) { return __fmul_rn(a, b); }
-__device__ __forceinline__ double tv_mul(double a, double b) { return __dmul_rn(a, b); }
-__device__ __forceinline__ float tv_div(float a, float b) { return __fdiv_rn(a, b); }
-__device__ __forceinline__ double tv_div(double a, double b) { return __ddiv_rn(a, b); }
-__device__ __forceinline__ float tv_sqrt(float a) { return __fsqrt_rn(a); }
-__device__ __forceinline__ double tv_sqrt(double a) { return __dsqrt_rn(a); }
-
-// The image's float type: float64 for integer images (img_as_float), float32 for float32 images.
-template <typename T>
-using TvF = typename std::conditional<std::is_same<T, float>::value, float, double>::type;
-
 // Per-image state, re-initialised by every call.
 struct TvState {
     double e_init, e_prev;   // energies, held exactly in double whatever the image's float type
@@ -59,7 +44,7 @@ struct TvGeom {
 };
 
 template <typename T>
-__device__ __forceinline__ TvF<T> tv_src(const T* src, int64_t off) {
+__device__ __forceinline__ SkFloat<T> tv_src(const T* src, int64_t off) {
     if constexpr (std::is_same<T, float>::value) return src[off];
     else return skb_as_float<T>((int)src[off]);
 }
@@ -68,9 +53,9 @@ __device__ __forceinline__ TvF<T> tv_src(const T* src, int64_t off) {
 // where the coordinate along a is >= 1; on the first pass p = 0 and upstream takes out = image.  Axis order is the
 // array's: (z, y, x) for volumes, (y, x) for planes.  *dval receives d.
 template <typename T, int ND>
-__device__ __forceinline__ TvF<T> tv_out(const T* src, const TvF<T>* p, const TvGeom& g, int64_t m, int z, int y, int x,
-                                         bool first, TvF<T>* dval) {
-    using F = TvF<T>;
+__device__ __forceinline__ SkFloat<T> tv_out(const T* src, const SkFloat<T>* p, const TvGeom& g, int64_t m, int z, int y, int x,
+                                         bool first, SkFloat<T>* dval) {
+    using F = SkFloat<T>;
     const F im = tv_src<T>(src, m * g.ssn + (int64_t)z * g.ssd + (int64_t)y * g.ssh + x);
     if (first) {
         *dval = F(0);
@@ -82,13 +67,13 @@ __device__ __forceinline__ TvF<T> tv_out(const T* src, const TvF<T>* p, const Tv
     const int64_t step[3] = {ND == 3 ? (int64_t)g.h * g.w : (int64_t)g.w, ND == 3 ? (int64_t)g.w : 1, 1};
     F s = p[v];
 #pragma unroll
-    for (int a = 1; a < ND; ++a) s = tv_add(s, p[a * cs + v]);
+    for (int a = 1; a < ND; ++a) s = rn_add(s, p[a * cs + v]);
     F d = -s;
 #pragma unroll
     for (int a = 0; a < ND; ++a)
-        if (coord[a] >= 1) d = tv_add(d, p[a * cs + v - step[a]]);
+        if (coord[a] >= 1) d = rn_add(d, p[a * cs + v - step[a]]);
     *dval = d;
-    return tv_add(im, d);
+    return rn_add(im, d);
 }
 
 // Fixed-order sum of (a, b) over the CTA (256 threads); the totals land in thread 0.
@@ -128,9 +113,9 @@ __host__ __device__ constexpr int tv_steps() { return ND == 3 ? kTvZ : kTvPlaneS
 // One pass of the loop (pass index `iter`, first == (iter == 0)) over every image of the batch that has not stopped.
 template <typename T, int ND>
 __global__ void __launch_bounds__(256)
-sk_tv_pass_kernel(const T* __restrict__ src, const TvF<T>* __restrict__ p_in, TvF<T>* __restrict__ p_out, TvGeom g,
-                  int iter, TvF<T> tau, TvF<T> tau_w, double weight, double eps, TvState* state, double2* partials) {
-    using F = TvF<T>;
+sk_tv_pass_kernel(const T* __restrict__ src, const SkFloat<T>* __restrict__ p_in, SkFloat<T>* __restrict__ p_out, TvGeom g,
+                  int iter, SkFloat<T> tau, SkFloat<T> tau_w, double weight, double eps, TvState* state, double2* partials) {
+    using F = SkFloat<T>;
     __shared__ double s_red[16];
     __shared__ int s_last;
     const int64_t m = blockIdx.x / g.tiles, tile = blockIdx.x % g.tiles;
@@ -149,7 +134,7 @@ sk_tv_pass_kernel(const T* __restrict__ src, const TvF<T>* __restrict__ p_in, Tv
         F d0, o;
         if (have_next) { o = o_next; d0 = d_next; }
         else o = tv_out<T, ND>(src, p_in, g, m, z, y, x, first, &d0);
-        sd += (double)tv_mul(d0, d0);
+        sd += (double)rn_mul(d0, d0);
         const int coord[3] = {ND == 3 ? z : y, ND == 3 ? y : x, x};
         F gr[ND];
 #pragma unroll
@@ -160,22 +145,22 @@ sk_tv_pass_kernel(const T* __restrict__ src, const TvF<T>* __restrict__ p_in, Tv
                           nx = x + (a == ND - 1);
                 F dn;
                 const F on = tv_out<T, ND>(src, p_in, g, m, nz, ny, nx, first, &dn);
-                gr[a] = tv_sub(on, o);
+                gr[a] = rn_sub(on, o);
                 if (ND == 3 && a == 0) { o_next = on; d_next = dn; }
             }
         }
         have_next = ND == 3 && coord[0] < lim[0] - 1;
-        F q = tv_mul(gr[0], gr[0]);
+        F q = rn_mul(gr[0], gr[0]);
 #pragma unroll
-        for (int a = 1; a < ND; ++a) q = tv_add(q, tv_mul(gr[a], gr[a]));
-        const F nrm = tv_sqrt(q);
+        for (int a = 1; a < ND; ++a) q = rn_add(q, rn_mul(gr[a], gr[a]));
+        const F nrm = rn_sqrt(q);
         sn += (double)nrm;
-        const F den = tv_add(tv_mul(nrm, tau_w), F(1));
+        const F den = rn_add(rn_mul(nrm, tau_w), F(1));
         const int64_t v = m * g.vox + ((int64_t)z * g.h + y) * g.w + x;
 #pragma unroll
         for (int a = 0; a < ND; ++a) {
             const F pv = first ? F(0) : p_in[a * cs + v];
-            p_out[a * cs + v] = tv_div(tv_sub(pv, tv_mul(tau, gr[a])), den);
+            p_out[a * cs + v] = rn_div(rn_sub(pv, rn_mul(tau, gr[a])), den);
         }
     }
     tv_block_sum2(sd, sn, s_red);
@@ -198,12 +183,12 @@ sk_tv_pass_kernel(const T* __restrict__ src, const TvF<T>* __restrict__ p_in, Tv
     tv_block_sum2(td, tn, s_red);
     if (threadIdx.x == 0) {
         TvState& st = state[m];
-        F e = tv_add((F)td, tv_mul((F)weight, (F)tn));
-        e = tv_div(e, (F)(double)g.vox);
+        F e = rn_add((F)td, rn_mul((F)weight, (F)tn));
+        e = rn_div(e, (F)(double)g.vox);
         if (first) {
             st.e_init = e;
             st.e_prev = e;
-        } else if (fabs(tv_sub((F)st.e_prev, e)) < tv_mul((F)eps, (F)st.e_init)) {
+        } else if (fabs(rn_sub((F)st.e_prev, e)) < rn_mul((F)eps, (F)st.e_init)) {
             st.done = 1;
             st.last = iter;
         } else {
@@ -221,9 +206,9 @@ __global__ void sk_tv_init_kernel(TvState* state, int64_t n, int last) {
 // dst = image + div(p entering pass `last`) of every image; iters[m] = last + 1 when iters is given.
 template <typename T, typename DstT, int ND>
 __global__ void __launch_bounds__(256)
-sk_tv_finish_kernel(const T* __restrict__ src, const TvF<T>* __restrict__ p0, const TvF<T>* __restrict__ p1, TvGeom g,
+sk_tv_finish_kernel(const T* __restrict__ src, const SkFloat<T>* __restrict__ p0, const SkFloat<T>* __restrict__ p1, TvGeom g,
                     DstT* __restrict__ dst, int64_t dsn, int64_t dsd, int64_t dsh, const TvState* state, int* iters) {
-    using F = TvF<T>;
+    using F = SkFloat<T>;
     const int64_t m = blockIdx.x / g.tiles, tile = blockIdx.x % g.tiles;
     const int last = state[m].last;
     if (iters && tile == 0 && threadIdx.x == 0) iters[m] = last + 1;
@@ -264,7 +249,7 @@ static size_t tv_workspace_bytes(int64_t n, int d, int h, int w, int nd, int src
 template <typename T, int ND>
 static void tv_launch(const T* src, void* dst, int dst_dtype, TvGeom g, int64_t dsn, int64_t dsd, int64_t dsh,
                       double weight, double eps, int max_num_iter, int* iters, uint8_t* ws, cudaStream_t st) {
-    using F = TvF<T>;
+    using F = SkFloat<T>;
     TvState* state = (TvState*)ws;
     ws += align256((size_t)g.n * sizeof(TvState));
     double2* partials = (double2*)ws;

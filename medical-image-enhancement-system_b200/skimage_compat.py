@@ -40,6 +40,13 @@ array instead: every (D, H, W) volume is one image with 3-D contextual regions, 
 volumetric=True) runs the 3-D algorithm on every volume.  RECALLED semantics, restated in oracle/skimage_twin.py (numpy,
 array-level) and oracle/mie_oracle.c (per pixel), which agree bit for bit; tests/test_live_pins.py compares all of it
 with the real package when it is importable.
+
+    structural_similarity(im1, im2, win_size, data_range, gaussian_weights, full, K1, K2, sigma, use_sample_covariance)
+                                                               <- skimage.metrics.structural_similarity
+
+scores every plane, or with volumetric=True every (D, H, W) volume, as one image with upstream's 'reflect' windows and
+sample covariance (csrc/sk_ssim.cu; RECALLED, numpy twin tests/sk_ssim_twin.py).  metrics.ssim is sewar's 2-D SSIM
+('valid' windows, population variance) and gives different numbers.
 """
 from __future__ import annotations
 
@@ -53,7 +60,7 @@ from ._ffi import (BORDER, DTYPE_CODE, MIE_F32, MIE_F64, as_planes, as_volumes, 
 from .filters import MAX_TAPS, denoise_nl_means, gaussian_blur2d, get_gaussian_kernel1d, median  # noqa: F401
 
 __all__ = ["gaussian", "unsharp_mask", "median", "denoise_nl_means", "SCIPY_MODES", "equalize_adapthist", "equalize_hist",
-           "denoise_bilateral", "denoise_tv_chambolle"]
+           "denoise_bilateral", "denoise_tv_chambolle", "structural_similarity"]
 
 SCIPY_MODES = {"nearest": "replicate", "reflect": "symmetric", "mirror": "reflect", "constant": "constant",
                "wrap": "circular"}
@@ -309,6 +316,109 @@ def denoise_tv_chambolle(image: torch.Tensor, weight: float = 0.1, eps: float = 
     treats a 3-D array.  Integer images are computed in float64 on the img_as_float scale, float32 images in float32;
     returns that float dtype, or `out_dtype`.  The iteration runs on the device with no host synchronisation."""
     return _denoise_tv_chambolle(image, weight, eps, max_num_iter, channel_axis, out_dtype, volumetric, None)
+
+
+_INT_DATA_RANGE = {torch.uint8: 255, torch.uint16: 65535, torch.int16: 65535}   # skimage dtype_range max - min
+_SSIM_KWARGS = ("K1", "K2", "sigma", "use_sample_covariance")
+
+
+def _ssim_taps(sigma: float, truncate: float) -> np.ndarray:
+    """scipy.ndimage's Gaussian weights in float64: exp(-0.5 / sigma^2 * x^2) / sum over x = -r .. r,
+    r = int(truncate * sigma + 0.5); a sigma scipy does not filter with (<= 1e-15) is the single weight 1."""
+    if sigma <= 1e-15:
+        return np.ones(1, np.float64)
+    r = int(truncate * sigma + 0.5)
+    x = np.arange(-r, r + 1)
+    phi = np.exp(-0.5 / (sigma * sigma) * x ** 2)
+    return phi / phi.sum()
+
+
+def structural_similarity(im1: torch.Tensor, im2: torch.Tensor, *, win_size=None, gradient: bool = False,
+                          data_range=None, channel_axis=None, gaussian_weights: bool = False, full: bool = False,
+                          volumetric: bool = False, **kwargs):
+    """skimage.metrics.structural_similarity of every (H, W) plane of im1 against the same plane of im2 ((H,W), (C,H,W),
+    (B,C,H,W)); with volumetric=True, of every (D, H, W) volume of a (D,H,W), (B,D,H,W) or (B,C,D,H,W) tensor as one
+    3-D image (7x7x7 windows by default).  kwargs: K1, K2, sigma, use_sample_covariance, as upstream.
+
+    Integer images are scored on their raw values in float64 (data_range defaults to the dtype's range), float32 images
+    in float32 (data_range required).  Returns a Python float for a single image, else a float64 CPU tensor shaped like
+    the leading dimensions; full=True returns (mssim, S) with S a CUDA tensor of the input's shape (float64 for integer
+    input, float32 for float32).  Bit-exact maps against scipy.ndimage's arithmetic (include/mie.h)."""
+    unknown = set(kwargs) - set(_SSIM_KWARGS)
+    if unknown:
+        raise TypeError(f"unexpected keyword arguments {sorted(unknown)}")
+    for name, t in (("im1", im1), ("im2", im2)):
+        if not isinstance(t, torch.Tensor) or t.dtype not in DTYPE_CODE:
+            raise TypeError(f"{name} must be a uint8, uint16, int16 or float32 torch.Tensor")
+    if im1.shape != im2.shape:
+        raise ValueError("Input images must have the same dimensions.")
+    if gradient:
+        raise NotImplementedError("gradient=True is not supported")
+    if channel_axis is not None:
+        raise NotImplementedError("images are scored separately; channel_axis is not supported")
+    if im1.dtype != im2.dtype:
+        raise NotImplementedError(f"im1 and im2 must have the same dtype; got {im1.dtype} and {im2.dtype}")
+    K1, K2, sigma = float(kwargs.get("K1", 0.01)), float(kwargs.get("K2", 0.03)), float(kwargs.get("sigma", 1.5))
+    if K1 < 0:
+        raise ValueError("K1 must be positive")
+    if K2 < 0:
+        raise ValueError("K2 must be positive")
+    if sigma < 0:
+        raise ValueError("sigma must be positive")
+    use_sample_covariance = kwargs.get("use_sample_covariance", True)
+    truncate = 3.5
+    if win_size is None:
+        win_size = 2 * int(truncate * sigma + 0.5) + 1 if gaussian_weights else 7
+    win_size = int(win_size)
+    ndim = 3 if volumetric else 2
+    if not ndim <= im1.dim() <= ndim + 2:
+        raise ValueError(f"expected (H,W), (C,H,W) or (B,C,H,W) with volumetric=False, (D,H,W), (B,D,H,W) or "
+                         f"(B,C,D,H,W) with volumetric=True; got shape {tuple(im1.shape)}")
+    dims = tuple(int(s) for s in im1.shape[-ndim:])
+    if any(s < win_size for s in dims):
+        raise ValueError("win_size exceeds image extent. Either ensure that your images are at least 7x7; or pass "
+                         "win_size explicitly in the function call, with an odd value less than or equal to the smaller "
+                         "side of your images.")
+    if win_size % 2 != 1:
+        raise ValueError("Window size must be odd.")
+    if data_range is None:
+        if im1.dtype == torch.float32:
+            raise ValueError("Since skimage 0.18, data_range must be supplied for floating-point inputs.")
+        data_range = _INT_DATA_RANGE[im1.dtype]
+    taps = _ssim_taps(sigma, truncate) if gaussian_weights else None
+    if win_size > MAX_TAPS or (taps is not None and taps.size > MAX_TAPS):
+        raise NotImplementedError(f"windows of up to {MAX_TAPS} taps are supported")
+    NP = win_size ** ndim
+    cov_norm = NP / (NP - 1) if use_sample_covariance else 1.0
+    C1 = (K1 * data_range) ** 2
+    C2 = (K2 * data_range) ** 2
+    require_cuda(im1, "im1")
+    require_cuda(im2, "im2")
+    if im1.device != im2.device:
+        raise ValueError("im1 and im2 must be on the same device")
+    if volumetric:
+        a, n, d, h, w = as_volumes(im1)
+    else:
+        a, n, h, w = as_planes(im1)
+    b = im2.contiguous()
+    code = DTYPE_CODE[a.dtype]
+    map_dtype = _float_default(a)
+    S = torch.empty(a.shape, dtype=map_dtype, device=a.device) if full else None
+    mssim = torch.empty(n, dtype=torch.float64, device=a.device)
+    L = lib()
+    if volumetric:
+        entry, layout = "mie_sk_structural_similarity3d", (*volume_layout(n, d, h, w), d * h * w, h * w, w)
+        nbytes = L.mie_sk_structural_similarity3d_workspace_bytes(n, d, h, w, code)
+    else:
+        entry, layout = "mie_sk_structural_similarity", (*plane_layout(n, h, w), h * w, w)
+        nbytes = L.mie_sk_structural_similarity_workspace_bytes(n, h, w, code)
+    ws = use_workspace(a.device, nbytes)
+    call(a.device, entry, a.data_ptr(), b.data_ptr(), None if S is None else S.data_ptr(), code, _OUT_CODE[map_dtype],
+         *layout, win_size, None if taps is None else taps.ctypes.data, 0 if taps is None else taps.size,
+         float(cov_norm), float(C1), float(C2), mssim.data_ptr(), ws.data_ptr(), ws.numel())
+    lead = tuple(a.shape[:-ndim])
+    result = float(mssim.item()) if not lead else mssim.cpu().reshape(lead)
+    return (result, S) if full else result
 
 
 def _denoise_tv_chambolle(image, weight, eps, max_num_iter, channel_axis, out_dtype, volumetric, iters):
