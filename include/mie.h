@@ -450,6 +450,90 @@ int mie_sk_structural_similarity3d(const void* a, const void* b, void* map, int 
                                    int win_size, const double* taps, int ntaps,
                                    double cov_norm, double c1, double c2, double* mssim,
                                    void* workspace, size_t workspace_bytes, void* stream);
+/* mie_sk_ridge_filter / mie_sk_ridge_filter3d: skimage.filters.frangi / hessian / sato / meijering(image, sigmas, ...,
+ * black_ridges, mode, cval) on every (h, w) plane (ndim 2) or every (d, h, w) volume (ndim 3) of the batch.
+ * mie_sk_hessian_matrix / mie_sk_hessian_matrix3d: skimage.feature.hessian_matrix(image, sigma, mode, cval, order='rc',
+ * use_gaussian_derivatives=True); mie_sk_hessian_eigvals: skimage.feature.hessian_matrix_eigvals.
+ * RECALLED semantics (upstream skimage/filters/ridges.py and skimage/feature/corner.py, 0.26; numpy twin
+ * tests/sk_ridges_twin.py):
+ *   F = float32 for f32 sources, float64 for u8 / u16 / i16 sources.  The ridge filters take image.astype(F) on RAW
+ *   values (negated when black_ridges == 0); hessian_matrix takes img_as_float (unsigned v / max, int16
+ *   (2 v + 1) / 65535).
+ *   Hessian: G_a = gaussian_filter(image, sigma, order = e_a, mode, cval), H_ab = gaussian_filter(G_a, sigma,
+ *   order = e_b) for (a, b) in combinations_with_replacement(range(ndim), 2): H00 H01 H11, or H00 H01 H02 H11 H12 H22.
+ *   Each gaussian_filter is a 1-D pass along axis 0, then 1, then 2, scipy's line arithmetic in float64 (checked
+ *   against scipy 1.18.1): the line extended by `mode` (MIE_BORDER_*: CONSTANT = scipy 'constant' with cval, SYMMETRIC
+ *   = 'reflect', REFLECT = 'mirror', REPLICATE = 'nearest', CIRCULAR = 'wrap', as often as needed), tmp = ext[c] w[r],
+ *   then tmp += (ext[c + j] + ext[c - j]) w[j + r] (order 0) or (ext[c + j] - ext[c - j]) w[j + r] (order 1) for
+ *   j = -r .. -1, no fma, rounded to F after each pass.  The elements are bit-exact.
+ *   Eigenvalues, decreasing: 2-D (m + hs, m - hs), m = (H00 + H11) / 2, hs = sqrt(H01^2 + ((H00 - H11) / 2)^2) in F
+ *   (bit-exact); 3-D cyclic Jacobi in float64, rounded to F (upstream: np.linalg.eigvalsh; both within a few ulp of
+ *   the largest |eigenvalue|).
+ *   filtered_max = 0; per sigma, in the order given: filtered_max = np.maximum(filtered_max, vals) with
+ *   FRANGI:    e sorted by |e| (stable); l2 (, l3) = max(e[1:], 1e-10); 2-D r_a = inf, r_b = |e0| / l2; 3-D
+ *              r_a = l2 / l3, r_b = |e0| / sqrt(l2 l3); s = sqrt(sum e^2); gamma < 0 (None): gamma = max(s) / 2 of the
+ *              FIRST sigma, per image (1 if that is 0), reused for every sigma;
+ *              vals = (1 - exp(-r_a^2 / 2 alpha^2)) exp(-r_b^2 / 2 beta^2) (1 - exp(-s^2 / 2 gamma^2)), in F;
+ *   HESSIAN:   frangi (the caller passes gamma = 15), then out[out <= 0] = 1;
+ *   SATO:      vals = sigma^2 * prod(max(e[:-1], 0)) ** (1 / (ndim - 1));
+ *   MEIJERING: vals = the entry of largest |.| (first on ties) of circulant([1, alpha, ...]) @ e, clamped at 0, divided
+ *              by its per-image max when that is > 0 (alpha: the caller passes 1 / (ndim + 1) for None).
+ * Taps are HOST float64 arrays computed by the caller as scipy does (_gaussian_kernel1d(sigma, order,
+ * int(4 sigma + 0.5))[::-1]), scale s at offset sum_{t < s} (2 radii[t] + 1) of taps0 (order 0) and taps1 (order 1),
+ * copied at call time.  Errors: MIE_E_KERNEL for a radius < 0 or > MIE_SK_RIDGE_MAX_RADIUS, taps0 not symmetric or
+ * taps1 not antisymmetric; MIE_E_RANGE for a sigma < 0 or not finite; MIE_E_NULL for null sigmas / radii / taps with
+ * nscales > 0; MIE_E_SHAPE for nscales < 0; MIE_E_BORDER for an unknown mode; MIE_E_UNSUPPORTED for an unknown filter;
+ * MIE_E_DTYPE for dst_dtype not MIE_F64 / MIE_F32 (the ridge filters; rounded once from F) or not F (hessian_matrix).
+ * nscales == 0 writes zeros (HESSIAN: ones).  n == 0 is a no-op.
+ * hessian_matrix writes element k of image i at dst + k dst_stride_e + i dst_stride_n + ... (dst_stride_e at least one
+ * whole batch, MIE_E_STRIDE otherwise).  eigvals: h and eig DEVICE arrays of `dtype` (MIE_F32 or MIE_F64), element k
+ * of voxel v at h[k h_stride_e + v] (ndim (ndim + 1) / 2 elements), eigenvalue k at eig[k eig_stride_e + v]; no
+ * workspace.
+ * Workspace (>= the query, 256-byte aligned): the batch runs in chunks of c = max(1, min(n, 2^24 / voxels, 65535))
+ * images, all scales of a chunk before the next, so it does not grow with n:
+ *   ridge, volumes:         9 align256(c voxels sizeof(F)) + 2 align256(8 c)
+ *   ridge, planes:          4 align256(c voxels sizeof(F)) + align256(8 c voxels) + 2 align256(8 c)
+ *   hessian_matrix:         5 (volumes) or 3 (planes) align256(c voxels sizeof(F))
+ * — 9 F-sized images for one 512^3 volume.  Planes keep the running maximum in float64: upstream's first frangi
+ * factor there is the float64 scalar 1 - exp(-inf), so its values are float64 from then on whatever F is.  Per scale: 24 pass launches for volumes (10 for planes) and one to three
+ * epilogue launches.  The per-image maxima are integer atomicMax on the bits of non-negative values (same bits on
+ * every run); no host synchronisation and no allocation, so the calls can be captured into a CUDA graph. */
+#define MIE_SK_RIDGE_MAX_RADIUS 64
+enum mie_sk_ridge { MIE_SK_FRANGI = 0, MIE_SK_HESSIAN = 1, MIE_SK_SATO = 2, MIE_SK_MEIJERING = 3 };
+size_t mie_sk_ridge_filter_workspace_bytes(int64_t n, int h, int w, int src_dtype);
+size_t mie_sk_ridge_filter3d_workspace_bytes(int64_t n, int d, int h, int w, int src_dtype);
+int mie_sk_ridge_filter(const void* src, void* dst, int src_dtype, int dst_dtype,
+                        int64_t n, int h, int w,
+                        int64_t src_stride_n, int64_t src_stride_h,
+                        int64_t dst_stride_n, int64_t dst_stride_h,
+                        int filter, int nscales, const double* sigmas, const int* radii,
+                        const double* taps0, const double* taps1, int mode, double cval, int black_ridges,
+                        double alpha, double beta, double gamma,
+                        void* workspace, size_t workspace_bytes, void* stream);
+int mie_sk_ridge_filter3d(const void* src, void* dst, int src_dtype, int dst_dtype,
+                          int64_t n, int d, int h, int w,
+                          int64_t src_stride_n, int64_t src_stride_d, int64_t src_stride_h,
+                          int64_t dst_stride_n, int64_t dst_stride_d, int64_t dst_stride_h,
+                          int filter, int nscales, const double* sigmas, const int* radii,
+                          const double* taps0, const double* taps1, int mode, double cval, int black_ridges,
+                          double alpha, double beta, double gamma,
+                          void* workspace, size_t workspace_bytes, void* stream);
+size_t mie_sk_hessian_matrix_workspace_bytes(int64_t n, int h, int w, int src_dtype);
+size_t mie_sk_hessian_matrix3d_workspace_bytes(int64_t n, int d, int h, int w, int src_dtype);
+int mie_sk_hessian_matrix(const void* src, void* dst, int src_dtype, int dst_dtype,
+                          int64_t n, int h, int w,
+                          int64_t src_stride_n, int64_t src_stride_h,
+                          int64_t dst_stride_n, int64_t dst_stride_h, int64_t dst_stride_e,
+                          int radius, const double* taps0, const double* taps1, int mode, double cval,
+                          void* workspace, size_t workspace_bytes, void* stream);
+int mie_sk_hessian_matrix3d(const void* src, void* dst, int src_dtype, int dst_dtype,
+                            int64_t n, int d, int h, int w,
+                            int64_t src_stride_n, int64_t src_stride_d, int64_t src_stride_h,
+                            int64_t dst_stride_n, int64_t dst_stride_d, int64_t dst_stride_h, int64_t dst_stride_e,
+                            int radius, const double* taps0, const double* taps1, int mode, double cval,
+                            void* workspace, size_t workspace_bytes, void* stream);
+int mie_sk_hessian_eigvals(const void* h, void* eig, int dtype, int ndim, int64_t count,
+                           int64_t h_stride_e, int64_t eig_stride_e, void* stream);
 size_t mie_sk_equalize_hist_workspace_bytes(int64_t n, int src_dtype);
 int mie_sk_equalize_hist(const void* src, void* dst, int src_dtype, int dst_dtype,
                          int64_t n, int h, int w,

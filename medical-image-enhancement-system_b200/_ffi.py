@@ -79,6 +79,17 @@ SIGNATURES = {
         [_p, _p, _p, _i, _i, *_planes, _i64, _i64, _i, _p, _i, _d, _d, _d, _p, _p, _sz, _p], _i),
     "mie_sk_structural_similarity3d": (
         [_p, _p, _p, _i, _i, *_volumes, _i64, _i64, _i64, _i, _p, _i, _d, _d, _d, _p, _p, _sz, _p], _i),
+    "mie_sk_ridge_filter_workspace_bytes": ([_i64, _i, _i, _i], _sz),
+    "mie_sk_ridge_filter3d_workspace_bytes": ([_i64, _i, _i, _i, _i], _sz),
+    "mie_sk_ridge_filter": (
+        [_p, _p, _i, _i, *_planes, _i, _i, _p, _p, _p, _p, _i, _d, _i, _d, _d, _d, _p, _sz, _p], _i),
+    "mie_sk_ridge_filter3d": (
+        [_p, _p, _i, _i, *_volumes, _i, _i, _p, _p, _p, _p, _i, _d, _i, _d, _d, _d, _p, _sz, _p], _i),
+    "mie_sk_hessian_matrix_workspace_bytes": ([_i64, _i, _i, _i], _sz),
+    "mie_sk_hessian_matrix3d_workspace_bytes": ([_i64, _i, _i, _i, _i], _sz),
+    "mie_sk_hessian_matrix": ([_p, _p, _i, _i, *_planes, _i64, _i, _p, _p, _i, _d, _p, _sz, _p], _i),
+    "mie_sk_hessian_matrix3d": ([_p, _p, _i, _i, *_volumes, _i64, _i, _p, _p, _i, _d, _p, _sz, _p], _i),
+    "mie_sk_hessian_eigvals": ([_p, _p, _i, _i, _i64, _i64, _i64, _p], _i),
     "mie_halo_exchange_available": ([], _i),
     "mie_halo_exchange_z": ([_p, _i, _i, _p, _p, _p, _p, _sz, _p], _i),
     "mie_enable_peer_access": ([_i], _i),

@@ -47,6 +47,14 @@ with the real package when it is importable.
 scores every plane, or with volumetric=True every (D, H, W) volume, as one image with upstream's 'reflect' windows and
 sample covariance (csrc/sk_ssim.cu; RECALLED, numpy twin tests/sk_ssim_twin.py).  metrics.ssim is sewar's 2-D SSIM
 ('valid' windows, population variance) and gives different numbers.
+
+    frangi / hessian / sato / meijering(image, sigmas, ..., black_ridges, mode, cval)  <- skimage.filters.*
+    hessian_matrix(image, sigma, mode, cval, use_gaussian_derivatives=True)           <- skimage.feature.hessian_matrix
+    hessian_matrix_eigvals(H_elems)                                  <- skimage.feature.hessian_matrix_eigvals
+
+are the Hessian-based ridge (vesselness) filters, per plane or, volumetric=True, per volume (csrc/sk_ridges.cu;
+RECALLED, numpy twin tests/sk_ridges_twin.py).  The Hessian elements are bit-exact against scipy.ndimage's arithmetic;
+3-D eigenvalues come from a float64 Jacobi solver instead of LAPACK.
 """
 from __future__ import annotations
 
@@ -60,7 +68,8 @@ from ._ffi import (BORDER, DTYPE_CODE, MIE_F32, MIE_F64, as_planes, as_volumes, 
 from .filters import MAX_TAPS, denoise_nl_means, gaussian_blur2d, get_gaussian_kernel1d, median  # noqa: F401
 
 __all__ = ["gaussian", "unsharp_mask", "median", "denoise_nl_means", "SCIPY_MODES", "equalize_adapthist", "equalize_hist",
-           "denoise_bilateral", "denoise_tv_chambolle", "structural_similarity"]
+           "denoise_bilateral", "denoise_tv_chambolle", "structural_similarity", "frangi", "hessian", "sato",
+           "meijering", "hessian_matrix", "hessian_matrix_eigvals"]
 
 SCIPY_MODES = {"nearest": "replicate", "reflect": "symmetric", "mirror": "reflect", "constant": "constant",
                "wrap": "circular"}
@@ -447,3 +456,179 @@ def _denoise_tv_chambolle(image, weight, eps, max_num_iter, channel_axis, out_dt
     call(x.device, entry, x.data_ptr(), dst.data_ptr(), DTYPE_CODE[x.dtype], _OUT_CODE[dst.dtype], *layout, float(weight),
          float(eps), int(max_num_iter), None if iters is None else iters.data_ptr(), ws.data_ptr(), ws.numel())
     return dst
+
+
+# ---------------------------------------------------------------------------------------------- ridge filters
+RIDGE_MAX_RADIUS = 64   # MIE_SK_RIDGE_MAX_RADIUS: sigma < 16 at scipy's truncate of 4
+_RIDGE_FILTER = {"frangi": 0, "hessian": 1, "sato": 2, "meijering": 3}
+
+
+def _gaussian_kernel1d(sigma: float, order: int, radius: int) -> np.ndarray:
+    """scipy.ndimage's _gaussian_kernel1d (float64), transcribed so that the taps are scipy's bit for bit."""
+    exponent_range = np.arange(order + 1)
+    sigma2 = sigma * sigma
+    x = np.arange(-radius, radius + 1)
+    phi_x = np.exp(-0.5 / sigma2 * x ** 2)
+    phi_x = phi_x / phi_x.sum()
+    if order == 0:
+        return phi_x
+    q = np.zeros(order + 1)
+    q[0] = 1
+    D = np.diag(exponent_range[1:], 1)
+    P = np.diag(np.ones(order) / -sigma2, -1)
+    Q_deriv = D + P
+    for _ in range(order):
+        q = Q_deriv.dot(q)
+    q = (x[:, None] ** exponent_range).dot(q)
+    return q * phi_x
+
+
+def _hessian_taps(sigma: float):
+    """(radius, order-0 taps, order-1 taps) of gaussian_filter(sigma, order, truncate=4.0) in correlation order:
+    scipy's gaussian_filter1d correlates with _gaussian_kernel1d(sigma, order, int(4 sigma + 0.5))[::-1]."""
+    sigma = float(sigma)
+    if sigma < 0.0 or sigma != sigma:
+        raise ValueError("Sigma values less than zero are not valid")
+    if sigma == 0.0:
+        raise NotImplementedError("sigma 0 (scipy then skips the derivative) is not supported")
+    r = int(4.0 * sigma + 0.5)
+    if r > RIDGE_MAX_RADIUS:
+        raise NotImplementedError(f"sigma {sigma} needs a filter radius of {r}; up to {RIDGE_MAX_RADIUS} is supported")
+    return r, np.ascontiguousarray(_gaussian_kernel1d(sigma, 0, r)[::-1]), \
+        np.ascontiguousarray(_gaussian_kernel1d(sigma, 1, r)[::-1])
+
+
+def _ridge_border(mode: str) -> int:
+    if mode not in SCIPY_MODES:
+        raise ValueError(f"mode must be one of {sorted(SCIPY_MODES)}. Got {mode!r}")
+    return BORDER[SCIPY_MODES[mode]]
+
+
+def _ridge_image(image: torch.Tensor, volumetric: bool):
+    """-> (dense tensor, n, d, h, w, layout arguments, entry point suffix)."""
+    if volumetric:
+        x, n, d, h, w = as_volumes(image)
+        require_cuda(x)
+        return x, n, d, h, w, volume_layout(n, d, h, w), "3d"
+    require_cuda(image)
+    x, n, h, w = as_planes(image)
+    return x, n, 1, h, w, plane_layout(n, h, w), ""
+
+
+def _ridge(image, name, sigmas, mode, cval, black_ridges, alpha, beta, gamma, out_dtype, volumetric):
+    sig = [float(s) for s in np.asarray(sigmas, dtype=np.float64).ravel()]
+    if any(s < 0.0 for s in sig):
+        raise ValueError("Sigma values less than zero are not valid")
+    taps = [_hessian_taps(s) for s in sig]
+    border = _ridge_border(mode)
+    x, n, d, h, w, layout, nd = _ridge_image(image, volumetric)
+    dst = new_out(x, out_dtype, _OUT_CODE, _float_default(x))
+    code = DTYPE_CODE[x.dtype]
+    L = lib()
+    if nd:
+        nbytes = L.mie_sk_ridge_filter3d_workspace_bytes(n, d, h, w, code)
+    else:
+        nbytes = L.mie_sk_ridge_filter_workspace_bytes(n, h, w, code)
+    sig_a = np.asarray(sig, np.float64)
+    radii = np.asarray([t[0] for t in taps], np.int32)
+    t0 = np.concatenate([t[1] for t in taps]) if taps else np.zeros(1)
+    t1 = np.concatenate([t[2] for t in taps]) if taps else np.zeros(1)
+    ws = use_workspace(x.device, nbytes)
+    call(x.device, "mie_sk_ridge_filter" + nd, x.data_ptr(), dst.data_ptr(), code, _OUT_CODE[dst.dtype], *layout,
+         _RIDGE_FILTER[name], len(sig), sig_a.ctypes.data, radii.ctypes.data, t0.ctypes.data, t1.ctypes.data, border,
+         float(cval), int(bool(black_ridges)), float(alpha), float(beta), -1.0 if gamma is None else abs(float(gamma)),
+         ws.data_ptr(), ws.numel())
+    return dst
+
+
+def _scales(sigmas, scale_range, scale_step):
+    if scale_range is not None and scale_step is not None:
+        return np.arange(scale_range[0], scale_range[1], scale_step)
+    return sigmas
+
+
+def frangi(image: torch.Tensor, sigmas=range(1, 10, 2), scale_range=None, scale_step=None, alpha=0.5, beta=0.5,
+           gamma=None, black_ridges=True, mode="reflect", cval=0, *, out_dtype=None,
+           volumetric: bool = False) -> torch.Tensor:
+    """skimage.filters.frangi on every (H, W) plane of `image` ((H,W), (C,H,W), (B,C,H,W)), each plane one image; with
+    volumetric=True on every (D, H, W) volume of a (D,H,W), (B,D,H,W) or (B,C,D,H,W) tensor.  gamma=None takes half the
+    largest Hessian norm of the first sigma, per image.  Integer images are filtered on their raw values in float64,
+    float32 images in float32; returns that float dtype, or `out_dtype` (float64 or float32, rounded once)."""
+    return _ridge(image, "frangi", _scales(sigmas, scale_range, scale_step), mode, cval, black_ridges, alpha, beta,
+                  gamma, out_dtype, volumetric)
+
+
+def hessian(image: torch.Tensor, sigmas=range(1, 10, 2), scale_range=None, scale_step=None, alpha=0.5, beta=0.5,
+            gamma=15, black_ridges=True, mode="reflect", cval=0, *, out_dtype=None,
+            volumetric: bool = False) -> torch.Tensor:
+    """skimage.filters.hessian: frangi with gamma=15, then every value <= 0 set to 1.  Layout and dtypes as frangi."""
+    return _ridge(image, "hessian", _scales(sigmas, scale_range, scale_step), mode, cval, black_ridges, alpha, beta,
+                  gamma, out_dtype, volumetric)
+
+
+def sato(image: torch.Tensor, sigmas=range(1, 10, 2), black_ridges=True, mode="reflect", cval=0, *, out_dtype=None,
+         volumetric: bool = False) -> torch.Tensor:
+    """skimage.filters.sato.  Layout and dtypes as frangi."""
+    return _ridge(image, "sato", sigmas, mode, cval, black_ridges, 0.0, 0.0, None, out_dtype, volumetric)
+
+
+def meijering(image: torch.Tensor, sigmas=range(1, 10, 2), alpha=None, black_ridges=True, mode="reflect", cval=0, *,
+              out_dtype=None, volumetric: bool = False) -> torch.Tensor:
+    """skimage.filters.meijering (alpha=None: 1 / (ndim + 1)); every scale is divided by its own per-image maximum.
+    Layout and dtypes as frangi."""
+    if alpha is None:
+        alpha = 1 / ((3 if volumetric else 2) + 1)
+    return _ridge(image, "meijering", sigmas, mode, cval, black_ridges, alpha, 0.0, None, out_dtype, volumetric)
+
+
+def hessian_matrix(image: torch.Tensor, sigma=1, mode="constant", cval=0, order="rc", use_gaussian_derivatives=None,
+                   *, volumetric: bool = False) -> list:
+    """skimage.feature.hessian_matrix(..., use_gaussian_derivatives=True) of every plane (or, volumetric=True, every
+    volume): [H00, H01, H11] or [H00, H01, H02, H11, H12, H22], CUDA tensors of the input's shape on the img_as_float
+    scale (float64 for integer input, float32 for float32), bit-exact against scipy.ndimage's arithmetic."""
+    if use_gaussian_derivatives is not True:
+        raise NotImplementedError("only use_gaussian_derivatives=True is built (the np.gradient path is not)")
+    if order == "xy":
+        raise NotImplementedError("order='xy' is not supported")
+    if order != "rc":
+        raise ValueError("order must be 'rc' or 'xy'")
+    if isinstance(sigma, (tuple, list)):
+        raise NotImplementedError("one sigma for every axis is supported")
+    r, t0, t1 = _hessian_taps(sigma)
+    border = _ridge_border(mode)
+    x, n, d, h, w, layout, nd = _ridge_image(image, volumetric)
+    ndim = 3 if nd else 2
+    dt = _float_default(x)
+    out = torch.empty((ndim * (ndim + 1) // 2, *x.shape), dtype=dt, device=x.device)
+    code = DTYPE_CODE[x.dtype]
+    L = lib()
+    if nd:
+        nbytes = L.mie_sk_hessian_matrix3d_workspace_bytes(n, d, h, w, code)
+    else:
+        nbytes = L.mie_sk_hessian_matrix_workspace_bytes(n, h, w, code)
+    ws = use_workspace(x.device, nbytes)
+    call(x.device, "mie_sk_hessian_matrix" + nd, x.data_ptr(), out.data_ptr(), code, _OUT_CODE[dt], *layout,
+         x.numel(), r, t0.ctypes.data, t1.ctypes.data, border, float(cval), ws.data_ptr(), ws.numel())
+    return list(out.unbind(0))
+
+
+def hessian_matrix_eigvals(H_elems) -> torch.Tensor:
+    """skimage.feature.hessian_matrix_eigvals: the eigenvalues of every voxel in decreasing order, a CUDA tensor of
+    shape (ndim, *H_elems[0].shape).  3 elements: 2-D (upstream's closed form, bit-exact); 6: 3-D (cyclic Jacobi in
+    float64, rounded to the elements' dtype)."""
+    H_elems = list(H_elems)
+    ndim = {3: 2, 6: 3}.get(len(H_elems))
+    if ndim is None:
+        raise ValueError(f"expected the 3 (2-D) or 6 (3-D) Hessian elements; got {len(H_elems)}")
+    first = H_elems[0]
+    for t in H_elems:
+        if not isinstance(t, torch.Tensor) or not t.is_cuda or t.dtype not in (torch.float32, torch.float64):
+            raise TypeError("H_elems must be float32 or float64 CUDA tensors")
+        if t.shape != first.shape or t.dtype != first.dtype or t.device != first.device:
+            raise ValueError("H_elems must share shape, dtype and device")
+    h = torch.stack([t.contiguous() for t in H_elems])
+    eig = torch.empty((ndim, *first.shape), dtype=first.dtype, device=first.device)
+    count = first.numel()
+    call(first.device, "mie_sk_hessian_eigvals", h.data_ptr(), eig.data_ptr(), _OUT_CODE[first.dtype], ndim, count,
+         count, count)
+    return eig

@@ -12,7 +12,7 @@ from __future__ import annotations
 
 import numpy as np
 
-__all__ = ["uniform", "phantom", "constant", "phantom_volume", "make"]
+__all__ = ["uniform", "phantom", "constant", "phantom_volume", "vessel_volume", "make"]
 
 
 def uniform(shape, dtype=np.uint16, seed: int = 0) -> np.ndarray:
@@ -73,6 +73,39 @@ def phantom_volume(shape, dtype=np.int16, seed: int = 0) -> np.ndarray:
     if np.dtype(dtype) == np.int16:
         out = out - 1024.0
     return np.rint(out).astype(dtype)
+
+
+def vessel_volume(shape, dtype=np.int16, seed: int = 0, tubes: int = 12) -> np.ndarray:
+    """(D, H, W) angiography-like volume: `tubes` bright straight vessels of radius 1 to 6 voxels in random orientations
+    (contrast-enhanced blood, 250 to 450 HU, with a soft edge) on soft tissue (40 HU) with N(0, 20) noise.  int16 is
+    in HU; uint16 is HU + 1024; uint8 is (HU + 1024) / 8 clipped to 255; float32 is (HU + 1024) / 4096."""
+    d, h, w = shape
+    rng = np.random.default_rng(seed)
+    centre = rng.uniform(0.2, 0.8, size=(tubes, 3)) * np.array([d, h, w])
+    axis = rng.normal(size=(tubes, 3))
+    axis /= np.linalg.norm(axis, axis=1, keepdims=True)
+    radius = rng.uniform(1.0, 6.0, size=tubes)
+    level = rng.uniform(250.0, 450.0, size=tubes)
+    out = np.empty((d, h, w), np.float32)
+    yy, xx = np.mgrid[0:h, 0:w].astype(np.float32)
+    for z in range(d):
+        sl = np.full((h, w), 40.0, np.float32)
+        for c, u, r, v in zip(centre, axis, radius, level):
+            pz, py, px = np.float32(z - c[0]), yy - np.float32(c[1]), xx - np.float32(c[2])
+            along = pz * np.float32(u[0]) + py * np.float32(u[1]) + px * np.float32(u[2])
+            dist2 = pz * pz + py * py + px * px - along * along
+            inside = np.clip(np.float32(r) + 0.5 - np.sqrt(np.maximum(dist2, 0.0)), 0.0, 1.0)
+            sl = np.maximum(sl, 40.0 + (v - 40.0) * inside)
+        out[z] = sl
+    out += rng.normal(0.0, 20.0, size=(d, h, w)).astype(np.float32)
+    dt = np.dtype(dtype)
+    if dt == np.int16:
+        return np.rint(out).astype(np.int16)
+    if dt == np.uint16:
+        return np.rint(out + 1024.0).clip(0, 65535).astype(np.uint16)
+    if dt == np.uint8:
+        return np.rint((out + 1024.0) / 8.0).clip(0, 255).astype(np.uint8)
+    return ((out + 1024.0) / 4096.0).astype(np.float32)
 
 
 def make(kind: str, shape, dtype=np.uint16, seed: int = 0) -> np.ndarray:
