@@ -244,6 +244,39 @@ int mie_median3d(const void* src, void* dst, int dtype, int d, int h, int w,
                  int64_t dst_stride_d, int64_t dst_stride_h,
                  const void* halo_lo, const void* halo_hi, int border, void* stream);
 
+/* mie_sk_median / mie_sk_median3d: skimage.filters.median(image, footprint, mode, cval) with ANY boolean footprint
+ * -> scipy.ndimage.median_filter(image, footprint=footprint, mode=mode, cval=cval), on n planes or n volumes
+ * (reference pyproject.toml:12; SURVEY.md §8(a) A6).  Semantics VERIFIED against scipy 1.18.1
+ * (tests/test_sk_median.py pins them on the CPU):
+ *   out[p] = element count / 2 (0-based) of the sorted samples in[p + c - extent / 2] over the set cells c of the
+ *   footprint (integer division per axis: even extents are legal and their centre sits at extent / 2), i.e. the upper
+ *   median when count is even.  Samples outside the image follow `border` (MIE_BORDER_*: SYMMETRIC = scipy 'reflect',
+ *   REFLECT = 'mirror', REPLICATE = 'nearest', CIRCULAR = 'wrap', folded as often as needed when the footprint is
+ *   longer than the axis; CONSTANT = 'constant', where the sample is cval).  Pure selection: dst_dtype == src_dtype ==
+ *   dtype, and every output is a sample or cval.  scipy's 'reflect' reads outside the image at offsets -2 n m (m >= 2)
+ *   of an axis of length n > 1; the kernels fold those like every other offset (filters.median refuses footprints that
+ *   reach them).  skimage.morphology.disk / ball (X^2 + Y^2 (+ Z^2) <= r^2) are RECALLED.  NaN in float images has no defined median (unspecified here as in
+ *   scipy); with both -0.0 and +0.0 in a window the sign of a zero result may differ from scipy's.
+ * footprint: HOST row-major uint8 mask of fy x fx (fz x fy x fx) cells, nonzero = set, read at call time.  Extents 1 ..
+ * MIE_SK_MEDIAN_MAX_EXTENT (planes) or 1 .. MIE_SK_MEDIAN3D_MAX_EXTENT (volumes) per axis.
+ * cval: the constant already cast to the image dtype as scipy casts it (the caller does the cast), so it must be
+ * exactly representable: an integer in the dtype's range, or a float32 value (inf and NaN included).
+ * Errors: MIE_E_KERNEL for an extent < 1 or above the bound, or a mask with no set cell; MIE_E_NULL for a null
+ * footprint (or null src / dst with n > 0); MIE_E_BORDER for an unknown mode; MIE_E_RANGE for a cval that is not
+ * representable; MIE_E_DTYPE, MIE_E_SHAPE and MIE_E_STRIDE as everywhere.  n == 0 is a no-op after the checks.
+ * No workspace, no allocation and no host synchronisation (the footprint travels in the kernel parameters), so the
+ * calls can be captured into a CUDA graph; 64-bit addressing. */
+#define MIE_SK_MEDIAN_MAX_EXTENT 65
+#define MIE_SK_MEDIAN3D_MAX_EXTENT 17
+int mie_sk_median(const void* src, void* dst, int dtype, int64_t n, int h, int w,
+                  int64_t src_stride_n, int64_t src_stride_h,
+                  int64_t dst_stride_n, int64_t dst_stride_h,
+                  const uint8_t* footprint, int fy, int fx, int border, double cval, void* stream);
+int mie_sk_median3d(const void* src, void* dst, int dtype, int64_t n, int d, int h, int w,
+                    int64_t src_stride_n, int64_t src_stride_d, int64_t src_stride_h,
+                    int64_t dst_stride_n, int64_t dst_stride_d, int64_t dst_stride_h,
+                    const uint8_t* footprint, int fz, int fy, int fx, int border, double cval, void* stream);
+
 /* ------------------------------------------------------------------ bilateral
  * Replaces kornia.filters.bilateral_blur(input, kernel_size, sigma_color,
  * sigma_space, border_type, color_distance_type) for single-channel planes

@@ -18,6 +18,9 @@ LIB_PATH = os.environ.get("MIE_B200_LIB") or os.path.join(PKG_DIR, "libmie_b200.
 
 MIE_U8, MIE_U16, MIE_I16, MIE_F32, MIE_F64 = 0, 1, 2, 3, 4
 BORDER = {"constant": 0, "reflect": 1, "replicate": 2, "circular": 3, "symmetric": 4}
+# scipy.ndimage / scikit-image mode names -> BORDER names
+SCIPY_MODES = {"nearest": "replicate", "reflect": "symmetric", "mirror": "reflect", "constant": "constant",
+               "wrap": "circular"}
 CLAHE_KORNIA, CLAHE_OPENCV = 0, 1
 
 DTYPE_CODE = {torch.uint8: MIE_U8, torch.uint16: MIE_U16, torch.int16: MIE_I16, torch.float32: MIE_F32}
@@ -53,6 +56,8 @@ SIGNATURES = {
     "mie_equalize": ([_p, _p, _i, _i, *_planes, _f, _f, _p, _sz, _p], _i),
     "mie_median2d": ([_p, _p, _i, *_planes, _i, _i, _i, _p], _i),
     "mie_median3d": ([_p, _p, _i, _i, _i, _i, _i64, _i64, _i64, _i64, _p, _p, _i, _p], _i),
+    "mie_sk_median": ([_p, _p, _i, *_planes, _p, _i, _i, _i, _d, _p], _i),
+    "mie_sk_median3d": ([_p, _p, _i, *_volumes, _p, _i, _i, _i, _i, _d, _p], _i),
     "mie_bilateral": ([_p, _p, _i, _i, *_planes, _p, _i, _i, _f, _i, _f, _f, _p], _i),
     "mie_nlm": ([_p, _p, _i, _i, *_planes, _i, _i, _f, _f, _f, _f, _p], _i),
     "mie_nlm_slow": ([_p, _p, _i, _i, *_planes, _i, _i, _d, _d, _f, _f, _p], _i),

@@ -4,17 +4,19 @@ call signatures, backed by the sm_100a kernels behind include/mie.h.
   gaussian_blur2d, unsharp_mask, median_blur, bilateral_blur
       <- kornia.filters.*            (reference pyproject.toml:8;  SURVEY.md §8(a) A3,A4,A5,A7)
   median
-      <- skimage.filters.median      (reference pyproject.toml:12; SURVEY.md §8(a) A6)
+      <- skimage.filters.median      (reference pyproject.toml:12; SURVEY.md §8(a) A6), any footprint and scipy mode
 
 Integer tensors are accepted directly (see enhance.py for the mapping rule).
 """
 from __future__ import annotations
 
+import math
+
 import numpy as np
 import torch
 
-from ._ffi import (BORDER, DTYPE_CODE, MIE_F64, as_planes, call, check_out, new_out, plane_layout, require_cuda,
-                   value_range_of)
+from ._ffi import (BORDER, DTYPE_CODE, MIE_F64, SCIPY_MODES, as_planes, call, check_out, new_out, plane_layout,
+                   require_cuda, value_range_of, volume_layout)
 
 __all__ = ["get_gaussian_kernel1d", "gaussian_blur2d", "unsharp_mask", "median_blur", "bilateral_blur", "median"]
 
@@ -164,30 +166,81 @@ def denoise_nl_means(image: torch.Tensor, patch_size: int = 7, patch_distance: i
     return dst
 
 
-_MEDIAN_MODES = {"nearest": "replicate", "constant": "constant"}
+MEDIAN_MAX_EXTENT = {2: 65, 3: 17}   # MIE_SK_MEDIAN_MAX_EXTENT, MIE_SK_MEDIAN3D_MAX_EXTENT (include/mie.h)
+_INT_RANGE = {torch.uint8: (0, 255), torch.uint16: (0, 65535), torch.int16: (-32768, 32767)}
+
+
+def median_cval(dtype: torch.dtype, cval, two_cell_box: bool = False) -> float:
+    """`cval` cast to the image dtype the way scipy.ndimage.median_filter casts it (checked against scipy 1.18.1):
+    float32 images round it to float32 (1e300 -> inf); integer images truncate it towards zero to a 32-bit integer
+    and keep its low bits (uint8: 300 -> 44, -1 -> 255; int16: -2.5 -> -2), before selection.  Outside the 32-bit
+    range, or not finite, scipy's result is the platform's out-of-range conversion: NotImplementedError.
+    `two_cell_box`: a footprint of two set cells and no unset one.  scipy then runs its separable maximum filter, which
+    compares the double cval and casts the result: a cval below the dtype's range never wins (the dtype minimum
+    does the same), and one above it is NotImplementedError (the cast result does not depend on the pixels)."""
+    c = float(cval)
+    if dtype == torch.float32:
+        with np.errstate(over="ignore"):
+            return float(np.float32(c))
+    lo, hi = _INT_RANGE[dtype]
+    if not math.isfinite(c) or not -2.0 ** 31 <= math.trunc(c) < 2.0 ** 31:
+        raise NotImplementedError(f"cval {cval!r} is outside the 32-bit range: scipy's cast of it to {dtype} is "
+                                  "platform-defined")
+    if two_cell_box:
+        if c > hi:
+            raise NotImplementedError(f"cval {cval!r} above the {dtype} range with a two-cell footprint is not supported")
+        return float(max(math.trunc(c), lo))
+    return float((math.trunc(c) - lo) % (hi - lo + 1) + lo)
+
+
+def _as_footprint(footprint) -> np.ndarray:
+    if isinstance(footprint, torch.Tensor):
+        footprint = footprint.detach().cpu().numpy()
+    return np.ascontiguousarray(np.asarray(footprint, dtype=bool))
 
 
 def median(image: torch.Tensor, footprint=None, out=None, mode: str = "nearest", cval: float = 0.0,
            behavior: str = "ndimage", *, halo_lo=None, halo_hi=None, peer_halos: bool = False) -> torch.Tensor:
-    """skimage.filters.median on a 2-D image (3x3 default) or 3-D volume (3x3x3 default)
-    -> scipy.ndimage.median_filter semantics (rank n//2).  Footprints: None or an all-ones
-    box of the default size.  `halo_lo` / `halo_hi`: the neighbouring slab's boundary
-    plane when the volume is one z-slab of a sharded volume (see volume.py); with `peer_halos=True` they may live on
-    another GPU of the box (the neighbour rank's slab mapped by CUDA IPC: the kernel reads them over NVLink)."""
+    """skimage.filters.median on a 2-D image or a 3-D volume -> scipy.ndimage.median_filter(image, footprint, mode=mode,
+    cval=cval): element count // 2 of the sorted window.  `footprint`: None (all-ones 3^ndim), or any numpy array,
+    torch tensor or nested list of the image's ndim, extents up to 65 (planes) or 17 (volumes); e.g.
+    skimage_compat.disk(r) / ball(r).  Modes 'nearest', 'reflect', 'mirror', 'wrap' and 'constant' (cval cast as
+    median_cval describes).
+
+    The default footprint in 'nearest', or in 'constant' with cval 0, runs mie_median2d / mie_median3d; every other
+    call runs mie_sk_median / mie_sk_median3d.  `halo_lo` / `halo_hi` (default footprint only): the neighbouring
+    slab's boundary plane when the volume is one z-slab of a sharded volume (see volume.py); with `peer_halos=True`
+    they may live on another GPU of the box (the neighbour rank's slab mapped by CUDA IPC: the kernel reads them over
+    NVLink)."""
     require_cuda(image)
     if behavior != "ndimage":
         raise NotImplementedError("behavior='rank' is not supported")
-    if mode not in _MEDIAN_MODES:
-        raise NotImplementedError(f"mode {mode!r} is not supported (nearest, constant)")
-    if mode == "constant" and cval != 0.0:
-        raise NotImplementedError("constant mode supports cval=0 only")
+    if mode not in SCIPY_MODES:
+        raise NotImplementedError(f"mode {mode!r} is not supported ({', '.join(SCIPY_MODES)})")
     if image.dim() not in (2, 3):
         raise ValueError("median expects a 2-D image or a 3-D volume")
-    if footprint is not None:
-        fp = np.asarray(footprint.cpu() if isinstance(footprint, torch.Tensor) else footprint)
-        if fp.shape != (3,) * image.dim() or not fp.all():
-            raise NotImplementedError("only the default all-ones 3^ndim footprint is supported")
-    border = BORDER[_MEDIAN_MODES[mode]]
+    ndim = image.dim()
+    box3 = footprint is None
+    if not box3:
+        fp = _as_footprint(footprint)
+        if fp.ndim != ndim:
+            raise RuntimeError(f"footprint.ndim ({fp.ndim}) must match len(axes) ({ndim})")
+        count = int(fp.sum())
+        if count == 0:
+            raise RuntimeError("rank not within filter footprint size")
+        if max(fp.shape) > MEDIAN_MAX_EXTENT[ndim]:
+            raise NotImplementedError(f"footprint extents up to {MEDIAN_MAX_EXTENT[ndim]} are supported for a {ndim}-D "
+                                      f"image; got {fp.shape}")
+        box3 = fp.shape == (3,) * ndim and count == fp.size
+        if mode == "reflect" and any(1 < n <= e // 8 for n, e in zip(image.shape, fp.shape)):
+            # scipy maps offset -2 n m (m >= 2) of an axis of length n to index -1 in 'reflect' mode and reads memory
+            # outside the image there
+            raise NotImplementedError(f"mode 'reflect' with footprint {fp.shape} reaches 4 times beyond an axis of "
+                                      f"image {tuple(image.shape)}, where scipy's result is undefined")
+    cv = 0.0
+    if mode == "constant":
+        cv = median_cval(image.dtype, cval, not box3 and count == 2 and count == fp.size)
+    default = box3 and (mode == "nearest" or (mode == "constant" and cv == 0.0))
     x = image.contiguous()
     dst = torch.empty_like(x) if out is None else check_out(x, out, (x.dtype,))
     if out is not None and out.untyped_storage().data_ptr() == x.untyped_storage().data_ptr():
@@ -195,6 +248,18 @@ def median(image: torch.Tensor, footprint=None, out=None, mode: str = "nearest",
                                                         x.data_ptr() + x.numel() * x.element_size())
         if lo < hi:
             raise ValueError("out must not overlap the input: the median kernels read neighbours they have not written yet")
+    border = BORDER[SCIPY_MODES[mode]]
+    if not default:
+        if halo_lo is not None or halo_hi is not None or peer_halos:
+            raise NotImplementedError("slab halos are supported with the default footprint only")
+        fp8 = np.ones((3,) * ndim, np.uint8) if footprint is None else fp.astype(np.uint8)
+        if ndim == 2:
+            call(x.device, "mie_sk_median", x.data_ptr(), dst.data_ptr(), DTYPE_CODE[x.dtype], *plane_layout(1, *x.shape),
+                 fp8.ctypes.data, *fp8.shape, border, cv)
+        else:
+            call(x.device, "mie_sk_median3d", x.data_ptr(), dst.data_ptr(), DTYPE_CODE[x.dtype],
+                 *volume_layout(1, *x.shape), fp8.ctypes.data, *fp8.shape, border, cv)
+        return dst
     if x.dim() == 2:
         call(x.device, "mie_median2d", x.data_ptr(), dst.data_ptr(), DTYPE_CODE[x.dtype], *plane_layout(1, *x.shape),
              3, 3, border)

@@ -10,7 +10,8 @@ kornia Gaussian with K = 2*int(truncate*sigma + 0.5) + 1 taps
 
     gaussian(image, sigma, mode=, truncate=)            <- skimage.filters.gaussian
     unsharp_mask(image, radius, amount, preserve_range) <- skimage.filters.unsharp_mask
-    median(image, ...)                                  <- skimage.filters.median           (filters.py)
+    median(image, footprint, mode=, cval=)              <- skimage.filters.median           (filters.py)
+    disk(radius), ball(radius)                          <- skimage.morphology.disk / ball (median footprints)
     denoise_nl_means(image, ...)                        <- skimage.restoration.denoise_nl_means (filters.py)
 
 Scale: skimage converts integer images to float with img_as_float (unsigned: v / max; signed: [-1, 1]).
@@ -63,16 +64,25 @@ import math
 import numpy as np
 import torch
 
-from ._ffi import (BORDER, DTYPE_CODE, MIE_F32, MIE_F64, as_planes, as_volumes, call, lib, new_out, plane_layout,
-                   require_cuda, use_workspace, value_range_of, volume_layout)
+from ._ffi import (BORDER, DTYPE_CODE, MIE_F32, MIE_F64, SCIPY_MODES, as_planes, as_volumes, call, lib, new_out,
+                   plane_layout, require_cuda, use_workspace, value_range_of, volume_layout)
 from .filters import MAX_TAPS, denoise_nl_means, gaussian_blur2d, get_gaussian_kernel1d, median  # noqa: F401
 
-__all__ = ["gaussian", "unsharp_mask", "median", "denoise_nl_means", "SCIPY_MODES", "equalize_adapthist", "equalize_hist",
+__all__ = ["gaussian", "unsharp_mask", "median", "disk", "ball", "denoise_nl_means", "SCIPY_MODES", "equalize_adapthist", "equalize_hist",
            "denoise_bilateral", "denoise_tv_chambolle", "structural_similarity", "frangi", "hessian", "sato",
            "meijering", "hessian_matrix", "hessian_matrix_eigvals"]
 
-SCIPY_MODES = {"nearest": "replicate", "reflect": "symmetric", "mirror": "reflect", "constant": "constant",
-               "wrap": "circular"}
+def disk(radius: int, dtype=np.uint8) -> np.ndarray:
+    """skimage.morphology.disk(radius) (RECALLED): the (2r+1)^2 uint8 mask X^2 + Y^2 <= r^2 over X, Y = -r .. r."""
+    g = np.arange(-int(radius), int(radius) + 1)
+    return np.asarray(g[:, None] ** 2 + g[None, :] ** 2 <= int(radius) ** 2, dtype=dtype)
+
+
+def ball(radius: int, dtype=np.uint8) -> np.ndarray:
+    """skimage.morphology.ball(radius) (RECALLED): the (2r+1)^3 uint8 mask X^2 + Y^2 + Z^2 <= r^2."""
+    g = np.arange(-int(radius), int(radius) + 1)
+    return np.asarray(g[:, None, None] ** 2 + g[None, :, None] ** 2 + g[None, None, :] ** 2 <= int(radius) ** 2,
+                      dtype=dtype)
 
 
 def _taps(sigma: float, truncate: float) -> int:
